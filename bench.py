@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- PC masker frames/s at 1080p (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload: synthetic 1920x1080 BGR sequence (pcm/synthetic.py, seed 0, 300 frames),
 default config.yaml params (20 trees, depth 5, "8 hsv_lab" -> 390 features/pixel,
@@ -21,6 +21,12 @@ the mask against the ground truth (computeBenchmark).
              float64 P(fg) written, SURVEY.md §8d) / its mean duration (CUDA events)
   cpu_baseline / --impl reference: oracle/ref_port.py (port of the reference's CPU
              path with the reference's cost structure), 1 core, bounded sample
+
+--dump-outputs DIR writes what the last step of the `value` loop handed its caller: the
+mask (DIR/mask.npy, float32 0/255) and its IoU counts (DIR/iou_counts.npy, float64
+intersection and union).  Only that loop is dumped: it is the path whose speed the line
+reports, and its seeded inputs are the same from run to run, so two builds compare output
+for output.  The reference arm and the sweep workload refuse the option.
 """
 import argparse
 import json
@@ -28,6 +34,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -305,6 +312,13 @@ def run_reference(args, rank, world):
     return out
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes every array as out_dir/<name>.npy, so that two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def workload_config():
     return {"workload": "synthetic 1920x1080 BGR sequence, 300 frames, crop = full frame (2073600 px), "
                         "3 models @ [0,100,200] blended, 16x16 grid labels",
@@ -390,6 +404,10 @@ def run_b200(args, rank, world, local_rank):
         barrier()
     ms_total = e0.elapsed_time(e1)
     launches = h.launch_count - launches0
+    if args.dump_outputs and rank == 0:
+        # what the last timed step handed its caller: the mask (0 / 255) and its (intersection, union) with the truth
+        dump_outputs(args.dump_outputs, {"mask": d_mask.cpu().numpy().astype(np.float32),
+                                         "iou_counts": d_counts[n_total - 1].cpu().numpy().astype(np.float64)})
     if dist is not None:
         t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -794,9 +812,7 @@ def sweep_run(args, rank, world):
         base = yaml.full_load(f)
     with open(os.path.join(PKG, "polygons.yaml")) as f:
         polygons = yaml.full_load(f)
-    return sweep.run(base, polygons, limit=args.sweep_limit or None, max_frames=args.sweep_max_frames or None,
-                     out_csv=os.path.join(ROOT, "gpurun_out", "benchmark_results.csv") if rank == 0 and
-                     os.path.isdir(os.path.join(ROOT, "gpurun_out")) else None, log=log,
+    return sweep.run(base, polygons, limit=args.sweep_limit or None, max_frames=args.sweep_max_frames or None, log=log,
                      seq_workers=args.sweep_workers or None)
 
 
@@ -856,10 +872,20 @@ def main():
     ap.add_argument("--sweep-limit", type=int, default=0, help="only the first N sequences of the 256")
     ap.add_argument("--sweep-max-frames", type=int, default=0)
     ap.add_argument("--sweep-workers", type=int, default=0, help="sequence threads per rank (0: cores_per_rank / 3, at most 6)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the mask and IoU counts of the last timed step as DIR/<name>.npy (1080p workload of the b200 arm)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "1080p"):
+        ap.error("--dump-outputs needs the 1080p workload of the b200 arm")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.e2e_only:
         args.steps = min(args.steps, 3)
+    # the CPU port (oracle/) caches its numba compilations on disk: in a directory of this run, never in the tree,
+    # which may be read-only
+    numba_cache = None
+    if "NUMBA_CACHE_DIR" not in os.environ:
+        numba_cache = tempfile.TemporaryDirectory(prefix="pcm_bench_numba_")
+        os.environ["NUMBA_CACHE_DIR"] = numba_cache.name
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

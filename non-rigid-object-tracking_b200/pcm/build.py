@@ -66,7 +66,7 @@ def build(force=False, verbose=False):
     if res.returncode != 0:
         raise RuntimeError("link failed (%d): %s" % (res.returncode, " ".join(link)))
     if LIB.endswith("libpcm_b200.so"):       # registers / spills / shared memory per kernel (ptxas -v), without timings
-        with open(os.path.join(PKG, "csrc", "ptxas_info.txt"), "w") as f:
+        with open(os.path.join(PKG, "build", "ptxas_info.txt"), "w") as f:
             f.write("".join(l for text in log for l in text.splitlines(True) if "Compile time" not in l))
     return LIB
 

@@ -2,8 +2,8 @@
 //
 // C-ABI face of the Felzenszwalb-Huttenlocher segmentation the reference vendors under
 // prim/src/FelzenSegment (segment-graph.h:48-81 segment_graph, segment_image_index.h:14-121
-// segment_image_index).  The reference's headers are #included from where they lie under
-// /root/reference (-I on the compiler command line, see oracle/build_ref.py); nothing of them is
+// segment_image_index).  The reference's headers are #included from where they lie in the
+// checkout named by PCM_REFERENCE_ROOT (-I on the compiler command line, see oracle/build_ref.py); nothing of them is
 // copied into this repository.  The resulting oracle/_ref/libfelzen_ref.so is used by
 // tests/test_felzenszwalb_ref.py to pin the parts of pcm_felzenszwalb that coincide with the
 // original algorithm: cost-ordered greedy merge with the k/|C| threshold, union-find, the

@@ -1,6 +1,8 @@
 """pcm_felzenszwalb against the Felzenszwalb-Huttenlocher code the reference vendors
-(/root/reference/prim/src/FelzenSegment: segment-graph.h:48-81, segment_image_index.h:14-121),
-compiled from where it lies into oracle/_ref/libfelzen_ref.so (oracle/build_ref.py).  SURVEY §8 row f-1.
+(prim/src/FelzenSegment: segment-graph.h:48-81, segment_image_index.h:14-121), compiled from a
+checkout of the reference named by PCM_REFERENCE_ROOT into oracle/_ref/libfelzen_ref.so; without
+one, against oracle/felzen_fh_restated.cpp, the published algorithm restated with the same
+arithmetic and entry points (oracle/build_ref.py).  SURVEY §8 row f-1.
 
 What coincides between that code and the scikit-image variant the product implements is checked
 EXACTLY on identical edge lists: the cost-ordered greedy merge with the k/|C| threshold, the
@@ -24,9 +26,7 @@ import build_ref  # noqa: E402
 
 @pytest.fixture(scope="module")
 def ref():
-    path = build_ref.build()
-    if path is None:
-        pytest.skip("oracle/_ref/libfelzen_ref.so is absent and /root/reference is not here to build it")
+    path, _ = build_ref.build()
     lib = C.CDLL(path)
     P, I, F = C.c_void_p, C.c_int, C.c_float
     lib.felzen_ref_graph.restype = I
