@@ -93,8 +93,16 @@ int pcm_add_model(pcm_handle* h, int n_frame, int n_trees, const int64_t* tree_o
                   int* model_index);
 
 /* Attach the novelty detector of a model: PCA mean_[F], components_[0][F]
- * (n_components == 1, config.yaml:27) (:205-213). */
+ * (n_components == 1, config.yaml:27) (:205-213).  Same as pcm_set_novelty_k with n_components = 1. */
 int pcm_set_novelty(pcm_handle* h, int model_index, const double* mean, const double* component, int n_features);
+
+/* The novelty detector of a PCA with several components (params.n_components, :203-213): mean_[F] and
+ * components_[n_components][F], row-major, as scikit-learn stores them.  1 <= n_components <= PCM_MAX_PCA_COMPONENTS
+ * (PCM_E_INVALID below, PCM_E_LIMIT above).  A frame whose current or next model has two or more components computes
+ * the reconstruction error in a kernel of its own (profile id 7); rank-1 models keep the score kernel's in-line pass. */
+#define PCM_MAX_PCA_COMPONENTS 8
+int pcm_set_novelty_k(pcm_handle* h, int model_index, const double* mean, const double* components, int n_components,
+                      int n_features);
 
 int pcm_num_models(const pcm_handle* h);
 
@@ -311,15 +319,20 @@ int pcm_fit_forest(pcm_handle* h, const int16_t* X, const uint8_t* y, int n_rows
 /* Upload a training-row set (as for pcm_fit_forest) without fitting; it stays resident under rows_id != 0. */
 int pcm_fit_rows(pcm_handle* h, const int16_t* X, const uint8_t* y, int n_rows, int n_features, long long rows_id);
 
-/* Novelty detector of addModel (:203-213: PCA(n_components=1).fit(X[labels == 1]), then the L1 reconstruction
+/* Novelty detector of addModel (:203-213: PCA(n_components=k).fit(X[labels == 1]), then the L1 reconstruction
  * error of every training row) on the RESIDENT rows `rows_id`:
- *   pcm_pca_moments    gram[F*F] = sum over class-1 rows of v v^T, sums[F] = sum of v (raw integer feature values,
- *                      exact), n_class1.  The caller forms sklearn's covariance (decomposition/_pca.py, solver
- *                      covariance_eigh) and takes its leading eigenvector (pcm/train.py: numpy.linalg.eigh).
- *   pcm_pca_residuals  err[n_rows] = sum_f |x_f - (t c_f + mean_f)|, t = x.c - mean.c, x = v / 255 (:208-211) for
- *                      every row; the caller takes np.percentile(err, 90) as the outlier threshold (:212). */
+ *   pcm_pca_moments      gram[F*F] = sum over class-1 rows of v v^T, sums[F] = sum of v (raw integer feature values,
+ *                        exact), n_class1.  The caller forms sklearn's covariance (decomposition/_pca.py, solver
+ *                        covariance_eigh) and takes its leading eigenvectors (pcm/train.py: numpy.linalg.eigh).
+ *   pcm_pca_residuals    err[n_rows] = sum_f |x_f - (t c_f + mean_f)|, t = x.c - mean.c, x = v / 255 (:208-211) for
+ *                        every row; the caller takes np.percentile(err, 90) as the outlier threshold (:212).
+ *   pcm_pca_residuals_k  the same for components[n_components][F] (row-major, 1 <= n_components <=
+ *                        PCM_MAX_PCA_COMPONENTS): t_j = x.c_j - mean.c_j, err = sum_f |x_f - (mean_f + sum_j t_j c_jf)|.
+ *                        With n_components = 1 it returns the bits of pcm_pca_residuals. */
 int pcm_pca_moments(pcm_handle* h, long long rows_id, double* gram, double* sums, int64_t* n_class1);
 int pcm_pca_residuals(pcm_handle* h, long long rows_id, const double* mean, const double* component, double* err);
+int pcm_pca_residuals_k(pcm_handle* h, long long rows_id, const double* mean, const double* components, int n_components,
+                        double* err);
 
 /* ---- parity taps (tests, smoke; not needed by the reference flow) -------- */
 
@@ -364,11 +377,12 @@ int pcm_transfer_bytes(const pcm_handle* h, int64_t out[2]);
  * launch while enabled).  Kernel ids: 0 score (fused star features + forests),
  * 1 (retired: the per-label reduction is K1's epilogue), 2 segment_decide, 3 (retired: the exact
  * re-evaluation is part of segment_decide), 4 mask_dilate, 5 iou,
- * 6 planes (colour conversion to planar tiles).
+ * 6 planes (colour conversion to planar tiles), 7 novelty (reconstruction error of PCAs with
+ * two or more components; launched only for frames that use one).
  * pcm_profile_read synchronises the stream, adds the finished launches to the
  * running totals and returns them (ms_sum[i], count[i] for i < n <= PCM_NUM_KERNELS);
  * reset != 0 clears the totals afterwards. */
-#define PCM_NUM_KERNELS 7
+#define PCM_NUM_KERNELS 8
 int pcm_profile_enable(pcm_handle* h, int on);
 int pcm_profile_read(pcm_handle* h, double* ms_sum, int64_t* count, int n, int reset);
 

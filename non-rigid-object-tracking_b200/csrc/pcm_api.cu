@@ -231,8 +231,11 @@ struct Model {
     DevBuf blob;                  // nodes | leaves | trees, one block (from the process-wide block cache)
     TopNodes top{};               // root + its children of the first MAX_TOP_TREES trees
     bool has_pca = false;
-    DevPCA pca{};
-    DevBuf pca_buf;               // comp | comp255 | mean, 3F doubles
+    int pca_k = 0;                // n_components of the PCA
+    DevPCA pca{};                 // rank 1: K1's in-line pass
+    DevBuf pca_buf;               // comp | comp255 | mean, 3F doubles (rank 1)
+    DevBuf pcak_buf;              // novelty_kernel's coefficients: [F][pca_k + 1] in its visiting order (any rank)
+    double pcak_mdc[MAX_PCA_K] = {0};   // mean_ . components_[j]
     int max_depth = 0;
 };
 
@@ -533,6 +536,7 @@ struct Encoder {
 static void free_model(Model& m) {
     m.blob.release();
     m.pca_buf.release();
+    m.pcak_buf.release();
     m = Model{};
 }
 
@@ -608,6 +612,12 @@ extern "C" int pcm_create(int device, pcm_handle** out) {
             CUDA_TRY(cudaFuncSetAttribute(qs_density_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ds.max_smem_optin));
             CUDA_TRY(cudaFuncSetAttribute(qs_density_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ds.max_smem_optin));
             CUDA_TRY(cudaFuncSetAttribute(qs_parent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ds.max_smem_optin));
+            CUDA_TRY(cudaFuncSetAttribute(novelty_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ds.max_smem_optin));
+            // once per device, never per call: the fits of a sweep run in several threads with different feature counts,
+            // and a per-call limit set by one thread could undercut another thread's launch
+            for (auto fn : {pca_residual_kernel<1>, pca_residual_kernel<2>, pca_residual_kernel<3>, pca_residual_kernel<4>,
+                            pca_residual_kernel<5>, pca_residual_kernel<6>, pca_residual_kernel<7>, pca_residual_kernel<8>})
+                CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, ds.max_smem_optin));
             ds.ready = true;
         }
     }
@@ -774,32 +784,68 @@ extern "C" int pcm_add_model(pcm_handle* h, int n_frame, int n_trees, const int6
     return PCM_OK;
 }
 
+static_assert(MAX_PCA_K == PCM_MAX_PCA_COMPONENTS, "novelty_kernel and the C ABI disagree on the component limit");
+
+extern "C" int pcm_set_novelty_k(pcm_handle* h, int model_index, const double* mean, const double* components,
+                                 int n_components, int n_features) {
+    if (!h || !mean || !components) return fail(PCM_E_INVALID, "pcm_set_novelty_k: NULL argument");
+    if (n_components < 1) return fail(PCM_E_INVALID, "pcm_set_novelty_k: n_components %d < 1", n_components);
+    if (n_components > PCM_MAX_PCA_COMPONENTS)
+        return fail(PCM_E_LIMIT, "pcm_set_novelty_k: n_components %d > PCM_MAX_PCA_COMPONENTS (%d)", n_components,
+                    PCM_MAX_PCA_COMPONENTS);
+    if (model_index < 0 || model_index >= (int)h->models.size())
+        return fail(PCM_E_INVALID, "pcm_set_novelty_k: model %d does not exist", model_index);
+    if (n_features != h->geom.F) return fail(PCM_E_INVALID, "pcm_set_novelty_k: n_features %d != F %d", n_features, h->geom.F);
+    CUDA_TRY(cudaSetDevice(h->device));
+    Model& m = h->models[model_index];
+    const Geom& g = h->geom;
+    const int F = g.F, k = n_components, nch = 3 * g.n_spaces;
+    // rank 1: K1's vectors in feature order
+    if (k == 1) {
+        std::vector<double> buf(3 * (size_t)F);
+        double mdc = 0.0;
+        for (int f = 0; f < F; ++f) {
+            buf[f] = components[f];
+            buf[F + f] = components[f] / 255.0;
+            buf[2 * F + f] = mean[f];
+            mdc += mean[f] * components[f];
+        }
+        CUDA_TRY(m.pca_buf.reserve(buf.size() * sizeof(double)));
+        CUDA_TRY(cudaMemcpyAsync(m.pca_buf.p, buf.data(), buf.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        m.pca.comp = m.pca_buf.as<double>();
+        m.pca.comp255 = m.pca.comp + F;
+        m.pca.mean = m.pca.comp + 2 * F;
+        m.pca.mean_dot_comp = mdc;
+    } else {
+        m.pca = DevPCA{};
+    }
+    // any rank: novelty_kernel's coefficients in its visiting order (a rank-1 model blended with a higher-rank one is
+    // scored there too)
+    std::vector<double> kb((size_t)F * (k + 1));
+    for (int it = 0; it < F; ++it) {
+        const int tap = it / nch, p = it - tap * nch;
+        const int f = (p / 3) * 3 * g.K + 3 * tap + (p % 3);
+        for (int j = 0; j < k; ++j) kb[(size_t)it * (k + 1) + j] = components[(size_t)j * F + f];
+        kb[(size_t)it * (k + 1) + k] = mean[f];
+    }
+    for (int j = 0; j < MAX_PCA_K; ++j) {
+        double mdc = 0.0;
+        if (j < k)
+            for (int f = 0; f < F; ++f) mdc += mean[f] * components[(size_t)j * F + f];
+        m.pcak_mdc[j] = mdc;
+    }
+    CUDA_TRY(m.pcak_buf.reserve(kb.size() * sizeof(double)));
+    CUDA_TRY(cudaMemcpyAsync(m.pcak_buf.p, kb.data(), kb.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
+    m.pca_k = k;
+    m.has_pca = true;
+    return PCM_OK;
+}
+
 extern "C" int pcm_set_novelty(pcm_handle* h, int model_index, const double* mean, const double* component,
                                int n_features) {
     if (!h || !mean || !component) return fail(PCM_E_INVALID, "pcm_set_novelty: NULL argument");
-    if (model_index < 0 || model_index >= (int)h->models.size())
-        return fail(PCM_E_INVALID, "pcm_set_novelty: model %d does not exist", model_index);
-    if (n_features != h->geom.F) return fail(PCM_E_INVALID, "pcm_set_novelty: n_features %d != F %d", n_features, h->geom.F);
-    CUDA_TRY(cudaSetDevice(h->device));
-    Model& m = h->models[model_index];
-    const int F = h->geom.F;
-    std::vector<double> buf(3 * (size_t)F);
-    double mdc = 0.0;
-    for (int f = 0; f < F; ++f) {
-        buf[f] = component[f];
-        buf[F + f] = component[f] / 255.0;
-        buf[2 * F + f] = mean[f];
-        mdc += mean[f] * component[f];
-    }
-    CUDA_TRY(m.pca_buf.reserve(buf.size() * sizeof(double)));
-    CUDA_TRY(cudaMemcpyAsync(m.pca_buf.p, buf.data(), buf.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    CUDA_TRY(cudaStreamSynchronize(h->stream));
-    m.pca.comp = m.pca_buf.as<double>();
-    m.pca.comp255 = m.pca.comp + F;
-    m.pca.mean = m.pca.comp + 2 * F;
-    m.pca.mean_dot_comp = mdc;
-    m.has_pca = true;
-    return PCM_OK;
+    return pcm_set_novelty_k(h, model_index, mean, component, 1, n_features);
 }
 
 // ---------------------------------------------------------------------------------
@@ -955,13 +1001,34 @@ static int enqueue_update(pcm_handle* h, const uint8_t* d_frame, int H, int W, i
         a.depth = std::max(a.depth, h->models[p->model_next].max_depth);
     }
     a.w0 = p->w_cur; a.w1 = p->w_next;
+    // a PCA of rank >= 2 on either model: novelty_kernel computes the (blended) error map between K0 and K1, which K1 and
+    // K2 read; otherwise K1's in-line rank-1 pass
+    const Model* m1 = a.blend ? &h->models[p->model_next] : nullptr;
+    const bool nov_k = p->novelty != 0 && (m0.pca_k > 1 || (m1 && m1->pca_k > 1));
     a.novelty = p->novelty != 0;
-    if (a.novelty) {
+    if (a.novelty && !nov_k) {
         a.pca0 = m0.pca;
-        if (a.blend) a.pca1 = h->models[p->model_next].pca;
+        if (a.blend) a.pca1 = m1->pca;
+    }
+    NoveltyArgs na{};
+    if (nov_k) {
+        CUDA_TRY(h->sa.reserve(npx * sizeof(double)));
+        a.nov_in = h->sa.as<double>();
+        na.g = g;
+        na.cw = cw; na.ch = ch;
+        na.coef0 = m0.pcak_buf.as<double>(); na.k0 = m0.pca_k;
+        for (int j = 0; j < MAX_PCA_K; ++j) na.mdc0[j] = m0.pcak_mdc[j];
+        na.blend = a.blend;
+        if (m1) {
+            na.coef1 = m1->pcak_buf.as<double>(); na.k1 = m1->pca_k;
+            for (int j = 0; j < MAX_PCA_K; ++j) na.mdc1[j] = m1->pcak_mdc[j];
+        }
+        na.w0 = a.w0; na.w1 = a.w1;
+        na.staged = (int)novelty_smem_bytes(g, na.k0, na.k1, a.blend, true) <= h->max_smem_optin;
+        na.out = h->sa.as<double>();
     }
     a.p1_out = keep_maps ? h->p1.as<double>() : nullptr;
-    a.sa_out = (keep_maps && a.novelty) ? h->sa.as<double>() : nullptr;
+    a.sa_out = (keep_maps && a.novelty && !nov_k) ? h->sa.as<double>() : nullptr;
     a.seg.labels = d_labels;
     a.seg.n_labels = S;
     a.seg.thr = p->outlier_threshold;
@@ -969,9 +1036,9 @@ static int enqueue_update(pcm_handle* h, const uint8_t* d_frame, int H, int W, i
     a.seg.rmin = pa.rmin; a.seg.rmax = pa.rmax; a.seg.cmin = pa.cmin; a.seg.cmax = pa.cmax; a.seg.err = h->d_err;
 
     // forests live in shared memory whenever one CTA's tiles + forests fit, else they are read through L1
-    ScoreSmem ls = score_smem_layout(a.g, a.f0, a.f1, a.blend, a.novelty, true);
+    ScoreSmem ls = score_smem_layout(a.g, a.f0, a.f1, a.blend, a.novelty && !nov_k, true);
     const bool forest_smem = (int)ls.total <= h->max_smem_optin;
-    if (!forest_smem) ls = score_smem_layout(a.g, a.f0, a.f1, a.blend, a.novelty, false);
+    if (!forest_smem) ls = score_smem_layout(a.g, a.f0, a.f1, a.blend, a.novelty && !nov_k, false);
     if ((int)ls.total > h->max_smem_optin)
         return fail(PCM_E_LIMIT, "update: tile needs %u B of shared memory (> %d)", ls.total, h->max_smem_optin);
     // CTAs per SM of an instantiation at this shared-memory size (queried once per distinct size: the runtime call
@@ -1035,9 +1102,37 @@ static int enqueue_update(pcm_handle* h, const uint8_t* d_frame, int H, int W, i
         CHECK_LAUNCH(h, sv.name);
         return PCM_OK;
     };
+    // novelty_kernel for the crop rows of K1's tile rows [ty0, ty1) (no launch unless a PCA of rank >= 2 is in use)
+    auto launch_nk = [&](int ty0, int ty1) -> int {
+        if (!nov_k) return PCM_OK;
+        NoveltyArgs b = na;
+        b.planes = pa.planes; b.pitch = pitch; b.plane_stride = plane_stride;
+        b.row0 = ty0 * tile_h;
+        b.rows = std::min(ch, ty1 * tile_h) - b.row0;
+        const size_t smem = novelty_smem_bytes(g, b.k0, b.k1, b.blend != 0, b.staged != 0);
+        int nk_occ = 0;
+        {
+            static std::mutex nk_m;
+            static std::vector<std::pair<size_t, int>> nk_cache;     // CTAs per SM by shared-memory size
+            std::lock_guard<std::mutex> lk(nk_m);
+            for (auto& e : nk_cache)
+                if (e.first == smem) nk_occ = e.second;
+            if (!nk_occ) {
+                CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nk_occ, novelty_kernel, NTHREADS, smem));
+                nk_occ = std::max(nk_occ, 1);
+                if (nk_cache.size() < 4096) nk_cache.push_back({smem, nk_occ});
+            }
+        }
+        const long long n_tiles = (long long)((cw + NOV_TW - 1) / NOV_TW) * ((b.rows + NOV_TH - 1) / NOV_TH);
+        const int grid = (int)std::max<long long>(1, std::min<long long>(n_tiles, (long long)h->sm_count * nk_occ));
+        KernelTimer kt(h, 7);
+        CUDA_TRY(launch_chain(novelty_kernel, dim3(grid), dim3(NTHREADS), smem, st, b));
+        CHECK_LAUNCH(h, "novelty_kernel");
+        return PCM_OK;
+    };
     int rc = PCM_OK;
     if (!feed) {
-        if ((rc = launch_k0(0, ch, true)) || (rc = launch_k1(0, tiles_y))) return rc;
+        if ((rc = launch_k0(0, ch, true)) || (rc = launch_nk(0, tiles_y)) || (rc = launch_k1(0, tiles_y))) return rc;
     } else {
         // bands of whole tile rows, at least ~512 Ki px each; band b needs the crop rows up to the lower halo of its last tile row
         static const int max_bands = [] { const char* e = getenv("PCM_FEED_BANDS"); int v = e ? atoi(e) : 0; return v >= 1 && v <= 4 ? v : 2; }();      // measured at 1080p: 1 / 2 / 3 bands -> update 0.434 / 0.429 / 0.471 ms
@@ -1054,7 +1149,7 @@ static int enqueue_update(pcm_handle* h, const uint8_t* d_frame, int H, int W, i
             if (!h->feed_events[b]) CUDA_TRY(cudaEventCreateWithFlags(&h->feed_events[b], cudaEventDisableTiming));
             CUDA_TRY(cudaEventRecord(h->feed_events[b], h->copy_stream));
             CUDA_TRY(cudaStreamWaitEvent(st, h->feed_events[b], 0));
-            if ((rc = launch_k0(rows_done, rows_end, b == 0)) || (rc = launch_k1(ty0, ty1))) return rc;
+            if ((rc = launch_k0(rows_done, rows_end, b == 0)) || (rc = launch_nk(ty0, ty1)) || (rc = launch_k1(ty0, ty1))) return rc;
             rows_done = rows_end;
         }
         h->bytes_h2d += (int64_t)(npx * 3);
@@ -1062,12 +1157,13 @@ static int enqueue_update(pcm_handle* h, const uint8_t* d_frame, int H, int W, i
 
     // ---- K2: per-label decision (+ exact path) ------------------------------------------------
     DecideArgs da{};
-    da.p1 = a.p1_out; da.sa = a.sa_out; da.labels = d_labels; da.cw = cw; da.thr = p->outlier_threshold;
+    da.p1 = a.p1_out; da.sa = nov_k && keep_maps ? a.nov_in : a.sa_out; da.labels = d_labels; da.cw = cw; da.thr = p->outlier_threshold;
     da.sum = pa.sum; da.asum = pa.asum; da.area = pa.area; da.rmin = pa.rmin; da.rmax = pa.rmax;
     da.cmin = pa.cmin; da.cmax = pa.cmax;
     da.ps.planes = pa.planes; da.ps.pitch = pitch; da.ps.plane_stride = plane_stride; da.ps.cw = cw; da.ps.ch = ch;
     da.ps.g = g; da.ps.f0 = a.f0; da.ps.f1 = a.f1; da.ps.depth = a.depth; da.ps.blend = a.blend;
-    da.ps.w0 = a.w0; da.ps.w1 = a.w1; da.ps.novelty = a.novelty; da.ps.pca0 = a.pca0; da.ps.pca1 = a.pca1;
+    da.ps.w0 = a.w0; da.ps.w1 = a.w1; da.ps.novelty = a.novelty && !nov_k; da.ps.pca0 = a.pca0; da.ps.pca1 = a.pca1;
+    da.ps.nov_map = a.nov_in;
     da.priors = d_priors;
     da.n_labels = S;
     da.prior_weight = p->prior_weight;
@@ -1106,7 +1202,7 @@ static int enqueue_update(pcm_handle* h, const uint8_t* d_frame, int H, int W, i
     CHECK_LAUNCH(h, "mask_dilate_kernel");
 
     h->last_cw = cw; h->last_ch = ch; h->last_S = S;
-    h->last_novelty = a.novelty;
+    h->last_novelty = p->novelty != 0;      // rank 1: K1 wrote h->sa (maps kept); rank >= 2: novelty_kernel did
     h->last_valid = true;
     h->last_pre = want_pre;
     h->last_maps = keep_maps;
@@ -1967,25 +2063,42 @@ extern "C" int pcm_pca_moments(pcm_handle* h, long long rows_id, double* gram, d
     return PCM_OK;
 }
 
-extern "C" int pcm_pca_residuals(pcm_handle* h, long long rows_id, const double* mean, const double* component, double* err) {
-    if (!h || !mean || !component || !err) return fail(PCM_E_INVALID, "pcm_pca_residuals: NULL argument");
-    if (rows_id == 0 || rows_id != h->fit_rows_id) return fail(PCM_E_STATE, "pcm_pca_residuals: rows %lld are not resident", rows_id);
+extern "C" int pcm_pca_residuals_k(pcm_handle* h, long long rows_id, const double* mean, const double* components,
+                                   int n_components, double* err) {
+    if (!h || !mean || !components || !err) return fail(PCM_E_INVALID, "pcm_pca_residuals_k: NULL argument");
+    if (n_components < 1) return fail(PCM_E_INVALID, "pcm_pca_residuals_k: n_components %d < 1", n_components);
+    if (n_components > PCM_MAX_PCA_COMPONENTS)
+        return fail(PCM_E_LIMIT, "pcm_pca_residuals_k: n_components %d > PCM_MAX_PCA_COMPONENTS (%d)", n_components,
+                    PCM_MAX_PCA_COMPONENTS);
+    if (rows_id == 0 || rows_id != h->fit_rows_id) return fail(PCM_E_STATE, "pcm_pca_residuals_k: rows %lld are not resident", rows_id);
     CUDA_TRY(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
     h->chain_tail = false;
-    const int F = h->fit_F, n = h->fit_n;
+    const int F = h->fit_F, n = h->fit_n, k = n_components;
     const long long n_pad = ((long long)n + 63) / 64 * 64;
-    const size_t fb = sizeof(double) * (size_t)F, eb = sizeof(double) * (size_t)n;
-    CUDA_TRY(h->fit_out.reserve(2 * fb + eb));
+    const size_t fb = sizeof(double) * (size_t)F, cb = fb * k, eb = sizeof(double) * (size_t)n;
+    CUDA_TRY(h->fit_out.reserve(cb + fb + eb));
     char* ob = h->fit_out.as<char>();
-    CUDA_TRY(cudaMemcpyAsync(ob, component, fb, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(ob + fb, mean, fb, cudaMemcpyHostToDevice, st));
-    pca_residual_kernel<<<(n + 255) / 256, 256, 2 * fb, st>>>(h->fit_xt.as<int16_t>(), n_pad, n, F, reinterpret_cast<double*>(ob + fb),
-                                                            reinterpret_cast<double*>(ob), reinterpret_cast<double*>(ob + 2 * fb));
+    CUDA_TRY(cudaMemcpyAsync(ob, components, cb, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(ob + cb, mean, fb, cudaMemcpyHostToDevice, st));
+    typedef void (*ResFn)(const int16_t*, long long, int, int, const double*, const double*, double*);
+    static const ResFn table[PCM_MAX_PCA_COMPONENTS] = {pca_residual_kernel<1>, pca_residual_kernel<2>, pca_residual_kernel<3>,
+                                                        pca_residual_kernel<4>, pca_residual_kernel<5>, pca_residual_kernel<6>,
+                                                        pca_residual_kernel<7>, pca_residual_kernel<8>};
+    const size_t smem = cb + fb;                       // components | mean
+    if ((long long)smem > h->max_smem_optin)
+        return fail(PCM_E_LIMIT, "pcm_pca_residuals_k: %d x %d components need %zu B of shared memory", k, F, smem);
+    table[k - 1]<<<(n + 255) / 256, 256, smem, st>>>(h->fit_xt.as<int16_t>(), n_pad, n, F, reinterpret_cast<double*>(ob + cb),
+                                                     reinterpret_cast<double*>(ob), reinterpret_cast<double*>(ob + cb + fb));
     CHECK_LAUNCH(h, "pca_residual_kernel");
-    CUDA_TRY(cudaMemcpyAsync(err, ob + 2 * fb, eb, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(err, ob + cb + fb, eb, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return PCM_OK;
+}
+
+extern "C" int pcm_pca_residuals(pcm_handle* h, long long rows_id, const double* mean, const double* component, double* err) {
+    if (!h || !mean || !component || !err) return fail(PCM_E_INVALID, "pcm_pca_residuals: NULL argument");
+    return pcm_pca_residuals_k(h, rows_id, mean, component, 1, err);
 }
 
 // ---------------------------------------------------------------------------------

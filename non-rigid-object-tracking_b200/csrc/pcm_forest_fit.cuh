@@ -366,27 +366,40 @@ __global__ void __launch_bounds__(256) pca_gram_kernel(const int16_t* __restrict
     if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) *n1 = (unsigned long long)ones;
 }
 
-// L1 reconstruction error of EVERY training row under the rank-1 PCA (:208-211):
-//   t = x . c - mean . c ;  err = sum_f |x_f - (t c_f + mean_f)|,  x = v / 255.   One thread per row.
+// L1 reconstruction error of EVERY training row under a PCA of KC components (:208-211), x = v / 255:
+//   t_j = x . c_j - mean . c_j  (both dot products fma-accumulated in feature order)
+//   err = sum_f |x_f - r_f|,  r_f = fma(t_{KC-1}, c_{KC-1,f}, ... fma(t_0, c_0f, mean_f))
+// For KC = 1 this is the rank-1 arithmetic t = x . c - mean . c, err = sum_f |x_f - fma(t, c_f, mean_f)|.  One thread per row.
+template <int KC>
 __global__ void __launch_bounds__(256) pca_residual_kernel(const int16_t* __restrict__ Xt, long long n_pad, int n, int F,
                                                            const double* __restrict__ mean, const double* __restrict__ comp,
                                                            double* __restrict__ err) {
-    extern __shared__ double sh[];          // comp[F] | mean[F]
-    for (int f = threadIdx.x; f < F; f += blockDim.x) { sh[f] = comp[f]; sh[F + f] = mean[f]; }
+    extern __shared__ double sh[];          // comp[KC][F] | mean[F]
+    for (int f = threadIdx.x; f < (KC + 1) * F; f += blockDim.x) sh[f] = f < KC * F ? comp[f] : mean[f - KC * F];
     __syncthreads();
+    const double* shm = sh + KC * F;
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= n) return;
-    double t = 0.0, mdc = 0.0;
+    double t[KC], mdc[KC];
+#pragma unroll
+    for (int j = 0; j < KC; ++j) { t[j] = 0.0; mdc[j] = 0.0; }
     for (int f = 0; f < F; ++f) {
         const double x = (double)Xt[(size_t)f * n_pad + r] / 255.0;
-        t = fma(x, sh[f], t);
-        mdc = fma(sh[F + f], sh[f], mdc);
+#pragma unroll
+        for (int j = 0; j < KC; ++j) {
+            t[j] = fma(x, sh[j * F + f], t[j]);
+            mdc[j] = fma(shm[f], sh[j * F + f], mdc[j]);
+        }
     }
-    t -= mdc;
+#pragma unroll
+    for (int j = 0; j < KC; ++j) t[j] -= mdc[j];
     double e = 0.0;
     for (int f = 0; f < F; ++f) {
         const double x = (double)Xt[(size_t)f * n_pad + r] / 255.0;
-        e += fabs(x - fma(t, sh[f], sh[F + f]));
+        double rec = shm[f];
+#pragma unroll
+        for (int j = 0; j < KC; ++j) rec = fma(t[j], sh[j * F + f], rec);
+        e += fabs(x - rec);
     }
     err[r] = e;
 }

@@ -1,6 +1,7 @@
 // pcm_kernels.cuh -- CUDA kernels of the PC masker hot path (sm_100a).
 //
 //  K0 planes_kernel, K1 score_kernel: pcm_score.cuh
+//  Kn novelty_kernel      PCA reconstruction error of models with two or more components, between K0 and K1
 //  K2 segment_decide      per-label score and decision (:240-242); labels inside the guard
 //                         band are re-evaluated exactly (sequential float32, raster order) from
 //                         per-pixel values the block recomputes for the label's bounding box
@@ -11,6 +12,166 @@
 #include "pcm_score.cuh"
 
 namespace pcm {
+
+// Kn -----------------------------------------------------------------------------
+// Novelty error of PCAs with two or more components (params.n_components > 1; :57-63, :88-93 with
+// PCA(n_components=k), :203-213).  Launched between K0 and K1 for a frame whose current or next model has such a PCA;
+// it writes the blended error of every crop pixel (blend2, as K1 blends), and K1 and K2's exact path read that map
+// instead of computing the term themselves, so both use the same bits.  Rank-1 models keep K1's in-line pass
+// (novelty_error, pcm_score.cuh) unless blended with a higher-rank one.
+//
+// Arithmetic (scikit-learn's transform / inverse_transform, whiten=False), per pixel and model, with x_f = v_f / 255
+// (v_f the plane byte, -1 outside the crop):
+//   t_j  = S_j / 255 - mdc_j,   S_j = sum_f v_f c_jf accumulated with fma (exact v_f),   mdc_j = mean . c_j (host,
+//          feature order)                                                        -> t_j = x . c_j - mean . c_j
+//   r_f  = fma(t_{k-1}, c_{k-1,f}, ... fma(t_1, c_1f, fma(t_0, c_0f, mean_f)))      -> mean_f + sum_j t_j c_jf
+//   err  = sum_f |fma(v_f, 1/255, -r_f)|                                             -> sum_f |x_f - r_f|
+// Every sum runs over the features in K1's order: tap by tap, plane by plane (entry it = k * nch + p holds feature
+// (p / 3) * 3K + 3k + p % 3).  The coefficients of a model are laid out in that order, k + 1 doubles per entry
+// ({c_0f .. c_{k-1}f, mean_f}), and staged in shared memory when they fit (always on sm_100: two models of F <= 1161,
+// k <= 8 take 167 KB), else read through L1.
+// A CTA scores tiles of NOV_TW x NOV_TH pixels (persistent, grid-stride); a thread owns NOV_PIX consecutive rows of one
+// column, so every coefficient load serves NOV_PIX pixels.  Plane bytes are read through L1 (the 2n+1 rows of taps of
+// a tile are reused by all of its pixels).
+constexpr int MAX_PCA_K = 8;
+constexpr int NOV_PIX = 4, NOV_TW = 32, NOV_TH = (NTHREADS / 32) * NOV_PIX;
+
+struct NoveltyArgs {
+    const uint8_t* planes;     // K0's planar crop (as PixelScorer)
+    long long pitch, plane_stride;
+    int cw, ch;
+    int row0, rows;            // crop rows [row0, row0 + rows) of this launch
+    Geom g;
+    const double* coef0;       // model 0: [F][k0 + 1] in visiting order (see above)
+    const double* coef1;       // model 1 (blend)
+    int k0, k1;
+    double mdc0[MAX_PCA_K], mdc1[MAX_PCA_K];
+    int blend;
+    double w0, w1;
+    int staged;                // 1: coefficients copied to shared memory
+    double* out;               // [ch*cw]
+};
+
+__host__ __device__ inline size_t novelty_smem_bytes(const Geom& g, int k0, int k1, bool blend, bool staged) {
+    return staged ? sizeof(double) * (size_t)g.F * ((k0 + 1) + (blend ? k1 + 1 : 0)) : 0;
+}
+
+template <int KC>
+__device__ __forceinline__ void pca_l1_error(const NoveltyArgs& a, const double* coef, const double* mdc,
+                                             int x, int y, double (&err)[NOV_PIX]) {
+    const Geom& g = a.g;
+    const int nch = 3 * g.n_spaces;
+    double t[KC][NOV_PIX];
+#pragma unroll
+    for (int i = 0; i < NOV_PIX; ++i) {
+        err[i] = 0.0;
+#pragma unroll
+        for (int j = 0; j < KC; ++j) t[j][i] = 0.0;
+    }
+#pragma unroll 1
+    for (int pass = 0; pass < 2; ++pass) {
+        const double* c = coef;
+#pragma unroll 1
+        for (int k = 0; k < g.K; ++k) {
+            int dr, dc;
+            star_tap(k, dr, dc);
+            const int xx = x + dc;
+            long long off[NOV_PIX];
+            bool ok[NOV_PIX];
+#pragma unroll
+            for (int i = 0; i < NOV_PIX; ++i) {
+                const int yy = y + i + dr;
+                ok[i] = xx >= 0 && xx < a.cw && yy >= 0 && yy < a.ch;
+                off[i] = ok[i] ? (long long)yy * a.pitch + xx : 0;
+            }
+#pragma unroll 1
+            for (int p = 0; p < nch; ++p, c += KC + 1) {
+                const uint8_t* plane = a.planes + (long long)p * a.plane_stride;
+                double xv[NOV_PIX];   // v_f
+#pragma unroll
+                for (int i = 0; i < NOV_PIX; ++i) xv[i] = ok[i] ? u8_to_double(__ldg(plane + off[i])) : -1.0;
+                if (pass == 0) {
+#pragma unroll
+                    for (int j = 0; j < KC; ++j) {
+                        const double cj = c[j];
+#pragma unroll
+                        for (int i = 0; i < NOV_PIX; ++i) t[j][i] = fma(xv[i], cj, t[j][i]);
+                    }
+                } else {
+                    double r[NOV_PIX];
+                    const double mu = c[KC];
+#pragma unroll
+                    for (int i = 0; i < NOV_PIX; ++i) r[i] = mu;
+#pragma unroll
+                    for (int j = 0; j < KC; ++j) {
+                        const double cj = c[j];
+#pragma unroll
+                        for (int i = 0; i < NOV_PIX; ++i) r[i] = fma(t[j][i], cj, r[i]);
+                    }
+#pragma unroll
+                    for (int i = 0; i < NOV_PIX; ++i) err[i] += fabs(fma(xv[i], 1.0 / 255.0, -r[i]));
+                }
+            }
+        }
+        if (pass == 0) {
+#pragma unroll
+            for (int j = 0; j < KC; ++j)
+#pragma unroll
+                for (int i = 0; i < NOV_PIX; ++i) t[j][i] = __dsub_rn(__ddiv_rn(t[j][i], 255.0), mdc[j]);
+        }
+    }
+}
+
+__device__ __forceinline__ void pca_l1_error_k(int k, const NoveltyArgs& a, const double* coef, const double* mdc,
+                                               int x, int y, double (&err)[NOV_PIX]) {
+    switch (k) {
+        case 1: pca_l1_error<1>(a, coef, mdc, x, y, err); break;
+        case 2: pca_l1_error<2>(a, coef, mdc, x, y, err); break;
+        case 3: pca_l1_error<3>(a, coef, mdc, x, y, err); break;
+        case 4: pca_l1_error<4>(a, coef, mdc, x, y, err); break;
+        case 5: pca_l1_error<5>(a, coef, mdc, x, y, err); break;
+        case 6: pca_l1_error<6>(a, coef, mdc, x, y, err); break;
+        case 7: pca_l1_error<7>(a, coef, mdc, x, y, err); break;
+        default: pca_l1_error<8>(a, coef, mdc, x, y, err); break;
+    }
+}
+
+__global__ void __launch_bounds__(NTHREADS) novelty_kernel(const NoveltyArgs a) {
+    extern __shared__ __align__(16) double nsm[];
+    const double* c0 = a.coef0;
+    const double* c1 = a.coef1;
+    if (a.staged) {                                       // model state only: overlaps K0's tail under PDL
+        const int n0 = (a.k0 + 1) * a.g.F, n1 = a.blend ? (a.k1 + 1) * a.g.F : 0;
+        double* s0 = nsm;
+        double* s1 = s0 + n0;
+        for (int i = threadIdx.x; i < n0; i += blockDim.x) s0[i] = a.coef0[i];
+        for (int i = threadIdx.x; i < n1; i += blockDim.x) s1[i] = a.coef1[i];
+        c0 = s0;
+        c1 = s1;
+    }
+    grid_dependency_wait();     // K0's planes are complete and visible (and, since K0 waits too, everything before K0)
+    grid_launch_dependents();
+    __syncthreads();
+    const int tiles_x = (a.cw + NOV_TW - 1) / NOV_TW, tiles_y = (a.rows + NOV_TH - 1) / NOV_TH;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int tile = blockIdx.x; tile < tiles_x * tiles_y; tile += gridDim.x) {
+        const int x = (tile % tiles_x) * NOV_TW + lane;
+        const int y = a.row0 + (tile / tiles_x) * NOV_TH + warp * NOV_PIX;
+        double e[NOV_PIX];
+        pca_l1_error_k(a.k0, a, c0, a.mdc0, x, y, e);
+        if (a.blend) {
+            double e1[NOV_PIX];
+            pca_l1_error_k(a.k1, a, c1, a.mdc1, x, y, e1);
+#pragma unroll
+            for (int i = 0; i < NOV_PIX; ++i) e[i] = blend2(e[i], e1[i], a.w0, a.w1);
+        }
+        if (x < a.cw) {
+#pragma unroll
+            for (int i = 0; i < NOV_PIX; ++i)
+                if (y + i < a.row0 + a.rows) a.out[(size_t)(y + i) * a.cw + x] = e[i];
+        }
+    }
+}
 
 // K2 -----------------------------------------------------------------------------
 // score = f32( (acc/area) * (1-w) + prior * w ) > 0.5 (:241-242), acc being the
@@ -32,8 +193,9 @@ struct PixelScorer {
     DevForest f0, f1;
     int depth, blend;
     double w0, w1;
-    int novelty;
+    int novelty;               // rank-1 novelty term, recomputed by ps_novelty
     DevPCA pca0, pca1;
+    const double* nov_map;     // [ch*cw] novelty_kernel's blended error (PCAs of rank >= 2), or nullptr
 };
 
 // the tile byte offset a node carries -> the plane sample of pixel (x, y) it means (0 outside the crop, like the TMA fill)
@@ -95,7 +257,9 @@ __device__ double ps_contribution(const PixelScorer& s, int x, int y, double thr
     double p = ps_forest(s, s.f0, x, y);
     if (s.blend) p = blend2(p, ps_forest(s, s.f1, x, y), s.w0, s.w1);
     double e = 0.0;
-    if (s.novelty) {
+    if (s.nov_map) {
+        e = s.nov_map[(size_t)y * s.cw + x];        // the value K1 read: identical bits
+    } else if (s.novelty) {
         e = ps_novelty(s, s.pca0, x, y);
         if (s.blend) e = blend2(e, ps_novelty(s, s.pca1, x, y), s.w0, s.w1);
     }

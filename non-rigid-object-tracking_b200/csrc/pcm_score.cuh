@@ -6,6 +6,7 @@
 //  K0 planes_kernel       BGR crop -> planar HSV/LAB/BGR planes + validity plane (cvtColor :294-309)
 //  K1 score_kernel        TMA tiles of those planes (smem, halo) -> star taps -> forest(s)
 //                         [-> PCA novelty error] [-> temporal blend] -> P(fg) f64 [, err f64]
+//                         (a PCA of two or more components: the error map of novelty_kernel, pcm_kernels.cuh)
 //                         replaces cvtColor + getFeatures + X/255 + predict_proba + PCA
 //                         (reference maskers/pixel_classification.py:53-63, :80-95)
 //                         epilogue: per-label sums / areas (np.unique :97 + first loop of
@@ -340,10 +341,12 @@ struct ScoreArgs {
     int blend;                       // 0/1: f1 (and pca1) valid
     double w0, w1;                   // np.average weights
     int novelty;                     // 0/1
-    DevPCA pca0, pca1;
+    DevPCA pca0, pca1;               // rank-1 PCAs of the in-line pass (unused when nov_in is set)
     double* p1_out;                  // [ch*cw], or NULL: not kept (only pcm_set_debug keeps the per-pixel maps; K2's exact
     double* sa_out;                  // path recomputes the few pixels it needs).  sa_out: novelty only
     SegAcc seg;                      // per-label accumulators (epilogue)
+    const double* nov_in;            // novelty on and a PCA of two or more components: [ch*cw] blended error computed by
+                                     // novelty_kernel, which K1 reads instead of running its rank-1 pass; else NULL
 };
 
 // One forest over the thread's PIX_PER_THREAD pixels; leaf fractions are added in
@@ -564,7 +567,7 @@ template <bool FOREST_SMEM, int DEPTH, int PIX_PER_THREAD>
 __global__ void __launch_bounds__(NTHREADS, PCM_MIN_CTAS) score_kernel(const __grid_constant__ CUtensorMap tmap, const ScoreArgs a) {
     extern __shared__ __align__(128) uint8_t smem[];
     const Geom& g = a.g;
-    const ScoreSmem L = score_smem_layout(g, a.f0, a.f1, a.blend != 0, a.novelty != 0, FOREST_SMEM);
+    const ScoreSmem L = score_smem_layout(g, a.f0, a.f1, a.blend != 0, a.novelty != 0 && !a.nov_in, FOREST_SMEM);
     constexpr int TILE_H = ROW_GROUPS * PIX_PER_THREAD;     // rows per tile; a.tiles_y = ceil(ch / TILE_H)
     const int PH = TILE_H + 2 * g.n;                        // rows of a TMA box (tile + vertical halo)
     const uint32_t tile_bytes = align_up(g.n_planes * g.PS, 128);
@@ -612,7 +615,7 @@ __global__ void __launch_bounds__(NTHREADS, PCM_MIN_CTAS) score_kernel(const __g
     // holds feature f = (p / 3) * 3K + 3k + p % 3 (:272), next to the feature's byte offset inside the tile
     const double *p0c = nullptr, *p0c255 = nullptr, *p0m = nullptr, *p1c = nullptr, *p1c255 = nullptr, *p1m = nullptr;
     const uint32_t* noff = reinterpret_cast<const uint32_t*>(smem + L.nov_off);
-    if (a.novelty) {
+    if (a.novelty && !a.nov_in) {
         const int nch = 3 * g.n_spaces;
         double* d0 = reinterpret_cast<double*>(smem + L.pca0);
         double* d1 = reinterpret_cast<double*>(smem + L.pca1);
@@ -695,7 +698,13 @@ __global__ void __launch_bounds__(NTHREADS, PCM_MIN_CTAS) score_kernel(const __g
         double e[PIX_PER_THREAD];
 #pragma unroll
         for (int i = 0; i < PIX_PER_THREAD; ++i) e[i] = 0.0;
-        if (a.novelty) {
+        if (a.novelty && a.nov_in) {
+#pragma unroll
+            for (int i = 0; i < PIX_PER_THREAD; ++i) {
+                const int oy = ty0 + row0 + i;
+                if (ox < a.cw && oy < a.ch) e[i] = __ldg(a.nov_in + (size_t)oy * a.cw + ox);
+            }
+        } else if (a.novelty) {
             // no tap of this thread's pixels can fall outside the crop: the validity plane need not be read
             const bool interior = ox >= g.n && ox + g.n < a.cw && ty0 + row0 >= g.n && ty0 + row0 + PIX_PER_THREAD - 1 + g.n < a.ch;
             auto run = [&](const double* c, const double* c255, const double* mu, double mdc, double (&out)[PIX_PER_THREAD]) {
@@ -729,7 +738,7 @@ __global__ void __launch_bounds__(NTHREADS, PCM_MIN_CTAS) score_kernel(const __g
                 const size_t o = (size_t)oy * a.cw + ox;
                 if (a.p1_out) {
                     a.p1_out[o] = p[i];
-                    if (a.novelty) a.sa_out[o] = e[i];
+                    if (a.novelty && !a.nov_in) a.sa_out[o] = e[i];
                 }
                 if (l < 0 || l >= a.seg.n_labels) { *a.seg.err = 1; l = -1; }
             }

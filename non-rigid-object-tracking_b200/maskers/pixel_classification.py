@@ -94,6 +94,16 @@ class PixelClassificationNonRigidMasker(Masker):
         self._prior_fn = fn
 
     # -- training (reference :166-228) -------------------------------------------
+    @staticmethod
+    def _n_components(params):
+        """params.n_components as the native novelty path takes it: an integer in 1..PCM_MAX_PCA_COMPONENTS.  A fraction
+        of explained variance (0 < n < 1) or "mle", which scikit-learn would also accept, is refused."""
+        k = params.get("n_components")
+        if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)) or not 1 <= k <= capi.MAX_PCA_COMPONENTS:
+            raise ValueError("n_components must be an integer between 1 and %d (PCM_MAX_PCA_COMPONENTS), got %r"
+                             % (capi.MAX_PCA_COMPONENTS, k))
+        return int(k)
+
     def _rows(self, frame, rect):
         """Raw feature rows of a rectangle, int16 in -1..255; the reference trains on these / 255 (:54-55, :192-196)."""
         return self.native.gather_features(frame, rect)
@@ -102,6 +112,7 @@ class PixelClassificationNonRigidMasker(Masker):
         if bbox_roni is None:
             raise ValueError("bbox_roni is required (the reference opens a GUI selector here, :287)")
         params = self.config["params"]
+        n_components = self._n_components(params) if params["novelty_detection"] else None
         cache = self.model_cache if self.model_cache is not None and self.cache_tag is not None else None
 
         def cached(key, make):
@@ -154,15 +165,11 @@ class PixelClassificationNonRigidMasker(Masker):
         if params["novelty_detection"]:
             def make_pca():
                 if gpu:
-                    if params["n_components"] != 1:
-                        raise ValueError("the native novelty path supports n_components == 1 (config.yaml:27)")
                     if not resident():
                         train.upload_rows(self.native, Xi, labels, rows_id)
-                    return train.fit_pca(self.native, rows_id, len(labels), Xi.shape[1])
+                    return train.fit_pca(self.native, rows_id, len(labels), Xi.shape[1], n_components)
                 X = Xi.astype(np.float64) / 255
-                pca = PCA(n_components=params["n_components"]).fit(X[labels == 1])
-                if pca.components_.shape[0] != 1:
-                    raise ValueError("the native novelty path supports n_components == 1 (config.yaml:27)")
+                pca = PCA(n_components=n_components).fit(X[labels == 1])
                 residual = np.sum(np.sqrt(np.power(X - pca.inverse_transform(pca.transform(X)), 2)), axis=1)
                 return pca, np.percentile(residual, 90)
             with stages.stage("fit_pca"):
@@ -173,7 +180,7 @@ class PixelClassificationNonRigidMasker(Masker):
         with stages.stage("export_model"):
             m = self.native.add_forest(n_frame, clf, n_trees)
             if pca is not None:
-                self.native.set_novelty(m, pca.mean_, pca.components_[0])
+                self.native.set_novelty(m, pca.mean_, pca.components_)
         self.models.append({"n_frame": n_frame, "model": clf, "n_trees": n_trees})
         self.novelty_det.append({"n_frame": n_frame, "model": pca, "threshold": threshold})
         return bbox_roni

@@ -67,6 +67,7 @@ def load_library():
         "pcm_num_features": (I, [P]),
         "pcm_add_model": (I, [P, I, I, P, P, P, P, P, P, C.POINTER(I)]),
         "pcm_set_novelty": (I, [P, I, P, P, I]),
+        "pcm_set_novelty_k": (I, [P, I, P, P, I, I]),
         "pcm_num_models": (I, [P]),
         "pcm_crop_rect": (I, [P, I, I, P]),
         "pcm_update": (I, [P, P, I, I, L, P, P, I, P, C.POINTER(UpdateParams), P, L, L]),
@@ -86,6 +87,7 @@ def load_library():
         "pcm_fit_rows": (I, [P, P, P, I, I, C.c_longlong]),
         "pcm_pca_moments": (I, [P, C.c_longlong, P, P, P]),
         "pcm_pca_residuals": (I, [P, C.c_longlong, P, P, P]),
+        "pcm_pca_residuals_k": (I, [P, C.c_longlong, P, P, I, P]),
         "pcm_fit_forest": (I, [P, P, P, I, I, C.c_longlong, I, I, I, P, P, I, P, P, P, P, P, P, P]),
         "pcm_run_frames": (I, [P, I, I, L, P, L, P, I]),
         "pcm_prior_device": (I, [P, P, P, I, P, L, I, I, P, P, I, P, I, I, I, P]),
@@ -116,14 +118,17 @@ def load_library():
 
 EXPORTED_SYMBOLS = [
     "pcm_abi_version", "pcm_last_error", "pcm_create", "pcm_destroy", "pcm_set_stream", "pcm_use_own_stream", "pcm_get_stream", "pcm_synchronize",
-    "pcm_set_features", "pcm_num_features", "pcm_add_model", "pcm_set_novelty", "pcm_num_models", "pcm_crop_rect",
+    "pcm_set_features", "pcm_num_features", "pcm_add_model", "pcm_set_novelty", "pcm_set_novelty_k", "pcm_num_models", "pcm_crop_rect",
     "pcm_update", "pcm_update_device", "pcm_iou", "pcm_iou_device", "pcm_quickshift", "pcm_quickshift_device", "pcm_quickshift_device_batch", "pcm_felzenszwalb", "pcm_felzenszwalb_graph", "pcm_slic",
-    "pcm_prior_device", "pcm_run_frames", "pcm_fit_forest", "pcm_fit_rows", "pcm_pca_moments", "pcm_pca_residuals", "pcm_convert", "pcm_gather_features",
+    "pcm_prior_device", "pcm_run_frames", "pcm_fit_forest", "pcm_fit_rows", "pcm_pca_moments", "pcm_pca_residuals", "pcm_pca_residuals_k", "pcm_convert", "pcm_gather_features",
     "pcm_set_debug", "pcm_debug_last", "pcm_debug_tables", "pcm_launch_count", "pcm_transfer_bytes", "pcm_set_label_cache", "pcm_profile_enable", "pcm_profile_read",
     "pcm_host_register", "pcm_host_unregister",
 ]
 
 KERNEL_NAMES = ["score", "segment_reduce", "segment_decide", "segment_resolve", "mask_dilate", "iou", "planes"]
+# every profile id of pcm_profile_read: KERNEL_NAMES plus the novelty kernel of PCAs with two or more components (id 7)
+ALL_KERNEL_NAMES = KERNEL_NAMES + ["novelty"]
+MAX_PCA_COMPONENTS = 8                 # PCM_MAX_PCA_COMPONENTS
 
 
 def _ptr(a):
@@ -350,8 +355,18 @@ class Handle:
         return self.add_model_arrays(n_frame, arrays)
 
     def set_novelty(self, model_index, mean, component):
+        """PCA novelty detector of a model: `component` is components_[0] (1-D, pcm_set_novelty) or the whole
+        components_ array, shape (n_components, F) (pcm_set_novelty_k)."""
         mean = np.ascontiguousarray(mean, np.float64).reshape(-1)
-        comp = np.ascontiguousarray(component, np.float64).reshape(-1)
+        comp = np.asarray(component, np.float64)
+        if comp.ndim == 2:
+            comp = np.ascontiguousarray(comp)
+            if comp.shape[1] != len(mean):
+                raise ValueError("components has %d features, mean %d" % (comp.shape[1], len(mean)))
+            self._check(self.lib.pcm_set_novelty_k(self._h, int(model_index), _ptr(mean), _ptr(comp), comp.shape[0],
+                                                   len(mean)))
+            return
+        comp = np.ascontiguousarray(comp).reshape(-1)
         self._check(self.lib.pcm_set_novelty(self._h, int(model_index), _ptr(mean), _ptr(comp), len(mean)))
 
     # -- hot path -------------------------------------------------------------
@@ -505,12 +520,14 @@ class Handle:
     def profile_enable(self, on=True):
         self._check(self.lib.pcm_profile_enable(self._h, int(bool(on))))
 
-    def profile_read(self, reset=False):
-        """{kernel name: (total ms, launches)} measured with CUDA events on the handle's stream."""
-        ms = np.zeros(len(KERNEL_NAMES), np.float64)
-        cnt = np.zeros(len(KERNEL_NAMES), np.int64)
-        self._check(self.lib.pcm_profile_read(self._h, _ptr(ms), _ptr(cnt), len(KERNEL_NAMES), int(bool(reset))))
-        return {k: (float(ms[i]), int(cnt[i])) for i, k in enumerate(KERNEL_NAMES)}
+    def profile_read(self, reset=False, names=None):
+        """{kernel name: (total ms, launches)} measured with CUDA events on the handle's stream; `names`: the first
+        len(names) profile ids (default KERNEL_NAMES; ALL_KERNEL_NAMES includes the novelty kernel)."""
+        names = KERNEL_NAMES if names is None else names
+        ms = np.zeros(len(names), np.float64)
+        cnt = np.zeros(len(names), np.int64)
+        self._check(self.lib.pcm_profile_read(self._h, _ptr(ms), _ptr(cnt), len(names), int(bool(reset))))
+        return {k: (float(ms[i]), int(cnt[i])) for i, k in enumerate(names)}
 
     def tables(self):
         gamma = np.empty(256, np.uint16)

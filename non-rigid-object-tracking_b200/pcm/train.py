@@ -107,12 +107,12 @@ def fit_forest(handle, X, y, n_estimators, max_depth, random_state=42, rows_id=0
 
 
 class GpuPCA:
-    """The two attributes of sklearn.decomposition.PCA(n_components=1) the masker reads."""
+    """The attributes of sklearn.decomposition.PCA(n_components=k) the masker reads: mean_ [F], components_ [k, F]."""
 
-    def __init__(self, mean, component):
+    def __init__(self, mean, components):
         self.mean_ = mean
-        self.components_ = component.reshape(1, -1)
-        self.n_components = 1
+        self.components_ = components.reshape(-1, len(mean))
+        self.n_components = self.components_.shape[0]
 
 
 def upload_rows(handle, X, y, rows_id):
@@ -122,14 +122,33 @@ def upload_rows(handle, X, y, rows_id):
                                           X.shape[0], X.shape[1], int(rows_id)))
 
 
-def fit_pca(handle, rows_id, n_rows, n_features):
-    """PCA(n_components=1).fit(X[labels == 1]) and the 90th percentile of the L1 reconstruction error of every
-    training row (reference :203-213) from the rows resident on `handle` under rows_id.
-    Mirrors sklearn/decomposition/_pca.py `_fit_full` with the covariance_eigh solver (the one scikit-learn 1.9
-    picks for these shapes): C = X^T X - n mean mean^T, C /= n - 1, leading eigenvector of C, sign chosen so that its
-    largest-magnitude entry is positive (svd_flip, u_based_decision=False).  The Gram matrix is accumulated on the
-    device over the raw integer feature values (exact) and scaled by 1/255^2 here.  Returns (GpuPCA, threshold)."""
+def pca_from_moments(gram, sums, n_class1, k=1):
+    """(mean [F], components [k, F]) of PCA(n_components=k).fit(X / 255) from the moments pcm_pca_moments returns for the
+    class-1 rows X (gram = X^T X and sums over the raw integer values, n_class1 rows), computed the way scikit-learn
+    1.9's covariance_eigh solver computes them (decomposition/_pca.py `_fit_full`): C = X^T X - n mean mean^T,
+    C /= n - 1, eigenvectors of C by decreasing eigenvalue, each with the sign that makes its largest-magnitude entry
+    positive (svd_flip, u_based_decision=False).  The Gram matrix is scaled by 1/255^2 here."""
+    m = int(n_class1)
+    mean = sums / 255.0 / m
+    Cov = gram / (255.0 * 255.0)
+    Cov -= m * mean.reshape(-1, 1) * mean.reshape(1, -1)
+    Cov /= m - 1
+    _, vecs = np.linalg.eigh(Cov)
+    comps = np.ascontiguousarray(vecs[:, ::-1][:, :k].T)
+    rows = np.arange(k)
+    signs = np.where(comps[rows, np.argmax(np.abs(comps), axis=1)] < 0, -1.0, 1.0)
+    comps *= signs[:, None]
+    return mean, comps
+
+
+def fit_pca(handle, rows_id, n_rows, n_features, n_components=1):
+    """PCA(n_components).fit(X[labels == 1]) and the 90th percentile of the L1 reconstruction error of every
+    training row (reference :203-213) from the rows resident on `handle` under rows_id: the Gram matrix is accumulated
+    on the device over the raw integer feature values (exact), the eigen-decomposition is `pca_from_moments`, the
+    residuals are pcm_pca_residuals_k.  Like scikit-learn, n_components may not exceed min(class-1 rows, features).
+    Returns (GpuPCA, threshold)."""
     F = n_features
+    k = int(n_components)
     G = np.empty((F, F), np.float64)
     S = np.empty(F, np.float64)
     n1 = np.zeros(1, np.int64)
@@ -138,14 +157,10 @@ def fit_pca(handle, rows_id, n_rows, n_features):
     m = int(n1[0])
     if m < 2:
         raise ValueError("PCA needs at least two foreground rows")
-    mean = S / 255.0 / m
-    Cov = G / (255.0 * 255.0)
-    Cov -= m * mean.reshape(-1, 1) * mean.reshape(1, -1)
-    Cov /= m - 1
-    _, vecs = np.linalg.eigh(Cov)
-    comp = np.ascontiguousarray(vecs[:, -1])
-    if comp[np.argmax(np.abs(comp))] < 0:
-        comp = -comp
+    if not 1 <= k <= min(m, F):
+        raise ValueError("n_components=%r must be between 1 and min(n_samples, n_features)=%d with svd_solver='covariance_eigh'"
+                         % (n_components, min(m, F)))
+    mean, comps = pca_from_moments(G, S, m, k)
     err = np.empty(n_rows, np.float64)
-    handle._check(handle.lib.pcm_pca_residuals(handle._h, int(rows_id), p(mean), p(comp), p(err)))
-    return GpuPCA(mean, comp), float(np.percentile(err, 90))
+    handle._check(handle.lib.pcm_pca_residuals_k(handle._h, int(rows_id), p(mean), p(comps), k, p(err)))
+    return GpuPCA(mean, comps), float(np.percentile(err, 90))
