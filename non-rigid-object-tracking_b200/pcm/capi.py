@@ -40,6 +40,58 @@ class FrameJob(C.Structure):
                 ("d_counts", C.c_void_p)]
 
 
+P, I, L, D = C.c_void_p, C.c_int, C.c_int64, C.c_double
+# (restype, argtypes) of every entry point of include/pcm_b200.h
+_SIGNATURES = {
+    "pcm_abi_version": (I, []),
+    "pcm_last_error": (C.c_char_p, []),
+    "pcm_create": (I, [I, C.POINTER(P)]),
+    "pcm_destroy": (None, [P]),
+    "pcm_set_stream": (I, [P, P]),
+    "pcm_use_own_stream": (I, [P]),
+    "pcm_get_stream": (I, [P, C.POINTER(P)]),
+    "pcm_synchronize": (I, [P]),
+    "pcm_set_features": (I, [P, I, I, P]),
+    "pcm_num_features": (I, [P]),
+    "pcm_add_model": (I, [P, I, I, P, P, P, P, P, P, C.POINTER(I)]),
+    "pcm_set_novelty": (I, [P, I, P, P, I]),
+    "pcm_set_novelty_k": (I, [P, I, P, P, I, I]),
+    "pcm_num_models": (I, [P]),
+    "pcm_crop_rect": (I, [P, I, I, P]),
+    "pcm_update": (I, [P, P, I, I, L, P, P, I, P, C.POINTER(UpdateParams), P, L, L]),
+    "pcm_update_device": (I, [P, P, I, I, L, P, P, I, P, C.POINTER(UpdateParams), P, L]),
+    "pcm_iou": (I, [P, P, L, L, P, L, I, I, I, P]),
+    "pcm_iou_device": (I, [P, P, L, P, L, I, I, I, P]),
+    "pcm_quickshift": (I, [P, P, I, I, L, P, D, D, D, P, P, C.POINTER(I)]),
+    "pcm_quickshift_device": (I, [P, P, I, I, L, P, D, D, D, P, P, C.POINTER(I)]),
+    "pcm_quickshift_device_batch": (I, [P, I, P, L, P, I, I, L, P, D, D, D, P, P, P, P]),
+    "pcm_felzenszwalb": (I, [P, I, I, L, P, D, D, I, P, I, P, C.POINTER(I)]),
+    "pcm_felzenszwalb_graph": (I, [I, I, P, P, P, D, I, P, C.POINTER(I)]),
+    "pcm_slic": (I, [P, I, I, L, P, I, D, D, P, I, I, I, P, C.POINTER(I)]),
+    "pcm_host_register": (I, [P, C.c_size_t]),
+    "pcm_host_unregister": (I, [P]),
+    "pcm_run_frames": (I, [P, I, I, L, P, L, P, I]),
+    "pcm_prior_device": (I, [P, P, P, I, P, L, I, I, P, P, I, P, I, I, I, P]),
+    "pcm_fit_rows": (I, [P, P, P, I, I, C.c_longlong]),
+    "pcm_pca_moments": (I, [P, C.c_longlong, P, P, P]),
+    "pcm_pca_residuals": (I, [P, C.c_longlong, P, P, P]),
+    "pcm_pca_residuals_k": (I, [P, C.c_longlong, P, P, I, P]),
+    "pcm_fit_forest": (I, [P, P, P, I, I, C.c_longlong, I, I, I, P, P, I, P, P, P, P, P, P, P]),
+    "pcm_convert": (I, [P, P, I, I, L, I, P, L]),
+    "pcm_gather_features": (I, [P, P, I, I, L, P, P]),
+    "pcm_set_debug": (I, [P, I]),
+    "pcm_debug_last": (I, [P, P, P, P, P, P, P]),
+    "pcm_debug_tables": (I, [P, P, P, P, P]),
+    "pcm_launch_count": (L, [P]),
+    "pcm_transfer_bytes": (I, [P, P]),
+    "pcm_set_label_cache": (I, [P, I]),
+    "pcm_profile_enable": (I, [P, I]),
+    "pcm_profile_read": (I, [P, P, P, I, I]),
+}
+del P, I, L, D
+EXPORTED_SYMBOLS = list(_SIGNATURES)
+
+
 def library_path():
     return _build.LIB
 
@@ -53,60 +105,7 @@ def load_library():
     if _build.needs_build():
         _build.build()
     lib = C.CDLL(_build.LIB)
-    P, I, L, D = C.c_void_p, C.c_int, C.c_int64, C.c_double
-    sig = {
-        "pcm_abi_version": (I, []),
-        "pcm_last_error": (C.c_char_p, []),
-        "pcm_create": (I, [I, C.POINTER(P)]),
-        "pcm_destroy": (None, [P]),
-        "pcm_set_stream": (I, [P, P]),
-        "pcm_use_own_stream": (I, [P]),
-        "pcm_get_stream": (I, [P, C.POINTER(P)]),
-        "pcm_synchronize": (I, [P]),
-        "pcm_set_features": (I, [P, I, I, P]),
-        "pcm_num_features": (I, [P]),
-        "pcm_add_model": (I, [P, I, I, P, P, P, P, P, P, C.POINTER(I)]),
-        "pcm_set_novelty": (I, [P, I, P, P, I]),
-        "pcm_set_novelty_k": (I, [P, I, P, P, I, I]),
-        "pcm_num_models": (I, [P]),
-        "pcm_crop_rect": (I, [P, I, I, P]),
-        "pcm_update": (I, [P, P, I, I, L, P, P, I, P, C.POINTER(UpdateParams), P, L, L]),
-        "pcm_update_device": (I, [P, P, I, I, L, P, P, I, P, C.POINTER(UpdateParams), P, L]),
-        "pcm_iou": (I, [P, P, L, L, P, L, I, I, I, P]),
-        "pcm_iou_device": (I, [P, P, L, P, L, I, I, I, P]),
-        "pcm_quickshift": (I, [P, P, I, I, L, P, D, D, D, P, P, C.POINTER(I)]),
-        "pcm_quickshift_device": (I, [P, P, I, I, L, P, D, D, D, P, P, C.POINTER(I)]),
-        "pcm_quickshift_device_batch": (I, [P, I, P, L, P, I, I, L, P, D, D, D, P, P, P, P]),
-        "pcm_felzenszwalb": (I, [P, I, I, L, P, D, D, I, P, I, P, C.POINTER(I)]),
-        "pcm_felzenszwalb_graph": (I, [I, I, P, P, P, D, I, P, C.POINTER(I)]),
-        "pcm_slic": (I, [P, I, I, L, P, I, D, D, P, I, I, I, P, C.POINTER(I)]),
-        "pcm_host_register": (I, [P, C.c_size_t]),
-        "pcm_host_unregister": (I, [P]),
-        "pcm_run_frames": (I, [P, I, I, L, P, L, P, I]),
-        "pcm_prior_device": (I, [P, P, P, I, P, L, I, I, P, P, I, P, I, I, I, P]),
-        "pcm_fit_rows": (I, [P, P, P, I, I, C.c_longlong]),
-        "pcm_pca_moments": (I, [P, C.c_longlong, P, P, P]),
-        "pcm_pca_residuals": (I, [P, C.c_longlong, P, P, P]),
-        "pcm_pca_residuals_k": (I, [P, C.c_longlong, P, P, I, P]),
-        "pcm_fit_forest": (I, [P, P, P, I, I, C.c_longlong, I, I, I, P, P, I, P, P, P, P, P, P, P]),
-        "pcm_run_frames": (I, [P, I, I, L, P, L, P, I]),
-        "pcm_prior_device": (I, [P, P, P, I, P, L, I, I, P, P, I, P, I, I, I, P]),
-        "pcm_fit_rows": (I, [P, P, P, I, I, C.c_longlong]),
-        "pcm_pca_moments": (I, [P, C.c_longlong, P, P, P]),
-        "pcm_pca_residuals": (I, [P, C.c_longlong, P, P, P]),
-        "pcm_fit_forest": (I, [P, P, P, I, I, C.c_longlong, I, I, I, P, P, I, P, P, P, P, P, P, P]),
-        "pcm_convert": (I, [P, P, I, I, L, I, P, L]),
-        "pcm_gather_features": (I, [P, P, I, I, L, P, P]),
-        "pcm_set_debug": (I, [P, I]),
-        "pcm_debug_last": (I, [P, P, P, P, P, P, P]),
-        "pcm_debug_tables": (I, [P, P, P, P, P]),
-        "pcm_launch_count": (L, [P]),
-        "pcm_transfer_bytes": (I, [P, P]),
-        "pcm_set_label_cache": (I, [P, I]),
-        "pcm_profile_enable": (I, [P, I]),
-        "pcm_profile_read": (I, [P, P, P, I, I]),
-    }
-    for name, (res, args) in sig.items():
+    for name, (res, args) in _SIGNATURES.items():
         fn = getattr(lib, name)
         fn.restype = res
         fn.argtypes = args
@@ -115,15 +114,6 @@ def load_library():
     _lib = lib
     return lib
 
-
-EXPORTED_SYMBOLS = [
-    "pcm_abi_version", "pcm_last_error", "pcm_create", "pcm_destroy", "pcm_set_stream", "pcm_use_own_stream", "pcm_get_stream", "pcm_synchronize",
-    "pcm_set_features", "pcm_num_features", "pcm_add_model", "pcm_set_novelty", "pcm_set_novelty_k", "pcm_num_models", "pcm_crop_rect",
-    "pcm_update", "pcm_update_device", "pcm_iou", "pcm_iou_device", "pcm_quickshift", "pcm_quickshift_device", "pcm_quickshift_device_batch", "pcm_felzenszwalb", "pcm_felzenszwalb_graph", "pcm_slic",
-    "pcm_prior_device", "pcm_run_frames", "pcm_fit_forest", "pcm_fit_rows", "pcm_pca_moments", "pcm_pca_residuals", "pcm_pca_residuals_k", "pcm_convert", "pcm_gather_features",
-    "pcm_set_debug", "pcm_debug_last", "pcm_debug_tables", "pcm_launch_count", "pcm_transfer_bytes", "pcm_set_label_cache", "pcm_profile_enable", "pcm_profile_read",
-    "pcm_host_register", "pcm_host_unregister",
-]
 
 KERNEL_NAMES = ["score", "segment_reduce", "segment_decide", "segment_resolve", "mask_dilate", "iou", "planes"]
 # every profile id of pcm_profile_read: KERNEL_NAMES plus the novelty kernel of PCAs with two or more components (id 7)
@@ -161,6 +151,17 @@ def crop_rect(bbox, frame_h, frame_w):
     return tuple(out)
 
 
+def _gaussian_weights(sigma):
+    """(weights, radius) of the 1-D Gaussian filter scipy.ndimage applies for `sigma` (truncated at 4 sigma);
+    (None, 0) when sigma is not positive."""
+    if not sigma > 0:
+        return None, 0
+    radius = int(4.0 * float(sigma) + 0.5)
+    x = np.arange(-radius, radius + 1)
+    phi = np.exp(-0.5 / (sigma * sigma) * x ** 2)
+    return np.ascontiguousarray(phi / phi.sum(), np.float64), radius
+
+
 def felzenszwalb(frame, rect, scale=100, sigma=0.5, min_size=50):
     """Felzenszwalb-Huttenlocher segmentation of the crop `rect` (defaults = the reference's call,
     pixel_classification.py:73).  Host code in the library; returns (labels int32 HxW, n_labels).
@@ -169,12 +170,7 @@ def felzenszwalb(frame, rect, scale=100, sigma=0.5, min_size=50):
     if frame.dtype != np.uint8 or frame.ndim != 3 or frame.shape[2] != 3 or frame.strides[2] != 1 or frame.strides[1] != 3:
         frame = np.ascontiguousarray(frame, np.uint8)
     r = (C.c_int * 4)(*[int(v) for v in rect])
-    kernel, radius = None, 0
-    if sigma > 0:
-        radius = int(4.0 * float(sigma) + 0.5)
-        x = np.arange(-radius, radius + 1)
-        phi = np.exp(-0.5 / (sigma * sigma) * x ** 2)
-        kernel = np.ascontiguousarray(phi / phi.sum(), np.float64)
+    kernel, radius = _gaussian_weights(sigma)
     out = np.empty((rect[3], rect[2]), np.int32)
     n = C.c_int(0)
     rc = lib.pcm_felzenszwalb(_ptr(frame), frame.shape[0], frame.shape[1], frame.strides[0], r, float(scale), float(sigma),
@@ -191,12 +187,7 @@ def slic(frame, rect, n_segments=250, compactness=10.0, sigma=1.0, max_iter=10, 
     if frame.dtype != np.uint8 or frame.ndim != 3 or frame.shape[2] != 3 or frame.strides[2] != 1 or frame.strides[1] != 3:
         frame = np.ascontiguousarray(frame, np.uint8)
     r = (C.c_int * 4)(*[int(v) for v in rect])
-    kernel, radius = None, 0
-    if sigma > 0:
-        radius = int(4.0 * float(sigma) + 0.5)
-        x = np.arange(-radius, radius + 1)
-        phi = np.exp(-0.5 / (sigma * sigma) * x ** 2)
-        kernel = np.ascontiguousarray(phi / phi.sum(), np.float64)
+    kernel, radius = _gaussian_weights(sigma)
     out = np.empty((rect[3], rect[2]), np.int32)
     n = C.c_int(0)
     rc = lib.pcm_slic(_ptr(frame), frame.shape[0], frame.shape[1], frame.strides[0], r, int(n_segments), float(compactness),
