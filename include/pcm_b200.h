@@ -141,7 +141,7 @@ int pcm_update(pcm_handle* h, const uint8_t* frame, int frame_h, int frame_w, in
                const pcm_update_params* params,
                uint8_t* mask, int64_t mask_row_stride, int64_t mask_pixel_stride);
 
-/* labels == NULL: continue from the preceding pcm_quickshift on this handle -- the label map
+/* labels == NULL: continue from the preceding pcm_quickshift or pcm_slic_gpu on this handle -- the label map
  * AND the crop pixels are the ones that call left on the device (`frame` and `rect` must be
  * the same as in that call; the frame is not read again).  n_labels is ignored. */
 
@@ -236,6 +236,41 @@ int pcm_felzenszwalb(const uint8_t* frame, int frame_h, int frame_w, int64_t fra
 int pcm_slic(const uint8_t* frame, int frame_h, int frame_w, int64_t frame_stride, const int rect[4], int n_segments,
              double compactness, double sigma, const double* kernel, int kernel_radius, int max_iter, int start_label,
              int32_t* labels_out, int* n_labels_out);
+
+/* pcm_slic on the GPU: the same labels and count as pcm_slic for the same arguments (DESIGN.md §10).  Only rgb2lab may
+ * differ from the host code, by at most 1e-12 on the image the k-means sees, because CUDA's pow / cbrt are not glibc's.
+ * The crop of a HOST frame is staged like pcm_quickshift's, and the label map stays on the device: pcm_update with
+ * labels == NULL (same frame and rect) continues from it.  Synchronous.
+ *   kernel      2 * kernel_radius + 1 Gaussian weights on the host, or NULL to compute them from sigma as pcm_slic does
+ *   labels_out  h*w int32 on the host, or NULL when only the device-resident map is needed
+ * Limits: crop of at most 2^28 pixels; n_segments >= 1, compactness > 0, max_iter >= 0, start_label >= 0. */
+int pcm_slic_gpu(pcm_handle* h, const uint8_t* frame, int frame_h, int frame_w, int64_t frame_stride, const int rect[4],
+                 int n_segments, double compactness, double sigma, const double* kernel, int kernel_radius, int max_iter,
+                 int start_label, int32_t* labels_out, int* n_labels_out);
+
+/* Device variant: d_frame and d_labels_out (h*w int32, may be NULL) are device pointers, `kernel` is on the host; waits
+ * for the stream to return the segment count. */
+int pcm_slic_device(pcm_handle* h, const uint8_t* d_frame, int frame_h, int frame_w, int64_t frame_stride, const int rect[4],
+                    int n_segments, double compactness, double sigma, const double* kernel, int kernel_radius, int max_iter,
+                    int start_label, int32_t* d_labels_out, int* n_labels_out);
+
+/* The SLIC maps of n crops of a device-resident clip in one call, laid out like pcm_quickshift_device_batch's: exactly n
+ * calls of pcm_slic_device without returning to the caller in between. */
+int pcm_slic_device_batch(pcm_handle* h, int n, const uint8_t* d_frames, int64_t frame_bytes, const int32_t* frame_index,
+                          int frame_h, int frame_w, int64_t frame_stride, const int32_t* rects, int n_segments, double compactness,
+                          double sigma, const double* kernel, int kernel_radius, int max_iter, int start_label,
+                          int32_t* d_labels_out, const int64_t* label_offsets, int32_t* n_labels_out);
+
+/* Parity tap: the device connectivity enforcement of pcm_slic_gpu on a caller's centre map `nearest` (width x height int32,
+ * host), with the caller's min_size / max_size (pcm_slic uses (long long)(0.5 s) and (long long)(3 s) for the segment size
+ * s = h*w / n_segments).  labels_out: width*height int32 (host); n_labels_out = largest label + 1. */
+int pcm_slic_connectivity(pcm_handle* h, const int32_t* nearest, int width, int height, long long min_size, long long max_size,
+                          int start_label, int32_t* labels_out, int* n_labels_out);
+
+/* Parity tap: the stage results of the last pcm_slic_gpu / pcm_slic_device on the handle, each h*w pixels of that crop:
+ * smoothed (3 float64 per pixel: /255 and the Gaussian), image (3 float64: rgb2lab / compactness, what the k-means sees),
+ * nearest (int32: the centre map after the last k-means iteration).  NULL skips a stage.  PCM_E_STATE before any SLIC. */
+int pcm_slic_debug_last(pcm_handle* h, double* smoothed, double* image, int32_t* nearest);
 
 /* Parity tap: the cost-ordered merge, union-find and min-size passes of pcm_felzenszwalb on a caller-provided
  * edge list (n_edges edges a[i]-b[i] with non-negative cost[i]; `scale` is the k of k/|C|, already on the scale

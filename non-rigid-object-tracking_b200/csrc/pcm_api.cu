@@ -9,9 +9,12 @@
 #include "pcm_quickshift.cuh"
 #include "pcm_forest_fit.cuh"
 #include "pcm_prior.cuh"
+#include "pcm_slic.cuh"
 #include "pcm_host.h"
 
 #include <cudaTypedefs.h>
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 
 #include <algorithm>
 #include <atomic>
@@ -300,6 +303,14 @@ struct pcm_handle {
     const uint8_t* qs_frame_ptr = nullptr;     // host frame the resident crop was staged from
     int qs_rect[4] = {0, 0, 0, 0};
 
+    // SLIC over-segmentation (pcm_slic_gpu / pcm_slic_device): the label map goes to qs_labels (and the count to
+    // qs_n_labels), so that pcm_update(labels == NULL) continues from it as from a quickshift map.  sl_smooth, sl_img and
+    // sl_nearest keep the stage results of the last call (pcm_slic_debug_last).
+    DevBuf sl_kernel, sl_smooth, sl_tmp, sl_img, sl_centers, sl_dmin, sl_best, sl_nearest, sl_keys, sl_iota, sl_sidx, sl_begin,
+           sl_end, sl_cub, sl_count;
+    DevBuf sl_parent, sl_root, sl_csize, sl_piece, sl_psize, sl_off, sl_queue, sl_seen, sl_adj, sl_nxt, sl_val, sl_labels;
+    PinBuf h_slic;                // Gaussian weights + seed centres
+    int sl_w = 0, sl_h = 0;       // crop of the stage results; 0: none
     // forest training (pcm_fit_forest): feature-major rows resident between calls, scratch, outputs
     DevBuf fit_x, fit_xt, fit_y, fit_counts, fit_rand, fit_samples, fit_tmp, fit_out;
     DevBuf prior_scratch;         // pcm_prior_device: per-keypoint match records
@@ -1306,7 +1317,7 @@ static int update_from_quickshift(pcm_handle* h, const uint8_t* frame, int H, in
                                   int64_t mask_row_stride, int64_t mask_pixel_stride) {
     if (!rect) return fail(PCM_E_INVALID, "pcm_update: NULL rect");
     if (!h->qs_valid || h->qs_frame_ptr != frame || memcmp(h->qs_rect, rect, sizeof h->qs_rect) != 0)
-        return fail(PCM_E_STATE, "pcm_update: labels == NULL needs a preceding pcm_quickshift of the same frame and rect");
+        return fail(PCM_E_STATE, "pcm_update: labels == NULL needs a preceding pcm_quickshift or pcm_slic_gpu of the same frame and rect");
     int rc = validate_update(h, H, W, rect, h->qs_n_labels, params);
     if (rc) return rc;
     CUDA_TRY(cudaSetDevice(h->device));
@@ -1351,7 +1362,7 @@ extern "C" int pcm_update(pcm_handle* h, const uint8_t* frame, int H, int W, int
     const bool reuse_labels = !labels;
     if (reuse_labels) {
         if (!rect || h->resident_labels <= 0 || rect[2] != h->resident_cw || rect[3] != h->resident_ch)
-            return fail(PCM_E_STATE, "pcm_update: labels == NULL needs a preceding pcm_quickshift of the same frame and rect, or a "
+            return fail(PCM_E_STATE, "pcm_update: labels == NULL needs a preceding pcm_quickshift or pcm_slic_gpu of the same frame and rect, or a "
                                      "preceding pcm_update with a label map for a crop of the same size");
         n_labels = h->resident_labels;
     }
@@ -1825,6 +1836,362 @@ extern "C" int pcm_felzenszwalb_graph(int n_vertices, int n_edges, const int32_t
     const int n = felzenszwalb_graph(n_vertices, n_edges, a, b, cost, scale, min_size, labels_out);
     if (n < 0) return fail(PCM_E_INVALID, "pcm_felzenszwalb_graph: vertex index out of range or negative / NaN cost");
     if (n_labels_out) *n_labels_out = n;
+    return PCM_OK;
+}
+
+// ---------------------------------------------------------------------------------
+// API: SLIC over-segmentation on the GPU (pcm_slic.cuh).  Same labels as pcm_slic; see DESIGN.md §10.
+// ---------------------------------------------------------------------------------
+// regular_grid((1, h, w), n_points) as pcm_slic.cpp's slic_grid computes it (same expressions, host code): start and step of
+// the seed grid along rows and columns; false: every pixel is a seed
+static bool slic_seed_grid(int h, int w, int n_points, int& start_y, int& step_y, int& start_x, int& step_x) {
+    const double space = (double)h * (double)w;
+    if (space <= (double)n_points) return false;
+    double steps[3] = {std::pow(space / n_points, 1.0 / 3), 0, 0};
+    steps[1] = steps[2] = steps[0];
+    const double dims[3] = {1.0, (double)std::min(h, w), (double)std::max(h, w)};
+    bool any_short = false;
+    for (int d = 0; d < 3; ++d) any_short = any_short || dims[d] < steps[d];
+    if (any_short) {
+        for (int d = 0; d < 3; ++d) {
+            steps[d] = dims[d];
+            double sp = 1.0;
+            for (int e = d + 1; e < 3; ++e) sp *= dims[e];
+            for (int e = d + 1; e < 3; ++e) steps[e] = std::pow(sp / n_points, 1.0 / (3 - d - 1));
+            bool ok = true;
+            for (int e = 0; e < 3; ++e) ok = ok && dims[e] >= steps[e];
+            if (ok) break;
+        }
+    }
+    const int s_min = (int)std::floor(steps[1] / 2), s_max = (int)std::floor(steps[2] / 2);
+    const int t_min = (int)std::nearbyint(steps[1]), t_max = (int)std::nearbyint(steps[2]);
+    if (h <= w) { start_y = s_min; step_y = t_min; start_x = s_max; step_x = t_max; }
+    else        { start_y = s_max; step_y = t_max; start_x = s_min; step_x = t_min; }
+    step_y = std::max(step_y, 1); step_x = std::max(step_x, 1);
+    return true;
+}
+
+static int bit_length(unsigned v) { int b = 0; while (v) { ++b; v >>= 1; } return b; }
+
+static int check_slic_args(const char* who, const int rect[4], int H, int W, int n_segments, double compactness, int max_iter,
+                           int start_label, const double* kernel, int kernel_radius) {
+    if (int rc = check_rect(who, rect, H, W)) return rc;
+    if ((long long)rect[2] * rect[3] > (1LL << 28)) return fail(PCM_E_LIMIT, "%s: crop too large (more than 2^28 pixels)", who);
+    if (n_segments < 1) return fail(PCM_E_INVALID, "%s: n_segments %d < 1", who, n_segments);
+    if (!(compactness > 0)) return fail(PCM_E_INVALID, "%s: compactness must be > 0", who);
+    if (max_iter < 0) return fail(PCM_E_INVALID, "%s: max_iter %d < 0", who, max_iter);
+    if (start_label < 0) return fail(PCM_E_INVALID, "%s: start_label %d", who, start_label);
+    if (kernel && kernel_radius < 0) return fail(PCM_E_INVALID, "%s: kernel_radius %d", who, kernel_radius);
+    return PCM_OK;
+}
+
+// CUB scratch for a stable sort of n (int key, int value) pairs and an exclusive sum of n ints
+static int reserve_slic_cub(pcm_handle* h, int n, size_t* bytes) {
+    size_t a = 0, b = 0;
+    CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, a, (const int*)nullptr, (int*)nullptr, (const int*)nullptr, (int*)nullptr, n));
+    CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, b, (const int*)nullptr, (int*)nullptr, n));
+    *bytes = std::max(a, b);
+    CUDA_TRY(h->sl_cub.reserve(*bytes));
+    return PCM_OK;
+}
+
+// S5 of pcm_slic.cuh: connectivity enforcement of the centre map d_seg (w x hh) into d_labels; the largest label goes to
+// sl_count.  Asynchronous.
+static int enqueue_slic_connectivity(pcm_handle* h, const int32_t* d_seg, int w, int hh, long long min_size, long long max_size,
+                                     int start_label, int32_t* d_labels) {
+    const int n = w * hh;
+    const size_t ib = (size_t)n * sizeof(int);
+    cudaStream_t st = h->stream;
+    for (DevBuf* b : {&h->sl_parent, &h->sl_root, &h->sl_csize, &h->sl_piece, &h->sl_psize, &h->sl_off, &h->sl_queue, &h->sl_seen,
+                      &h->sl_adj, &h->sl_nxt, &h->sl_val, &h->sl_keys, &h->sl_iota, &h->sl_sidx})
+        CUDA_TRY(b->reserve(ib));
+    CUDA_TRY(h->sl_count.reserve(sizeof(int)));
+    size_t cub_bytes = 0;
+    if (int rc = reserve_slic_cub(h, n, &cub_bytes)) return rc;
+    const int blocks = (int)std::min<long long>((n + SLIC_THREADS - 1) / SLIC_THREADS, (long long)h->sm_count * 16);
+    int* parent = h->sl_parent.as<int>();
+    int* root = h->sl_root.as<int>();
+    int* csize = h->sl_csize.as<int>();
+    int* piece = h->sl_piece.as<int>();
+    int* psize = h->sl_psize.as<int>();
+    int* off = h->sl_off.as<int>();
+    int* iota = h->sl_iota.as<int>();
+    slic_ccl_init_kernel<<<blocks, SLIC_THREADS, 0, st>>>(iota, n);
+    CHECK_LAUNCH(h, "slic_ccl_init_kernel");
+    slic_ccl_init_kernel<<<blocks, SLIC_THREADS, 0, st>>>(parent, n);
+    CHECK_LAUNCH(h, "slic_ccl_init_kernel");
+    slic_ccl_merge_kernel<<<blocks, SLIC_THREADS, 0, st>>>(d_seg, parent, w, hh);
+    CHECK_LAUNCH(h, "slic_ccl_merge_kernel");
+    CUDA_TRY(cudaMemsetAsync(csize, 0, ib, st));
+    slic_ccl_flatten_kernel<<<blocks, SLIC_THREADS, 0, st>>>(parent, root, csize, n);
+    CHECK_LAUNCH(h, "slic_ccl_flatten_kernel");
+    CUDA_TRY(cudaMemsetAsync(psize, 0, ib, st));
+    slic_piece_init_kernel<<<blocks, SLIC_THREADS, 0, st>>>(root, csize, max_size, piece, psize, n);
+    CHECK_LAUNCH(h, "slic_piece_init_kernel");
+    // the pixels of each component in raster order: stable sort by root; the component of root r starts at coff[r]
+    CUDA_TRY(cub::DeviceRadixSort::SortPairs(h->sl_cub.p, cub_bytes, root, h->sl_keys.as<int>(), iota, h->sl_sidx.as<int>(), n, 0,
+                                             std::max(1, bit_length((unsigned)(n - 1))), st));
+    CUDA_TRY(cub::DeviceScan::ExclusiveSum(h->sl_cub.p, cub_bytes, csize, off, n, st));
+    slic_split_kernel<<<blocks, SLIC_THREADS, 0, st>>>(d_seg, csize, off, h->sl_sidx.as<int>(), w, hh, max_size, piece, psize,
+                                                       h->sl_queue.as<int>());
+    CHECK_LAUNCH(h, "slic_split_kernel");
+    CUDA_TRY(cub::DeviceScan::ExclusiveSum(h->sl_cub.p, cub_bytes, psize, off, n, st));
+    CUDA_TRY(cudaMemsetAsync(h->sl_seen.p, 0, ib, st));
+    slic_small_kernel<<<blocks, SLIC_THREADS, 0, st>>>(piece, psize, off, w, hh, min_size, max_size, h->sl_queue.as<int>(),
+                                                       h->sl_seen.as<int>(), h->sl_adj.as<int>());
+    CHECK_LAUNCH(h, "slic_small_kernel");
+    slic_flag_kernel<<<blocks, SLIC_THREADS, 0, st>>>(psize, min_size, parent, n);
+    CHECK_LAUNCH(h, "slic_flag_kernel");
+    CUDA_TRY(cub::DeviceScan::ExclusiveSum(h->sl_cub.p, cub_bytes, parent, off, n, st));
+    slic_link_kernel<<<blocks, SLIC_THREADS, 0, st>>>(psize, off, h->sl_adj.as<int>(), min_size, start_label, h->sl_nxt.as<int>(),
+                                                      h->sl_val.as<int>(), n);
+    CHECK_LAUNCH(h, "slic_link_kernel");
+    for (int r = bit_length((unsigned)n); r >= 0; --r) {          // a chain of at most n pieces: ceil(log2 n) + 1 rounds
+        slic_jump_kernel<<<blocks, SLIC_THREADS, 0, st>>>(psize, h->sl_nxt.as<int>(), n);
+        CHECK_LAUNCH(h, "slic_jump_kernel");
+    }
+    CUDA_TRY(cudaMemsetAsync(h->sl_count.p, 0xff, sizeof(int), st));
+    slic_label_kernel<<<blocks, SLIC_THREADS, 0, st>>>(piece, h->sl_nxt.as<int>(), h->sl_val.as<int>(), d_labels, h->sl_count.as<int>(), n);
+    CHECK_LAUNCH(h, "slic_label_kernel");
+    return PCM_OK;
+}
+
+// The whole SLIC of the crop (cx, cy, w, hh) of a device frame into qs_labels (and d_labels_out when given).  Asynchronous
+// apart from the host-side staging of the weights and seeds; the caller waits for sl_count (read_slic_count).
+static int enqueue_slic(pcm_handle* h, const uint8_t* d_frame, int64_t stride, int cx, int cy, int w, int hh, int n_segments,
+                        double compactness, double sigma, const double* kernel, int radius, int max_iter, int start_label,
+                        int32_t* d_labels_out) {
+    const int n = w * hh;
+    cudaStream_t st = h->stream;
+    h->chain_tail = false;
+    h->sl_w = h->sl_h = 0;
+    // Gaussian weights: the caller's, or scipy's _gaussian_kernel1d computed as pcm_slic.cpp does (truncate = 4)
+    std::vector<double> kw;
+    if (sigma > 0 && !kernel) {
+        radius = (int)(4.0 * sigma + 0.5);
+        kw.resize(2 * radius + 1);
+        double sum = 0;
+        for (int x = -radius; x <= radius; ++x) { kw[x + radius] = std::exp(-0.5 / (sigma * sigma) * (double)(x * x)); sum += kw[x + radius]; }
+        for (double& v : kw) v /= sum;
+        kernel = kw.data();
+    }
+    if (!(sigma > 0)) radius = 0;
+    // seeds on the regular grid (every pixel when there are no more pixels than segments)
+    int sy = 0, ty = 1, sx = 0, tx = 1;
+    const bool grid = slic_seed_grid(hh, w, n_segments, sy, ty, sx, tx);
+    if (!grid) { sy = sx = 0; ty = tx = 1; }
+    const int ny = sy < hh ? (hh - sy + ty - 1) / ty : 0, nx = sx < w ? (w - sx + tx - 1) / tx : 0;
+    const long long K = (long long)ny * nx;
+    if (K < 1) return fail(PCM_E_INVALID, "slic: no seed inside the %dx%d crop", w, hh);
+    const double step = (double)std::max(1, std::max(ty, tx));
+    const double spatial_weight = 1.0 / (step * step);
+    const size_t nk = sigma > 0 ? (size_t)(2 * radius + 1) : 0;
+    const size_t cbytes = (size_t)K * 5 * sizeof(double);
+    CUDA_TRY(h->h_slic.reserve(nk * sizeof(double) + cbytes));
+    double* hk = h->h_slic.as<double>();
+    if (nk) memcpy(hk, kernel, nk * sizeof(double));
+    double* hc = hk + nk;
+    for (int a = 0; a < ny; ++a)
+        for (int b = 0; b < nx; ++b) {
+            double* c = hc + ((size_t)a * nx + b) * 5;
+            c[0] = sy + a * ty; c[1] = sx + b * tx; c[2] = c[3] = c[4] = 0.0;
+        }
+    const size_t ib = (size_t)n * sizeof(int), db = (size_t)n * 3 * sizeof(double);
+    CUDA_TRY(h->sl_kernel.reserve(std::max<size_t>(nk, 1) * sizeof(double)));
+    CUDA_TRY(h->sl_centers.reserve(cbytes));
+    CUDA_TRY(h->sl_smooth.reserve(db));
+    CUDA_TRY(h->sl_tmp.reserve(db));
+    CUDA_TRY(h->sl_img.reserve(db));
+    CUDA_TRY(h->sl_dmin.reserve((size_t)n * sizeof(unsigned long long)));
+    for (DevBuf* b : {&h->sl_best, &h->sl_nearest, &h->sl_keys, &h->sl_iota, &h->sl_sidx}) CUDA_TRY(b->reserve(ib));
+    CUDA_TRY(h->sl_begin.reserve((size_t)K * sizeof(int)));
+    CUDA_TRY(h->sl_end.reserve((size_t)K * sizeof(int)));
+    CUDA_TRY(h->qs_labels.reserve(ib));
+    size_t cub_bytes = 0;
+    if (int rc = reserve_slic_cub(h, n, &cub_bytes)) return rc;
+    if (nk) CUDA_TRY(cudaMemcpyAsync(h->sl_kernel.p, hk, nk * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(h->sl_centers.p, hc, cbytes, cudaMemcpyHostToDevice, st));
+    h->bytes_h2d += (int64_t)(nk * sizeof(double) + cbytes);
+
+    const int blocks = (int)std::min<long long>(((long long)n + SLIC_THREADS - 1) / SLIC_THREADS, (long long)h->sm_count * 16);
+    const double* dk = h->sl_kernel.as<double>();
+    double* smooth = h->sl_smooth.as<double>();
+    slic_load_kernel<<<blocks, SLIC_THREADS, 0, st>>>(d_frame, stride, cx, cy, w, hh, dk, radius, sigma > 0 ? 1 : 0, smooth);
+    CHECK_LAUNCH(h, "slic_load_kernel");
+    if (sigma > 0) {
+        slic_smooth_kernel<<<blocks, SLIC_THREADS, 0, st>>>(smooth, h->sl_tmp.as<double>(), hh, w, 0, dk, radius);
+        CHECK_LAUNCH(h, "slic_smooth_kernel");
+        slic_smooth_kernel<<<blocks, SLIC_THREADS, 0, st>>>(h->sl_tmp.as<double>(), smooth, hh, w, 1, dk, radius);
+        CHECK_LAUNCH(h, "slic_smooth_kernel");
+    }
+    const double* img = h->sl_img.as<double>();
+    slic_lab_kernel<<<blocks, SLIC_THREADS, 0, st>>>(smooth, h->sl_img.as<double>(), n, 1.0 / compactness);
+    CHECK_LAUNCH(h, "slic_lab_kernel");
+
+    int* nearest = h->sl_nearest.as<int>();
+    int* iota = h->sl_iota.as<int>();
+    double* centers = h->sl_centers.as<double>();
+    CUDA_TRY(cudaMemsetAsync(nearest, 0, ib, st));
+    slic_ccl_init_kernel<<<blocks, SLIC_THREADS, 0, st>>>(iota, n);
+    CHECK_LAUNCH(h, "slic_ccl_init_kernel");
+    const int key_bits = std::max(1, bit_length((unsigned)(K - 1)));
+    for (int it = 0; it < max_iter; ++it) {
+        CUDA_TRY(cudaMemsetAsync(h->sl_dmin.p, 0xff, (size_t)n * sizeof(unsigned long long), st));
+        CUDA_TRY(cudaMemsetAsync(h->sl_best.p, 0x7f, ib, st));
+        slic_assign_kernel<false><<<(unsigned)K, SLIC_THREADS, 0, st>>>(img, centers, hh, w, ty, tx, spatial_weight,
+                                                                         h->sl_dmin.as<unsigned long long>(), h->sl_best.as<int>());
+        CHECK_LAUNCH(h, "slic_assign_kernel<false>");
+        slic_assign_kernel<true><<<(unsigned)K, SLIC_THREADS, 0, st>>>(img, centers, hh, w, ty, tx, spatial_weight,
+                                                                        h->sl_dmin.as<unsigned long long>(), h->sl_best.as<int>());
+        CHECK_LAUNCH(h, "slic_assign_kernel<true>");
+        slic_settle_kernel<<<blocks, SLIC_THREADS, 0, st>>>(h->sl_best.as<int>(), nearest, n);
+        CHECK_LAUNCH(h, "slic_settle_kernel");
+        CUDA_TRY(cub::DeviceRadixSort::SortPairs(h->sl_cub.p, cub_bytes, nearest, h->sl_keys.as<int>(), iota, h->sl_sidx.as<int>(), n,
+                                                 0, key_bits, st));
+        CUDA_TRY(cudaMemsetAsync(h->sl_begin.p, 0, (size_t)K * sizeof(int), st));
+        CUDA_TRY(cudaMemsetAsync(h->sl_end.p, 0, (size_t)K * sizeof(int), st));
+        slic_bounds_kernel<<<blocks, SLIC_THREADS, 0, st>>>(h->sl_keys.as<int>(), n, h->sl_begin.as<int>(), h->sl_end.as<int>());
+        CHECK_LAUNCH(h, "slic_bounds_kernel");
+        slic_update_kernel<<<(unsigned)((K + 127) / 128), 128, 0, st>>>(h->sl_sidx.as<int>(), h->sl_begin.as<int>(), h->sl_end.as<int>(),
+                                                                         img, w, (int)K, centers);
+        CHECK_LAUNCH(h, "slic_update_kernel");
+    }
+    // connectivity: min_size_factor 0.5, max_size_factor 3 of the requested segment size
+    const double segment_size = (double)hh * (double)w / n_segments;
+    const long long min_size = (long long)(0.5 * segment_size), max_size = (long long)(3 * segment_size);
+    if (int rc = enqueue_slic_connectivity(h, nearest, w, hh, min_size, max_size, start_label, h->qs_labels.as<int32_t>())) return rc;
+    if (d_labels_out) CUDA_TRY(cudaMemcpyAsync(d_labels_out, h->qs_labels.p, ib, cudaMemcpyDeviceToDevice, st));
+    h->sl_w = w; h->sl_h = hh;
+    return PCM_OK;
+}
+
+// waits for the stream; *n_labels = largest label + 1, as pcm_slic counts
+static int read_slic_count(pcm_handle* h, int* n_labels) {
+    CUDA_TRY(h->h_small.reserve(64));
+    int* hs = h->h_small.as<int>() + 12;
+    CUDA_TRY(cudaMemcpyAsync(hs, h->sl_count.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
+    *n_labels = *hs + 1;
+    return PCM_OK;
+}
+
+extern "C" int pcm_slic_device(pcm_handle* h, const uint8_t* d_frame, int H, int W, int64_t stride, const int rect[4],
+                               int n_segments, double compactness, double sigma, const double* kernel, int kernel_radius,
+                               int max_iter, int start_label, int32_t* d_labels_out, int* n_labels_out) {
+    if (!h || !d_frame || !rect) return fail(PCM_E_INVALID, "pcm_slic_device: NULL argument");
+    int rc = check_slic_args("pcm_slic_device", rect, H, W, n_segments, compactness, max_iter, start_label, kernel, kernel_radius);
+    if (rc) return rc;
+    if (stride < (int64_t)W * 3) return fail(PCM_E_INVALID, "pcm_slic_device: stride %lld < 3*W", (long long)stride);
+    CUDA_TRY(cudaSetDevice(h->device));
+    h->qs_valid = false;
+    CUDA_TRY(cudaStreamSynchronize(h->stream));      // the pinned seed buffer is reused between calls
+    rc = enqueue_slic(h, d_frame, stride, rect[0], rect[1], rect[2], rect[3], n_segments, compactness, sigma, kernel, kernel_radius,
+                      max_iter, start_label, d_labels_out);
+    if (rc) return rc;
+    int count = 0;
+    if ((rc = read_slic_count(h, &count))) return rc;
+    if (n_labels_out) *n_labels_out = count;
+    return PCM_OK;
+}
+
+extern "C" int pcm_slic_device_batch(pcm_handle* h, int n, const uint8_t* d_frames, int64_t frame_bytes, const int32_t* frame_index,
+                                     int H, int W, int64_t stride, const int32_t* rects, int n_segments, double compactness,
+                                     double sigma, const double* kernel, int kernel_radius, int max_iter, int start_label,
+                                     int32_t* d_labels_out, const int64_t* label_offsets, int32_t* n_labels_out) {
+    if (!h || !d_frames || !frame_index || !rects || !d_labels_out || !label_offsets || !n_labels_out)
+        return fail(PCM_E_INVALID, "pcm_slic_device_batch: NULL argument");
+    if (n < 0 || frame_bytes < 0) return fail(PCM_E_INVALID, "pcm_slic_device_batch: bad count / frame size");
+    for (int k = 0; k < n; ++k) {
+        if (frame_index[k] < 0 || label_offsets[k] < 0) return fail(PCM_E_INVALID, "pcm_slic_device_batch: crop %d: negative index", k);
+        int count = 0;
+        const int rect[4] = {rects[4 * k], rects[4 * k + 1], rects[4 * k + 2], rects[4 * k + 3]};
+        const int rc = pcm_slic_device(h, d_frames + (int64_t)frame_index[k] * frame_bytes, H, W, stride, rect, n_segments, compactness,
+                                       sigma, kernel, kernel_radius, max_iter, start_label, d_labels_out + label_offsets[k], &count);
+        if (rc) return rc;
+        n_labels_out[k] = count;
+    }
+    return PCM_OK;
+}
+
+extern "C" int pcm_slic_gpu(pcm_handle* h, const uint8_t* frame, int H, int W, int64_t stride, const int rect[4], int n_segments,
+                            double compactness, double sigma, const double* kernel, int kernel_radius, int max_iter,
+                            int start_label, int32_t* labels_out, int* n_labels_out) {
+    if (!h || !frame || !rect) return fail(PCM_E_INVALID, "pcm_slic_gpu: NULL argument");
+    int rc = check_slic_args("pcm_slic_gpu", rect, H, W, n_segments, compactness, max_iter, start_label, kernel, kernel_radius);
+    if (rc) return rc;
+    if (stride < (int64_t)W * 3) return fail(PCM_E_INVALID, "pcm_slic_gpu: stride %lld < 3*W", (long long)stride);
+    CUDA_TRY(cudaSetDevice(h->device));
+    const int cx = rect[0], cy = rect[1], cw = rect[2], ch = rect[3];
+    const size_t npx = (size_t)cw * ch, row_bytes = (size_t)cw * 3;
+    cudaStream_t st = h->stream;
+    h->qs_valid = false;
+    CUDA_TRY(h->h_frame.reserve(npx * 3));
+    CUDA_TRY(h->frame.reserve(npx * 3));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    // crop rows -> pinned -> device, one pool dispatch (the crop stays there for pcm_update with labels == NULL)
+    const int frame_rows = rows_per_chunk((size_t)1 << 20, row_bytes);
+    const uint8_t* crop0 = frame + (size_t)cy * stride + (size_t)cx * 3;
+    uint8_t* hf = h->h_frame.as<uint8_t>();
+    uint8_t* df = h->frame.as<uint8_t>();
+    rc = stage_items(h, "pcm_slic_gpu", (ch + frame_rows - 1) / frame_rows, [&](int item) -> cudaError_t {
+        const int r0 = item * frame_rows;
+        return stage_rows(h, df, hf, crop0, (size_t)stride, row_bytes, r0, std::min(ch, r0 + frame_rows));
+    });
+    if (rc) return rc;
+    rc = enqueue_slic(h, df, (int64_t)row_bytes, 0, 0, cw, ch, n_segments, compactness, sigma, kernel, kernel_radius, max_iter,
+                      start_label, nullptr);
+    if (rc) return rc;
+    if (labels_out) {
+        CUDA_TRY(h->h_labels.reserve(npx * sizeof(int32_t)));
+        h->label_cache_px = 0;                        // the pinned label buffer no longer mirrors `labels`
+        CUDA_TRY(cudaMemcpyAsync(h->h_labels.p, h->qs_labels.p, npx * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        h->bytes_d2h += (int64_t)(npx * sizeof(int32_t));
+    }
+    int count = 0;
+    if ((rc = read_slic_count(h, &count))) return rc;
+    if (n_labels_out) *n_labels_out = count;
+    if (labels_out) memcpy(labels_out, h->h_labels.p, npx * sizeof(int32_t));
+    h->qs_n_labels = count;
+    h->qs_cw = cw; h->qs_ch = ch;
+    h->qs_frame_ptr = frame;
+    memcpy(h->qs_rect, rect, sizeof h->qs_rect);
+    h->qs_valid = true;
+    return PCM_OK;
+}
+
+extern "C" int pcm_slic_connectivity(pcm_handle* h, const int32_t* nearest, int width, int height, long long min_size,
+                                     long long max_size, int start_label, int32_t* labels_out, int* n_labels_out) {
+    if (!h || !nearest || !labels_out) return fail(PCM_E_INVALID, "pcm_slic_connectivity: NULL argument");
+    if (width <= 0 || height <= 0 || (long long)width * height > (1LL << 28))
+        return fail(PCM_E_INVALID, "pcm_slic_connectivity: bad size %dx%d", width, height);
+    if (start_label < 0) return fail(PCM_E_INVALID, "pcm_slic_connectivity: start_label %d", start_label);
+    CUDA_TRY(cudaSetDevice(h->device));
+    const size_t ib = (size_t)width * height * sizeof(int32_t);
+    cudaStream_t st = h->stream;
+    h->chain_tail = false;
+    CUDA_TRY(h->sl_best.reserve(ib));
+    CUDA_TRY(h->sl_labels.reserve(ib));
+    CUDA_TRY(cudaMemcpyAsync(h->sl_best.p, nearest, ib, cudaMemcpyHostToDevice, st));
+    int rc = enqueue_slic_connectivity(h, h->sl_best.as<int32_t>(), width, height, min_size, max_size, start_label,
+                                       h->sl_labels.as<int32_t>());
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(labels_out, h->sl_labels.p, ib, cudaMemcpyDeviceToHost, st));
+    int count = 0;
+    if ((rc = read_slic_count(h, &count))) return rc;
+    if (n_labels_out) *n_labels_out = count;
+    return PCM_OK;
+}
+
+extern "C" int pcm_slic_debug_last(pcm_handle* h, double* smoothed, double* image, int32_t* nearest) {
+    if (!h) return fail(PCM_E_INVALID, "pcm_slic_debug_last: NULL handle");
+    if (!h->sl_w) return fail(PCM_E_STATE, "pcm_slic_debug_last: no SLIC on this handle yet");
+    CUDA_TRY(cudaSetDevice(h->device));
+    const size_t n = (size_t)h->sl_w * h->sl_h;
+    cudaStream_t st = h->stream;
+    if (smoothed) CUDA_TRY(cudaMemcpyAsync(smoothed, h->sl_smooth.p, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (image) CUDA_TRY(cudaMemcpyAsync(image, h->sl_img.p, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (nearest) CUDA_TRY(cudaMemcpyAsync(nearest, h->sl_nearest.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
     return PCM_OK;
 }
 

@@ -70,11 +70,15 @@ class PixelClassificationNonRigidMasker(Masker):
         self.spaces = tokens[1].split("_")
         self.native = capi.Handle(device)
         self.native.set_features(self.n_neighbors, self.spaces)
-        # over-segmentation (:70-75), SURVEY §8 f-1: quickshift runs on the GPU (pcm_quickshift),
-        # felzenszwalb and SLIC in the library's host code (pcm_felzenszwalb: inherently sequential; pcm_slic)
+        # over-segmentation (:70-75), SURVEY §8 f-1: quickshift and SLIC run on the GPU (pcm_quickshift, pcm_slic_gpu),
+        # felzenszwalb in the library's host code (pcm_felzenszwalb: inherently sequential).  config `slic_provider`:
+        # "gpu" (default) or "host" (pcm_slic, the library's host code; same labels)
         self.native_quickshift = segment_fn is None and params["over_segmentation"] == "quickshift"
         self.native_felzenszwalb = segment_fn is None and params["over_segmentation"] == "felzenszwalb"
         self.native_slic = segment_fn is None and params["over_segmentation"] == "SLIC"
+        self.slic_provider = self.config.get("slic_provider") or "gpu"
+        if self.slic_provider not in ("gpu", "host"):
+            raise ValueError("slic_provider must be gpu or host, got %r" % (self.slic_provider,))
         self.segment_fn = segment_fn or (None if (self.native_quickshift or self.native_felzenszwalb or self.native_slic)
                                          else make_segment_provider(params["over_segmentation"]))
         self._qs_noise_shape = None
@@ -207,18 +211,24 @@ class PixelClassificationNonRigidMasker(Masker):
             return self.prior_fn(self.prevFrame, self.prevForegroundMask, crop, segs, n)
         n_labels, priors = 0, None             # 0: the library takes max(label) + 1 while staging
         same_labels, self._seg_next = False, None
-        if self.native_quickshift:
-            # quickshift(crop, kernel_size=3, max_dist=6, ratio=0.5, random_seed=42) (:71); the label
+        if self.native_quickshift or (self.native_slic and self.slic_provider == "gpu"):
+            # quickshift(crop, kernel_size=3, max_dist=6, ratio=0.5, random_seed=42) (:71) or
+            # slic(crop, n_segments=250, compactness=10, sigma=1, start_label=0) (:75) on the GPU; the label
             # map stays on the device and only travels to the host when the SIFT prior needs it
             if frame.strides[2] != 1 or frame.strides[1] != 3:
                 frame = np.ascontiguousarray(frame)
-            noise = None
-            if self._qs_noise_shape != (h, w):
-                noise = np.random.RandomState(42).normal(scale=0.00001, size=(h, w))
-                self._qs_noise_shape = (h, w)
-            with stages.stage("gpu_quickshift_call"):
-                segments, n_labels = self.native.quickshift(frame, (x, y, w, h), ratio=0.5, kernel_size=3, max_dist=6,
-                                                            noise=noise, want_labels=want_prior)
+            if self.native_quickshift:
+                noise = None
+                if self._qs_noise_shape != (h, w):
+                    noise = np.random.RandomState(42).normal(scale=0.00001, size=(h, w))
+                    self._qs_noise_shape = (h, w)
+                with stages.stage("gpu_quickshift_call"):
+                    segments, n_labels = self.native.quickshift(frame, (x, y, w, h), ratio=0.5, kernel_size=3, max_dist=6,
+                                                                noise=noise, want_labels=want_prior)
+            else:
+                with stages.stage("gpu_slic_call"):
+                    segments, n_labels = self.native.slic(frame, (x, y, w, h), n_segments=250, compactness=10.0, sigma=1.0,
+                                                          start_label=0, want_labels=want_prior)
             if want_prior:
                 with stages.stage("sift_prior"):
                     priors = prior(segments, n_labels)
@@ -237,7 +247,7 @@ class PixelClassificationNonRigidMasker(Masker):
                     else:
                         segments, n_labels = segment()
             elif self.native_slic:
-                # slic(crop, n_segments=250, compactness=10, sigma=1, start_label=0) (:75)
+                # slic(crop, n_segments=250, compactness=10, sigma=1, start_label=0) (:75), slic_provider "host"
                 with stages.stage("slic"):
                     segments, n_labels = capi.slic(frame, (x, y, w, h), n_segments=250, compactness=10.0, sigma=1.0, start_label=0)
             else:

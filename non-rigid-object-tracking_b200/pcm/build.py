@@ -17,7 +17,7 @@ UNITS = [("pcm_api.cu", [], "pcm_api.o"),
          ("pcm_felzenszwalb.cpp", [], "pcm_felzenszwalb.o"),
          ("pcm_slic.cpp", [], "pcm_slic.o")]
 DEPS = ["pcm_api.cu", "pcm_score_inst.cu", "pcm_score_variants.h", "pcm_score.cuh", "pcm_kernels.cuh", "pcm_device.cuh", "pcm_host.h",
-        "pcm_host_simd.cpp", "pcm_felzenszwalb.cpp", "pcm_slic.cpp", "pcm_quickshift.cuh", "pcm_forest_fit.cuh", "pcm_prior.cuh",
+        "pcm_host_simd.cpp", "pcm_felzenszwalb.cpp", "pcm_slic.cpp", "pcm_slic.cuh", "pcm_quickshift.cuh", "pcm_forest_fit.cuh", "pcm_prior.cuh",
         os.path.join("..", "..", "include", "pcm_b200.h")]
 
 NVCC_FLAGS = [

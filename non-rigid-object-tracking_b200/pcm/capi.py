@@ -68,6 +68,11 @@ _SIGNATURES = {
     "pcm_felzenszwalb": (I, [P, I, I, L, P, D, D, I, P, I, P, C.POINTER(I)]),
     "pcm_felzenszwalb_graph": (I, [I, I, P, P, P, D, I, P, C.POINTER(I)]),
     "pcm_slic": (I, [P, I, I, L, P, I, D, D, P, I, I, I, P, C.POINTER(I)]),
+    "pcm_slic_gpu": (I, [P, P, I, I, L, P, I, D, D, P, I, I, I, P, C.POINTER(I)]),
+    "pcm_slic_device": (I, [P, P, I, I, L, P, I, D, D, P, I, I, I, P, C.POINTER(I)]),
+    "pcm_slic_device_batch": (I, [P, I, P, L, P, I, I, L, P, I, D, D, P, I, I, I, P, P, P]),
+    "pcm_slic_connectivity": (I, [P, P, I, I, C.c_longlong, C.c_longlong, I, P, C.POINTER(I)]),
+    "pcm_slic_debug_last": (I, [P, P, P, P]),
     "pcm_host_register": (I, [P, C.c_size_t]),
     "pcm_host_unregister": (I, [P]),
     "pcm_run_frames": (I, [P, I, I, L, P, L, P, I]),
@@ -437,6 +442,74 @@ class Handle:
                                                          float(max_dist), C.c_void_p(d_noise) if d_noise else None,
                                                          C.c_void_p(d_labels_out), _ptr(off), _ptr(counts)))
         return counts
+
+    def slic(self, frame, rect, n_segments=250, compactness=10.0, sigma=1.0, max_iter=10, start_label=0, want_labels=True,
+             kernel=None):
+        """SLIC over-segmentation of the crop `rect` on the GPU (pcm_slic_gpu; defaults = the reference's call,
+        pixel_classification.py:75): the labels and count of the host `capi.slic`.  Returns (labels int32 HxW or None,
+        n_labels); the map also stays on the device for `update(..., labels=None)`.  `kernel`: Gaussian weights, or None
+        to compute them from sigma as scipy.ndimage does."""
+        if frame.dtype != np.uint8 or frame.ndim != 3 or frame.shape[2] != 3 or frame.strides[2] != 1 \
+                or frame.strides[1] != 3:
+            raise ValueError("frame must be an HxWx3 uint8 array with packed pixels")
+        r = (C.c_int * 4)(*[int(v) for v in rect])
+        weights, radius = self._slic_weights(sigma, kernel)
+        out = np.empty((rect[3], rect[2]), np.int32) if want_labels else None
+        n = C.c_int(0)
+        self._check(self.lib.pcm_slic_gpu(self._h, _ptr(frame), frame.shape[0], frame.shape[1], frame.strides[0], r,
+                                          int(n_segments), float(compactness), float(sigma), _ptr(weights), radius,
+                                          int(max_iter), int(start_label), _ptr(out), C.byref(n)))
+        self._slic_shape = (int(rect[3]), int(rect[2]))
+        return out, n.value
+
+    @staticmethod
+    def _slic_weights(sigma, kernel):
+        if kernel is None:
+            return _gaussian_weights(sigma)
+        k = np.ascontiguousarray(kernel, np.float64).reshape(-1)
+        if k.size % 2 != 1:
+            raise ValueError("kernel must have 2 * radius + 1 weights")
+        return k, k.size // 2
+
+    def slic_device_batch(self, d_frames, frame_bytes, frame_index, frame_h, frame_w, stride, rects, d_labels_out, label_offsets,
+                          n_segments=250, compactness=10.0, sigma=1.0, max_iter=10, start_label=0):
+        """SLIC of many crops of a device-resident clip in ONE native call (pcm_slic_device_batch), laid out like
+        quickshift_device_batch.  Returns the segment counts (int32 array)."""
+        fi = np.ascontiguousarray(frame_index, np.int32)
+        rc = np.ascontiguousarray(rects, np.int32).reshape(-1, 4)
+        off = np.ascontiguousarray(label_offsets, np.int64)
+        if not (len(fi) == len(rc) == len(off)):
+            raise ValueError("frame_index, rects and label_offsets must have one entry per crop")
+        weights, radius = _gaussian_weights(sigma)
+        counts = np.zeros(len(fi), np.int32)
+        self._check(self.lib.pcm_slic_device_batch(self._h, len(fi), C.c_void_p(d_frames), int(frame_bytes), _ptr(fi), int(frame_h),
+                                                   int(frame_w), int(stride), _ptr(rc), int(n_segments), float(compactness),
+                                                   float(sigma), _ptr(weights), radius, int(max_iter), int(start_label),
+                                                   C.c_void_p(d_labels_out), _ptr(off), _ptr(counts)))
+        if len(fi):
+            self._slic_shape = (int(rc[-1, 3]), int(rc[-1, 2]))
+        return counts
+
+    def slic_connectivity(self, nearest, min_size, max_size, start_label=0):
+        """Parity tap: the device connectivity enforcement of SLIC on a centre map (HxW ints).  Returns (labels int32 HxW,
+        n_labels)."""
+        seg = np.ascontiguousarray(nearest, np.int32)
+        if seg.ndim != 2:
+            raise ValueError("nearest must be HxW")
+        out = np.empty_like(seg)
+        n = C.c_int(0)
+        self._check(self.lib.pcm_slic_connectivity(self._h, _ptr(seg), seg.shape[1], seg.shape[0], int(min_size), int(max_size),
+                                                   int(start_label), _ptr(out), C.byref(n)))
+        return out, n.value
+
+    def slic_debug_last(self):
+        """Stage results of the last SLIC on this handle: smoothed (HxWx3 float64), image (HxWx3 float64, what the
+        k-means sees) and nearest (HxW int32, the centre map after the last iteration)."""
+        h, w = getattr(self, "_slic_shape", (0, 0))
+        smoothed, image = np.empty((h, w, 3), np.float64), np.empty((h, w, 3), np.float64)
+        nearest = np.empty((h, w), np.int32)
+        self._check(self.lib.pcm_slic_debug_last(self._h, _ptr(smoothed), _ptr(image), _ptr(nearest)))
+        return dict(smoothed=smoothed, image=image, nearest=nearest)
 
     def prior_device(self, d_pts_prev, d_des_prev, n_prev, d_prev_mask, prev_stride, prev_w, prev_h, d_pts, d_des, n_cur,
                      d_labels, crop_w, crop_h, n_labels, d_priors):

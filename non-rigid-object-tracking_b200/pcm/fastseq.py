@@ -5,8 +5,9 @@ What is shared by all sequences of a clip is computed once per rank and kept on 
   * the decoded frames and the ground truth (gray, cv.cvtColor(BGR2GRAY) as main.py:285);
   * the tracker boxes of every frame -- they depend on the frames and on the (known) frames at which the masker
     switches models, never on the masks (main.py:287-339);
-  * the over-segmentation of every frame's crop: quickshift on the GPU (pcm_quickshift_device) or felzenszwalb in
-    the library's host code (pixel_classification.py:70-73) -- a function of frame and crop only;
+  * the over-segmentation of every frame's crop: quickshift or SLIC on the GPU (pcm_quickshift_device_batch,
+    pcm_slic_device_batch) or felzenszwalb in the library's host code (pixel_classification.py:70-75) -- a function of
+    frame and crop only;
   * the SIFT keypoints / descriptors of every crop (pixel_classification.py:129-163), when a prior is asked for.
 A sequence is then ONE pass that enqueues, per frame, the masker kernels (`update_resident` -> pcm_update_device)
 and the IoU kernel (pcm_iou_device) on a stream and synchronises once at the end -- unless the SIFT prior is on,
@@ -103,7 +104,7 @@ class ClipContext:
                 self.d_truth = torch.from_numpy(gray).to(self.dev)
             torch.cuda.synchronize(self.dev)
         self.once = _Once()
-        self.handle = capi.Handle(device)            # clip-level GPU work (quickshift label maps)
+        self.handle = capi.Handle(device)            # clip-level GPU work (quickshift and SLIC label maps)
         self.handle_lock = threading.Lock()
 
     def close(self):
@@ -121,12 +122,13 @@ class ClipContext:
         """Everything the sequences of this clip share, computed NOW by the calling thread: tracker boxes, the label
         maps of the over-segmentations in `kinds`, SIFT features.  With a `share` of several ranks this is a collective:
         every member must call it with the same arguments, in the same order relative to its other clips.  (The
-        quickshift maps alone are no collective -- every rank computes them on its GPU -- and may be prepared from
-        another thread at the same time.)"""
+        quickshift and SLIC maps alone are no collective -- every rank computes them on its GPU -- and may be prepared
+        from another thread at the same time.)"""
         bboxes, switch = self.selections(config)
         box_key, _, rects, _ = self.schedule(config, bboxes, switch)
-        if not want_sift and list(kinds) == ["quickshift"]:
-            self.labels("quickshift", box_key, rects)
+        if not want_sift and set(kinds) <= {"quickshift", "SLIC"}:
+            for kind in sorted(kinds):
+                self.labels(kind, box_key, rects)
             return
         self._collective_ok = True
         try:
@@ -171,7 +173,7 @@ class ClipContext:
 
     # ---- over-segmentation ----------------------------------------------------------------------------------
     def labels(self, kind, box_key, rects, want_host=False):
-        """LabelArena of `kind` in {"quickshift", "felzenszwalb"} for the crops `rects` (entry k = frame k // T,
+        """LabelArena of `kind` in {"quickshift", "felzenszwalb", "SLIC"} for the crops `rects` (entry k = frame k // T,
         target k % T)."""
         torch = self.torch
 
@@ -197,6 +199,15 @@ class ClipContext:
                     n_labels.extend(int(v) for v in self.handle.quickshift_device_batch(
                         self.d_frames.data_ptr(), fb, [k // T for k in range(len(flat))], self.H, self.W, self.W * 3, flat,
                         0.5, 3, 6, d_noise.data_ptr(), d.data_ptr(), offsets[:len(flat)]))
+                host = None
+            elif kind == "SLIC":
+                with stages.stage("slic_maps"), self.handle_lock:
+                    # slic(crop, n_segments=250, compactness=10, sigma=1, start_label=0) (:75), one native call for the clip
+                    torch.cuda.current_stream(self.dev).synchronize()
+                    n_labels.extend(int(v) for v in self.handle.slic_device_batch(
+                        self.d_frames.data_ptr(), self.H * self.W * 3, [k // T for k in range(len(flat))], self.H, self.W,
+                        self.W * 3, flat, d.data_ptr(), offsets[:len(flat)], n_segments=250, compactness=10.0, sigma=1.0,
+                        start_label=0))
                 host = None
             elif kind == "felzenszwalb":
                 self._check_collective("felzenszwalb label maps")
@@ -325,7 +336,7 @@ def _precomputable(config):
         return False
     if config.get("masker") in (config.get("custom_trackers") or []):
         return False
-    return config["params"]["over_segmentation"] in ("quickshift", "felzenszwalb")
+    return config["params"]["over_segmentation"] in ("quickshift", "felzenszwalb", "SLIC")
 
 
 def _frame_loop(clip, maskers, rects, arena, sift, d_mask, d_counts, d_pri, gpu_prior, host_prior, model_cache, cache_tag):

@@ -244,7 +244,7 @@ def run_shard(items, base, polygons, device=0, videos_path="Input/SegTrack2/Vide
             clips = dict(zip(order_v, pool.map(open_clip, order_v)))
 
     gpu_prior = (base.get("prior_provider") or "gpu") == "gpu"
-    PREPARE_STEPS = ("quickshift", "felzenszwalb", "sift")
+    PREPARE_STEPS = ("quickshift", "SLIC", "felzenszwalb", "sift")
 
     def prepare_clips(step):
         # (measured, round 2: preparing the clips of a single-GPU run side by side instead of one after the other made the
@@ -252,7 +252,7 @@ def run_shard(items, base, polygons, device=0, videos_path="Input/SegTrack2/Vide
         """One kind of what all sequences of a clip share -- the label maps of an over-segmentation, or the SIFT features
         -- for every clip of the shard, in the same (step, clip) order on every rank: the ranks that share a clip split
         the per-frame host work and all-reduce the pieces (felzenszwalb, sift: calling thread of run_shard only; the
-        quickshift step involves no collective and may run on another thread)."""
+        quickshift and SLIC steps involve no collective and may run on another thread)."""
         needs = clip_needs(all_items or items)
         for v in order_v:
             cfg = sequence_config(base, polygons, v, items[0][3], videos_path, truth_path)
