@@ -150,7 +150,7 @@ int pcm_update(pcm_handle* h, const uint8_t* frame, int frame_h, int frame_w, in
  * whole map (default: on). */
 int pcm_set_label_cache(pcm_handle* h, int on);
 
-/* labels == NULL with no pcm_quickshift pending: the label map the previous pcm_update left on the device is used
+/* labels == NULL with no pcm_quickshift / pcm_slic_gpu pending: the label map the previous pcm_update left on the device is used
  * again (same crop size required; n_labels is ignored).  The caller vouches that the map has not changed -- the
  * plugin does this when its over-segmentation provider hands back the very same read-only array. */
 
@@ -201,7 +201,8 @@ int pcm_quickshift(pcm_handle* h, const uint8_t* frame, int frame_h, int frame_w
                    const double* noise, int32_t* labels_out, int* n_labels_out);
 
 /* Device variant: d_frame / d_noise (may be NULL: no noise) / d_labels_out (h*w int32, may be
- * NULL) are device pointers; waits for the stream to return the segment count. */
+ * NULL) are device pointers; waits for the stream to return the segment count.
+ * Limits: those of pcm_quickshift, and frame_stride >= 3 * frame_w. */
 int pcm_quickshift_device(pcm_handle* h, const uint8_t* d_frame, int frame_h, int frame_w, int64_t frame_stride,
                           const int rect[4], double ratio, double kernel_size, double max_dist,
                           const double* d_noise, int32_t* d_labels_out, int* n_labels_out);

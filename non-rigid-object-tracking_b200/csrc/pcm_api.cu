@@ -293,19 +293,24 @@ struct pcm_handle {
     std::vector<int> label_chunk_max;
     bool label_cache_on = true;   // pcm_set_label_cache
 
-    // quickshift over-segmentation (pcm_quickshift): scratch, the resident label map and the crop
-    // it was computed from (pcm_update with labels == NULL continues from here)
-    DevBuf qs_lab, qs_dens, qs_noise, qs_parent, qs_root, qs_flag, qs_rank, qs_sums, qs_labels, qs_lin, qs_count;
-    PinBuf h_noise;
-    int qs_cw = 0, qs_ch = 0, qs_n_labels = 0;
-    int qs_noise_cw = 0, qs_noise_ch = 0;
-    bool qs_valid = false;
-    const uint8_t* qs_frame_ptr = nullptr;     // host frame the resident crop was staged from
-    int qs_rect[4] = {0, 0, 0, 0};
+    // over-segmentation on the GPU (quickshift, SLIC): the label map of the last call, and the handoff to pcm_update with
+    // labels == NULL, armed by pcm_quickshift / pcm_slic_gpu: the crop `rect` of the host frame `frame` is in `frame` (the
+    // device buffer above) and its map of n_labels segments in seg_labels
+    DevBuf seg_labels;
+    struct {
+        bool valid;
+        const uint8_t* frame;
+        int rect[4];
+        int n_labels;
+    } handoff = {false, nullptr, {0, 0, 0, 0}, 0};
 
-    // SLIC over-segmentation (pcm_slic_gpu / pcm_slic_device): the label map goes to qs_labels (and the count to
-    // qs_n_labels), so that pcm_update(labels == NULL) continues from it as from a quickshift map.  sl_smooth, sl_img and
-    // sl_nearest keep the stage results of the last call (pcm_slic_debug_last).
+    // quickshift (pcm_quickshift*): scratch; the noise of the last call with noise and its crop size
+    DevBuf qs_lab, qs_dens, qs_noise, qs_parent, qs_root, qs_flag, qs_rank, qs_sums, qs_lin, qs_count;
+    PinBuf h_noise;
+    int qs_noise_cw = 0, qs_noise_ch = 0;
+
+    // SLIC (pcm_slic_gpu / pcm_slic_device*): scratch.  sl_smooth, sl_img and sl_nearest keep the stage results of the last
+    // call (pcm_slic_debug_last).
     DevBuf sl_kernel, sl_smooth, sl_tmp, sl_img, sl_centers, sl_dmin, sl_best, sl_nearest, sl_keys, sl_iota, sl_sidx, sl_begin,
            sl_end, sl_cub, sl_count;
     DevBuf sl_parent, sl_root, sl_csize, sl_piece, sl_psize, sl_off, sl_queue, sl_seen, sl_adj, sl_nxt, sl_val, sl_labels;
@@ -1311,14 +1316,14 @@ static int upload_priors(pcm_handle* h, const float* priors, int n, const float*
 }
 
 // pcm_update(labels == NULL): the crop pixels and the label map are the ones the preceding
-// pcm_quickshift on this handle left on the device
-static int update_from_quickshift(pcm_handle* h, const uint8_t* frame, int H, int W, int64_t stride, const int rect[4],
-                                  const float* priors, const pcm_update_params* params, uint8_t* mask,
-                                  int64_t mask_row_stride, int64_t mask_pixel_stride) {
+// pcm_quickshift or pcm_slic_gpu on this handle left on the device (h->handoff)
+static int update_from_handoff(pcm_handle* h, const uint8_t* frame, int H, int W, int64_t stride, const int rect[4],
+                               const float* priors, const pcm_update_params* params, uint8_t* mask,
+                               int64_t mask_row_stride, int64_t mask_pixel_stride) {
     if (!rect) return fail(PCM_E_INVALID, "pcm_update: NULL rect");
-    if (!h->qs_valid || h->qs_frame_ptr != frame || memcmp(h->qs_rect, rect, sizeof h->qs_rect) != 0)
+    if (!h->handoff.valid || h->handoff.frame != frame || memcmp(h->handoff.rect, rect, sizeof h->handoff.rect) != 0)
         return fail(PCM_E_STATE, "pcm_update: labels == NULL needs a preceding pcm_quickshift or pcm_slic_gpu of the same frame and rect");
-    int rc = validate_update(h, H, W, rect, h->qs_n_labels, params);
+    int rc = validate_update(h, H, W, rect, h->handoff.n_labels, params);
     if (rc) return rc;
     CUDA_TRY(cudaSetDevice(h->device));
     h->trace.start();
@@ -1329,12 +1334,12 @@ static int update_from_quickshift(pcm_handle* h, const uint8_t* frame, int H, in
     const float* d_priors = nullptr;
     if (priors) {
         CUDA_TRY(cudaStreamSynchronize(h->stream));
-        if ((rc = upload_priors(h, priors, h->qs_n_labels, &d_priors))) return rc;
+        if ((rc = upload_priors(h, priors, h->handoff.n_labels, &d_priors))) return rc;
     }
     h->trace.lap(HostTrace::UPD_STAGE);
     const int crop_rect[4] = {0, 0, cw, ch};
-    rc = enqueue_update(h, h->frame.as<uint8_t>(), ch, cw, (int64_t)cw * 3, crop_rect, h->qs_labels.as<int32_t>(),
-                        h->qs_n_labels, d_priors, params, h->mask.as<uint8_t>(), W, rect[0], rect[1], h->keep_pre);
+    rc = enqueue_update(h, h->frame.as<uint8_t>(), ch, cw, (int64_t)cw * 3, crop_rect, h->seg_labels.as<int32_t>(),
+                        h->handoff.n_labels, d_priors, params, h->mask.as<uint8_t>(), W, rect[0], rect[1], h->keep_pre);
     if (rc) return rc;
     h->trace.lap(HostTrace::UPD_ENQUEUE);
     return finish_host_update(h, rect, mask, mask_row_stride, mask_pixel_stride);
@@ -1356,8 +1361,8 @@ extern "C" int pcm_update(pcm_handle* h, const uint8_t* frame, int H, int W, int
                           const int32_t* labels, int n_labels, const float* priors, const pcm_update_params* params,
                           uint8_t* mask, int64_t mask_row_stride, int64_t mask_pixel_stride) {
     if (!h || !frame || !mask) return fail(PCM_E_INVALID, "pcm_update: NULL argument");
-    if (!labels && h->qs_valid) return update_from_quickshift(h, frame, H, W, stride, rect, priors, params, mask, mask_row_stride, mask_pixel_stride);
-    // labels == NULL without a pending quickshift: the label map of the previous pcm_update (same crop size) is still on
+    if (!labels && h->handoff.valid) return update_from_handoff(h, frame, H, W, stride, rect, priors, params, mask, mask_row_stride, mask_pixel_stride);
+    // labels == NULL without a pending handoff: the label map of the previous pcm_update (same crop size) is still on
     // the device and the caller vouches that it has not changed
     const bool reuse_labels = !labels;
     if (reuse_labels) {
@@ -1366,7 +1371,7 @@ extern "C" int pcm_update(pcm_handle* h, const uint8_t* frame, int H, int W, int
                                      "preceding pcm_update with a label map for a crop of the same size");
         n_labels = h->resident_labels;
     }
-    h->qs_valid = false;                               // the resident crop is about to be replaced
+    h->handoff.valid = false;                          // the resident crop is about to be replaced
     h->chain_tail = false;
     const bool auto_labels = n_labels <= 0;            // n_labels = max(label) + 1, found while staging
     if (auto_labels && priors) return fail(PCM_E_INVALID, "pcm_update: priors need an explicit n_labels");
@@ -1501,7 +1506,7 @@ extern "C" int pcm_iou(pcm_handle* h, const uint8_t* mask, int64_t mask_row_stri
     CUDA_TRY(h->counts.reserve(2 * sizeof(int64_t)));
     CUDA_TRY(h->h_small.reserve(64));
     CUDA_TRY(cudaStreamSynchronize(st));
-    h->qs_valid = false;                               // the frame scratch is reused for the truth image
+    h->handoff.valid = false;                          // the frame scratch is reused for the truth image
     h->chain_tail = false;
     h->trace.start();
     uint8_t* hm = h->h_mask.as<uint8_t>();
@@ -1603,11 +1608,113 @@ extern "C" int pcm_host_unregister(void* p) {
 }
 
 // ---------------------------------------------------------------------------------
+// over-segmentation on the GPU: the front end quickshift and SLIC share.  Each algorithm's enqueue_* queues it on a crop
+// of a device frame, writes the label map into h->seg_labels and leaves its count in a device word.
+// ---------------------------------------------------------------------------------
+// The checks and set-up every entry point below starts with.  The handoff ends here: the call replaces the label map,
+// and a host entry point also the staged crop.
+static int begin_seg(pcm_handle* h, const char* who, const uint8_t* frame, int H, int W, int64_t stride, const int rect[4]) {
+    if (!h || !frame || !rect) return fail(PCM_E_INVALID, "%s: NULL argument", who);
+    if (int rc = check_rect(who, rect, H, W)) return rc;
+    if (stride < (int64_t)W * 3) return fail(PCM_E_INVALID, "%s: stride %lld < 3*W", who, (long long)stride);
+    CUDA_TRY(cudaSetDevice(h->device));
+    h->handoff.valid = false;
+    return PCM_OK;
+}
+
+// Waits for the stream; *n = the device word d_count + bias (0: quickshift counts its segments; 1: SLIC leaves its largest
+// label, and pcm_slic counts largest label + 1)
+static int read_seg_count(pcm_handle* h, const int* d_count, int bias, int* n) {
+    CUDA_TRY(h->h_small.reserve(64));
+    int* hs = h->h_small.as<int>() + 8;
+    CUDA_TRY(cudaMemcpyAsync(hs, d_count, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
+    *n = *hs + bias;
+    return PCM_OK;
+}
+
+// Host entry points, before the algorithm: the crop rows of the host frame -> pinned -> h->frame (dense rows of 3 * w
+// bytes, where pcm_update with labels == NULL finds them), and n_extra items of the caller's in the same pool dispatch
+// (extra(i) stages item i and returns the error of the copy it queued)
+template <typename Extra>
+static int stage_crop(pcm_handle* h, const char* who, const uint8_t* frame, int64_t stride, const int rect[4], int n_extra,
+                      Extra&& extra) {
+    const int ch = rect[3];
+    const size_t row_bytes = (size_t)rect[2] * 3;
+    CUDA_TRY(h->h_frame.reserve(row_bytes * ch));
+    CUDA_TRY(h->frame.reserve(row_bytes * ch));
+    CUDA_TRY(cudaStreamSynchronize(h->stream));       // the staging buffers are reused between calls
+    const int frame_rows = rows_per_chunk((size_t)1 << 20, row_bytes);
+    const int n_frame_items = (ch + frame_rows - 1) / frame_rows;
+    const uint8_t* crop0 = frame + (size_t)rect[1] * stride + (size_t)rect[0] * 3;
+    uint8_t* hf = h->h_frame.as<uint8_t>();
+    uint8_t* df = h->frame.as<uint8_t>();
+    return stage_items(h, who, n_frame_items + n_extra, [&](int item) -> cudaError_t {
+        if (item >= n_frame_items) return extra(item - n_frame_items);
+        const int r0 = item * frame_rows;
+        return stage_rows(h, df, hf, crop0, (size_t)stride, row_bytes, r0, std::min(ch, r0 + frame_rows));
+    });
+}
+
+// Host entry points, after the algorithm: the label map to labels_out (when given), the count (read_seg_count), and the
+// handoff armed for this frame and rect
+static int finish_host_seg(pcm_handle* h, const uint8_t* frame, const int rect[4], const int* d_count, int bias,
+                           int32_t* labels_out, int* n_labels_out) {
+    const size_t label_bytes = (size_t)rect[2] * rect[3] * sizeof(int32_t);
+    if (labels_out) {
+        CUDA_TRY(h->h_labels.reserve(label_bytes));
+        h->label_cache_px = 0;                        // the pinned label buffer no longer mirrors `labels`
+        CUDA_TRY(cudaMemcpyAsync(h->h_labels.p, h->seg_labels.p, label_bytes, cudaMemcpyDeviceToHost, h->stream));
+        h->bytes_d2h += (int64_t)label_bytes;
+    }
+    int n = 0;
+    if (int rc = read_seg_count(h, d_count, bias, &n)) return rc;
+    if (n_labels_out) *n_labels_out = n;
+    if (labels_out) memcpy(labels_out, h->h_labels.p, label_bytes);
+    h->handoff = {true, frame, {rect[0], rect[1], rect[2], rect[3]}, n};
+    return PCM_OK;
+}
+
+// Device entry points: enqueue() queues the algorithm on the crop `rect` of d_frame; the map is then copied into
+// d_labels_out (when given) and the count read from h->*count (read_seg_count)
+template <typename Enqueue>
+static int seg_device(pcm_handle* h, const char* who, const uint8_t* d_frame, int H, int W, int64_t stride, const int rect[4],
+                      DevBuf pcm_handle::*count, int bias, int32_t* d_labels_out, int* n_labels_out, Enqueue&& enqueue) {
+    if (int rc = begin_seg(h, who, d_frame, H, W, stride, rect)) return rc;
+    if (int rc = enqueue()) return rc;
+    if (d_labels_out)
+        CUDA_TRY(cudaMemcpyAsync(d_labels_out, h->seg_labels.p, (size_t)rect[2] * rect[3] * sizeof(int32_t), cudaMemcpyDeviceToDevice,
+                                 h->stream));
+    int n = 0;
+    if (int rc = read_seg_count(h, (h->*count).as<int>(), bias, &n)) return rc;
+    if (n_labels_out) *n_labels_out = n;
+    return PCM_OK;
+}
+
+// The *_device_batch entry points: crop k = rects[4k .. 4k+3] of the frame d_frames + frame_index[k] * frame_bytes through
+// one(d_frame, rect, d_labels, &count), the single-crop entry point, into d_labels_out + label_offsets[k]
+template <typename One>
+static int seg_device_batch(pcm_handle* h, const char* who, int n, const uint8_t* d_frames, int64_t frame_bytes,
+                            const int32_t* frame_index, const int32_t* rects, int32_t* d_labels_out, const int64_t* label_offsets,
+                            int32_t* n_labels_out, One&& one) {
+    if (!h || !d_frames || !frame_index || !rects || !d_labels_out || !label_offsets || !n_labels_out)
+        return fail(PCM_E_INVALID, "%s: NULL argument", who);
+    if (n < 0 || frame_bytes < 0) return fail(PCM_E_INVALID, "%s: bad count / frame size", who);
+    for (int k = 0; k < n; ++k) {
+        if (frame_index[k] < 0 || label_offsets[k] < 0) return fail(PCM_E_INVALID, "%s: crop %d: negative index", who, k);
+        int count = 0;
+        const int rect[4] = {rects[4 * k], rects[4 * k + 1], rects[4 * k + 2], rects[4 * k + 3]};
+        if (int rc = one(d_frames + (int64_t)frame_index[k] * frame_bytes, rect, d_labels_out + label_offsets[k], &count)) return rc;
+        n_labels_out[k] = count;
+    }
+    return PCM_OK;
+}
+
+// ---------------------------------------------------------------------------------
 // API: quickshift over-segmentation (SURVEY.md §8 f-1)
 // ---------------------------------------------------------------------------------
 static int enqueue_quickshift(pcm_handle* h, const uint8_t* d_frame, int64_t stride, int cx, int cy, int cw, int ch,
-                              double ratio, double kernel_size, double max_dist, const double* d_noise,
-                              int32_t* d_labels_out) {
+                              double ratio, double kernel_size, double max_dist, const double* d_noise) {
     if (!(kernel_size >= 1.0)) return fail(PCM_E_INVALID, "quickshift: kernel_size must be >= 1");
     const int kw = (int)ceil(3.0 * kernel_size);
     if (kw > QS_MAX_KW) return fail(PCM_E_LIMIT, "quickshift: window half width %d > %d", kw, QS_MAX_KW);
@@ -1623,7 +1730,7 @@ static int enqueue_quickshift(pcm_handle* h, const uint8_t* d_frame, int64_t str
     CUDA_TRY(h->qs_rank.reserve(n * sizeof(int)));
     const int n_blocks = (int)((n + QS_SCAN_ELEMS - 1) / QS_SCAN_ELEMS);
     CUDA_TRY(h->qs_sums.reserve((size_t)n_blocks * sizeof(int)));
-    CUDA_TRY(h->qs_labels.reserve(n * sizeof(int32_t)));
+    CUDA_TRY(h->seg_labels.reserve(n * sizeof(int32_t)));
     CUDA_TRY(h->qs_count.reserve(sizeof(int)));
     if (!h->qs_lin.p) {
         // sRGB companding table of skimage.color.rgb2xyz for the 256 byte values
@@ -1687,117 +1794,64 @@ static int enqueue_quickshift(pcm_handle* h, const uint8_t* d_frame, int64_t str
     CHECK_LAUNCH(h, "qs_scan_sums_kernel");
     qs_scan_apply_kernel<<<n_blocks, 256, 0, st>>>(h->qs_flag.as<int>(), (int)n, h->qs_sums.as<int>(), h->qs_rank.as<int>());
     CHECK_LAUNCH(h, "qs_scan_apply_kernel");
-    qs_label_kernel<<<flat_blocks, 256, 0, st>>>(a.root, h->qs_rank.as<int>(), h->qs_labels.as<int32_t>(), (int)n);
+    qs_label_kernel<<<flat_blocks, 256, 0, st>>>(a.root, h->qs_rank.as<int>(), h->seg_labels.as<int32_t>(), (int)n);
     CHECK_LAUNCH(h, "qs_label_kernel");
-    if (d_labels_out) CUDA_TRY(cudaMemcpyAsync(d_labels_out, h->qs_labels.p, n * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
-    return PCM_OK;
-}
-
-static int read_qs_count(pcm_handle* h, int* n_labels_out) {
-    CUDA_TRY(h->h_small.reserve(64));
-    int* hs = h->h_small.as<int>() + 8;
-    CUDA_TRY(cudaMemcpyAsync(hs, h->qs_count.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(cudaStreamSynchronize(h->stream));
-    h->qs_n_labels = *hs;
-    if (n_labels_out) *n_labels_out = *hs;
     return PCM_OK;
 }
 
 extern "C" int pcm_quickshift_device(pcm_handle* h, const uint8_t* d_frame, int H, int W, int64_t stride, const int rect[4],
                                      double ratio, double kernel_size, double max_dist, const double* d_noise,
                                      int32_t* d_labels_out, int* n_labels_out) {
-    if (!h || !d_frame || !rect) return fail(PCM_E_INVALID, "pcm_quickshift_device: NULL argument");
-    int rc = check_rect("pcm_quickshift_device", rect, H, W);
-    if (rc) return rc;
-    CUDA_TRY(cudaSetDevice(h->device));
-    h->qs_valid = false;
-    rc = enqueue_quickshift(h, d_frame, stride, rect[0], rect[1], rect[2], rect[3], ratio, kernel_size, max_dist, d_noise,
-                                d_labels_out);
-    if (rc) return rc;
-    return read_qs_count(h, n_labels_out);
+    return seg_device(h, "pcm_quickshift_device", d_frame, H, W, stride, rect, &pcm_handle::qs_count, 0, d_labels_out, n_labels_out,
+                      [&] {
+                          return enqueue_quickshift(h, d_frame, stride, rect[0], rect[1], rect[2], rect[3], ratio, kernel_size,
+                                                    max_dist, d_noise);
+                      });
 }
 
 extern "C" int pcm_quickshift_device_batch(pcm_handle* h, int n, const uint8_t* d_frames, int64_t frame_bytes,
                                            const int32_t* frame_index, int H, int W, int64_t stride, const int32_t* rects,
                                            double ratio, double kernel_size, double max_dist, const double* d_noise,
                                            int32_t* d_labels_out, const int64_t* label_offsets, int32_t* n_labels_out) {
-    if (!h || !d_frames || !frame_index || !rects || !d_labels_out || !label_offsets || !n_labels_out)
-        return fail(PCM_E_INVALID, "pcm_quickshift_device_batch: NULL argument");
-    if (n < 0 || frame_bytes < 0) return fail(PCM_E_INVALID, "pcm_quickshift_device_batch: bad count / frame size");
-    for (int k = 0; k < n; ++k) {
-        if (frame_index[k] < 0 || label_offsets[k] < 0) return fail(PCM_E_INVALID, "pcm_quickshift_device_batch: crop %d: negative index", k);
-        int count = 0;
-        const int rect[4] = {rects[4 * k], rects[4 * k + 1], rects[4 * k + 2], rects[4 * k + 3]};
-        const int rc = pcm_quickshift_device(h, d_frames + (int64_t)frame_index[k] * frame_bytes, H, W, stride, rect, ratio, kernel_size,
-                                             max_dist, d_noise, d_labels_out + label_offsets[k], &count);
-        if (rc) return rc;
-        n_labels_out[k] = count;
-    }
-    return PCM_OK;
+    return seg_device_batch(h, "pcm_quickshift_device_batch", n, d_frames, frame_bytes, frame_index, rects, d_labels_out, label_offsets,
+                            n_labels_out, [&](const uint8_t* d_frame, const int rect[4], int32_t* d_labels, int* count) {
+                                return pcm_quickshift_device(h, d_frame, H, W, stride, rect, ratio, kernel_size, max_dist, d_noise,
+                                                             d_labels, count);
+                            });
 }
 
 extern "C" int pcm_quickshift(pcm_handle* h, const uint8_t* frame, int H, int W, int64_t stride, const int rect[4],
                               double ratio, double kernel_size, double max_dist, const double* noise,
                               int32_t* labels_out, int* n_labels_out) {
-    if (!h || !frame || !rect) return fail(PCM_E_INVALID, "pcm_quickshift: NULL argument");
-    int rc = check_rect("pcm_quickshift", rect, H, W);
+    int rc = begin_seg(h, "pcm_quickshift", frame, H, W, stride, rect);
     if (rc) return rc;
-    if (stride < (int64_t)W * 3) return fail(PCM_E_INVALID, "pcm_quickshift: stride %lld < 3*W", (long long)stride);
-    CUDA_TRY(cudaSetDevice(h->device));
-    const int cx = rect[0], cy = rect[1], cw = rect[2], ch = rect[3];
-    const size_t npx = (size_t)cw * ch, row_bytes = (size_t)cw * 3;
-    cudaStream_t st = h->stream;
-    h->qs_valid = false;
-    CUDA_TRY(h->h_frame.reserve(npx * 3));
-    CUDA_TRY(h->frame.reserve(npx * 3));
+    const int cw = rect[2], ch = rect[3];
+    const size_t npx = (size_t)cw * ch;
     if (noise) {
         CUDA_TRY(h->h_noise.reserve(npx * sizeof(double)));
         CUDA_TRY(h->qs_noise.reserve(npx * sizeof(double)));
     } else if (h->qs_noise_cw != cw || h->qs_noise_ch != ch) {
         return fail(PCM_E_STATE, "pcm_quickshift: noise == NULL needs a previous call with noise for the same %dx%d crop", cw, ch);
     }
-    CUDA_TRY(cudaStreamSynchronize(st));
-    // crop rows (and, when given, the tie-breaking noise) -> pinned -> device, one pool dispatch
+    // the tie-breaking noise, when given, travels with the crop rows
     constexpr size_t CHUNK = 1u << 20;
-    const int frame_rows = rows_per_chunk(CHUNK, row_bytes);
-    const int n_frame_items = (ch + frame_rows - 1) / frame_rows;
     const size_t noise_bytes = noise ? npx * sizeof(double) : 0;
-    const int n_noise_items = (int)((noise_bytes + CHUNK - 1) / CHUNK);
-    const uint8_t* crop0 = frame + (size_t)cy * stride + (size_t)cx * 3;
-    uint8_t* hf = h->h_frame.as<uint8_t>();
-    uint8_t* df = h->frame.as<uint8_t>();
     uint8_t* hn = h->h_noise.as<uint8_t>();
     uint8_t* dn = h->qs_noise.as<uint8_t>();
     const uint8_t* nsrc = reinterpret_cast<const uint8_t*>(noise);
-    rc = stage_items(h, "pcm_quickshift", n_frame_items + n_noise_items, [&](int item) -> cudaError_t {
-        if (item < n_frame_items) {
-            const int r0 = item * frame_rows;
-            return stage_rows(h, df, hf, crop0, (size_t)stride, row_bytes, r0, std::min(ch, r0 + frame_rows));
-        }
-        const size_t o = (size_t)(item - n_frame_items) * CHUNK, len = std::min(CHUNK, noise_bytes - o);
+    rc = stage_crop(h, "pcm_quickshift", frame, stride, rect, (int)((noise_bytes + CHUNK - 1) / CHUNK), [&](int item) -> cudaError_t {
+        const size_t o = (size_t)item * CHUNK, len = std::min(CHUNK, noise_bytes - o);
         memcpy(hn + o, nsrc + o, len);
-        const cudaError_t e = cudaMemcpyAsync(dn + o, hn + o, len, cudaMemcpyHostToDevice, st);
+        const cudaError_t e = cudaMemcpyAsync(dn + o, hn + o, len, cudaMemcpyHostToDevice, h->stream);
         h->bytes_h2d += (int64_t)len;
         return e;
     });
     if (rc) return rc;
     if (noise) { h->qs_noise_cw = cw; h->qs_noise_ch = ch; }
-    rc = enqueue_quickshift(h, df, (int64_t)row_bytes, 0, 0, cw, ch, ratio, kernel_size, max_dist, h->qs_noise.as<double>(), nullptr);
+    rc = enqueue_quickshift(h, h->frame.as<uint8_t>(), (int64_t)cw * 3, 0, 0, cw, ch, ratio, kernel_size, max_dist,
+                            h->qs_noise.as<double>());
     if (rc) return rc;
-    if (labels_out) {
-        CUDA_TRY(h->h_labels.reserve(npx * sizeof(int32_t)));
-        h->label_cache_px = 0;                        // the pinned label buffer no longer mirrors `labels`
-        CUDA_TRY(cudaMemcpyAsync(h->h_labels.p, h->qs_labels.p, npx * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        h->bytes_d2h += (int64_t)(npx * sizeof(int32_t));
-    }
-    rc = read_qs_count(h, n_labels_out);
-    if (rc) return rc;
-    if (labels_out) memcpy(labels_out, h->h_labels.p, npx * sizeof(int32_t));
-    h->qs_cw = cw; h->qs_ch = ch;
-    h->qs_frame_ptr = frame;
-    memcpy(h->qs_rect, rect, sizeof h->qs_rect);
-    h->qs_valid = true;
-    return PCM_OK;
+    return finish_host_seg(h, frame, rect, h->qs_count.as<int>(), 0, labels_out, n_labels_out);
 }
 
 extern "C" int pcm_felzenszwalb(const uint8_t* frame, int H, int W, int64_t stride, const int rect[4], double scale,
@@ -1814,14 +1868,24 @@ extern "C" int pcm_felzenszwalb(const uint8_t* frame, int H, int W, int64_t stri
     return PCM_OK;
 }
 
+// the arguments of pcm_slic and its GPU variants besides the frame and a crop rect already checked with check_rect
+static int check_slic_args(const char* who, const int rect[4], int n_segments, double compactness, int max_iter, int start_label,
+                           const double* kernel, int kernel_radius) {
+    if ((long long)rect[2] * rect[3] > (1LL << 28)) return fail(PCM_E_LIMIT, "%s: crop too large (more than 2^28 pixels)", who);
+    if (n_segments < 1) return fail(PCM_E_INVALID, "%s: n_segments %d < 1", who, n_segments);
+    if (!(compactness > 0)) return fail(PCM_E_INVALID, "%s: compactness must be > 0", who);
+    if (max_iter < 0) return fail(PCM_E_INVALID, "%s: max_iter %d < 0", who, max_iter);
+    if (start_label < 0) return fail(PCM_E_INVALID, "%s: start_label %d", who, start_label);
+    if (kernel && kernel_radius < 0) return fail(PCM_E_INVALID, "%s: kernel_radius %d", who, kernel_radius);
+    return PCM_OK;
+}
+
 extern "C" int pcm_slic(const uint8_t* frame, int H, int W, int64_t stride, const int rect[4], int n_segments,
                         double compactness, double sigma, const double* kernel, int kernel_radius, int max_iter,
                         int start_label, int32_t* labels_out, int* n_labels_out) {
     if (!frame || !rect || !labels_out) return fail(PCM_E_INVALID, "pcm_slic: NULL argument");
     if (int rc = check_rect("pcm_slic", rect, H, W)) return rc;
-    if ((long long)rect[2] * rect[3] > (1LL << 28)) return fail(PCM_E_LIMIT, "pcm_slic: crop too large");
-    if (kernel && kernel_radius < 0) return fail(PCM_E_INVALID, "pcm_slic: kernel_radius %d", kernel_radius);
-    if (start_label < 0) return fail(PCM_E_INVALID, "pcm_slic: start_label %d", start_label);
+    if (int rc = check_slic_args("pcm_slic", rect, n_segments, compactness, max_iter, start_label, kernel, kernel_radius)) return rc;
     const int n = slic(frame, stride, rect[0], rect[1], rect[2], rect[3], n_segments, compactness, sigma, kernel, kernel_radius,
                        max_iter, start_label, labels_out);
     if (n < 0) return fail(PCM_E_INVALID, "pcm_slic: bad arguments (n_segments >= 1, compactness > 0, max_iter >= 0)");
@@ -1872,18 +1936,6 @@ static bool slic_seed_grid(int h, int w, int n_points, int& start_y, int& step_y
 }
 
 static int bit_length(unsigned v) { int b = 0; while (v) { ++b; v >>= 1; } return b; }
-
-static int check_slic_args(const char* who, const int rect[4], int H, int W, int n_segments, double compactness, int max_iter,
-                           int start_label, const double* kernel, int kernel_radius) {
-    if (int rc = check_rect(who, rect, H, W)) return rc;
-    if ((long long)rect[2] * rect[3] > (1LL << 28)) return fail(PCM_E_LIMIT, "%s: crop too large (more than 2^28 pixels)", who);
-    if (n_segments < 1) return fail(PCM_E_INVALID, "%s: n_segments %d < 1", who, n_segments);
-    if (!(compactness > 0)) return fail(PCM_E_INVALID, "%s: compactness must be > 0", who);
-    if (max_iter < 0) return fail(PCM_E_INVALID, "%s: max_iter %d < 0", who, max_iter);
-    if (start_label < 0) return fail(PCM_E_INVALID, "%s: start_label %d", who, start_label);
-    if (kernel && kernel_radius < 0) return fail(PCM_E_INVALID, "%s: kernel_radius %d", who, kernel_radius);
-    return PCM_OK;
-}
 
 // CUB scratch for a stable sort of n (int key, int value) pairs and an exclusive sum of n ints
 static int reserve_slic_cub(pcm_handle* h, int n, size_t* bytes) {
@@ -1956,11 +2008,10 @@ static int enqueue_slic_connectivity(pcm_handle* h, const int32_t* d_seg, int w,
     return PCM_OK;
 }
 
-// The whole SLIC of the crop (cx, cy, w, hh) of a device frame into qs_labels (and d_labels_out when given).  Asynchronous
-// apart from the host-side staging of the weights and seeds; the caller waits for sl_count (read_slic_count).
+// The whole SLIC of the crop (cx, cy, w, hh) of a device frame into seg_labels.  Asynchronous apart from the host-side
+// staging of the weights and seeds; the largest label goes to sl_count.
 static int enqueue_slic(pcm_handle* h, const uint8_t* d_frame, int64_t stride, int cx, int cy, int w, int hh, int n_segments,
-                        double compactness, double sigma, const double* kernel, int radius, int max_iter, int start_label,
-                        int32_t* d_labels_out) {
+                        double compactness, double sigma, const double* kernel, int radius, int max_iter, int start_label) {
     const int n = w * hh;
     cudaStream_t st = h->stream;
     h->chain_tail = false;
@@ -2006,7 +2057,7 @@ static int enqueue_slic(pcm_handle* h, const uint8_t* d_frame, int64_t stride, i
     for (DevBuf* b : {&h->sl_best, &h->sl_nearest, &h->sl_keys, &h->sl_iota, &h->sl_sidx}) CUDA_TRY(b->reserve(ib));
     CUDA_TRY(h->sl_begin.reserve((size_t)K * sizeof(int)));
     CUDA_TRY(h->sl_end.reserve((size_t)K * sizeof(int)));
-    CUDA_TRY(h->qs_labels.reserve(ib));
+    CUDA_TRY(h->seg_labels.reserve(ib));
     size_t cub_bytes = 0;
     if (int rc = reserve_slic_cub(h, n, &cub_bytes)) return rc;
     if (nk) CUDA_TRY(cudaMemcpyAsync(h->sl_kernel.p, hk, nk * sizeof(double), cudaMemcpyHostToDevice, st));
@@ -2059,104 +2110,45 @@ static int enqueue_slic(pcm_handle* h, const uint8_t* d_frame, int64_t stride, i
     // connectivity: min_size_factor 0.5, max_size_factor 3 of the requested segment size
     const double segment_size = (double)hh * (double)w / n_segments;
     const long long min_size = (long long)(0.5 * segment_size), max_size = (long long)(3 * segment_size);
-    if (int rc = enqueue_slic_connectivity(h, nearest, w, hh, min_size, max_size, start_label, h->qs_labels.as<int32_t>())) return rc;
-    if (d_labels_out) CUDA_TRY(cudaMemcpyAsync(d_labels_out, h->qs_labels.p, ib, cudaMemcpyDeviceToDevice, st));
+    if (int rc = enqueue_slic_connectivity(h, nearest, w, hh, min_size, max_size, start_label, h->seg_labels.as<int32_t>())) return rc;
     h->sl_w = w; h->sl_h = hh;
-    return PCM_OK;
-}
-
-// waits for the stream; *n_labels = largest label + 1, as pcm_slic counts
-static int read_slic_count(pcm_handle* h, int* n_labels) {
-    CUDA_TRY(h->h_small.reserve(64));
-    int* hs = h->h_small.as<int>() + 12;
-    CUDA_TRY(cudaMemcpyAsync(hs, h->sl_count.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(cudaStreamSynchronize(h->stream));
-    *n_labels = *hs + 1;
     return PCM_OK;
 }
 
 extern "C" int pcm_slic_device(pcm_handle* h, const uint8_t* d_frame, int H, int W, int64_t stride, const int rect[4],
                                int n_segments, double compactness, double sigma, const double* kernel, int kernel_radius,
                                int max_iter, int start_label, int32_t* d_labels_out, int* n_labels_out) {
-    if (!h || !d_frame || !rect) return fail(PCM_E_INVALID, "pcm_slic_device: NULL argument");
-    int rc = check_slic_args("pcm_slic_device", rect, H, W, n_segments, compactness, max_iter, start_label, kernel, kernel_radius);
-    if (rc) return rc;
-    if (stride < (int64_t)W * 3) return fail(PCM_E_INVALID, "pcm_slic_device: stride %lld < 3*W", (long long)stride);
-    CUDA_TRY(cudaSetDevice(h->device));
-    h->qs_valid = false;
-    CUDA_TRY(cudaStreamSynchronize(h->stream));      // the pinned seed buffer is reused between calls
-    rc = enqueue_slic(h, d_frame, stride, rect[0], rect[1], rect[2], rect[3], n_segments, compactness, sigma, kernel, kernel_radius,
-                      max_iter, start_label, d_labels_out);
-    if (rc) return rc;
-    int count = 0;
-    if ((rc = read_slic_count(h, &count))) return rc;
-    if (n_labels_out) *n_labels_out = count;
-    return PCM_OK;
+    return seg_device(h, "pcm_slic_device", d_frame, H, W, stride, rect, &pcm_handle::sl_count, 1, d_labels_out, n_labels_out, [&] {
+        if (int rc = check_slic_args("pcm_slic_device", rect, n_segments, compactness, max_iter, start_label, kernel, kernel_radius))
+            return rc;
+        CUDA_TRY(cudaStreamSynchronize(h->stream));      // the pinned seed buffer is reused between calls
+        return enqueue_slic(h, d_frame, stride, rect[0], rect[1], rect[2], rect[3], n_segments, compactness, sigma, kernel,
+                            kernel_radius, max_iter, start_label);
+    });
 }
 
 extern "C" int pcm_slic_device_batch(pcm_handle* h, int n, const uint8_t* d_frames, int64_t frame_bytes, const int32_t* frame_index,
                                      int H, int W, int64_t stride, const int32_t* rects, int n_segments, double compactness,
                                      double sigma, const double* kernel, int kernel_radius, int max_iter, int start_label,
                                      int32_t* d_labels_out, const int64_t* label_offsets, int32_t* n_labels_out) {
-    if (!h || !d_frames || !frame_index || !rects || !d_labels_out || !label_offsets || !n_labels_out)
-        return fail(PCM_E_INVALID, "pcm_slic_device_batch: NULL argument");
-    if (n < 0 || frame_bytes < 0) return fail(PCM_E_INVALID, "pcm_slic_device_batch: bad count / frame size");
-    for (int k = 0; k < n; ++k) {
-        if (frame_index[k] < 0 || label_offsets[k] < 0) return fail(PCM_E_INVALID, "pcm_slic_device_batch: crop %d: negative index", k);
-        int count = 0;
-        const int rect[4] = {rects[4 * k], rects[4 * k + 1], rects[4 * k + 2], rects[4 * k + 3]};
-        const int rc = pcm_slic_device(h, d_frames + (int64_t)frame_index[k] * frame_bytes, H, W, stride, rect, n_segments, compactness,
-                                       sigma, kernel, kernel_radius, max_iter, start_label, d_labels_out + label_offsets[k], &count);
-        if (rc) return rc;
-        n_labels_out[k] = count;
-    }
-    return PCM_OK;
+    return seg_device_batch(h, "pcm_slic_device_batch", n, d_frames, frame_bytes, frame_index, rects, d_labels_out, label_offsets,
+                            n_labels_out, [&](const uint8_t* d_frame, const int rect[4], int32_t* d_labels, int* count) {
+                                return pcm_slic_device(h, d_frame, H, W, stride, rect, n_segments, compactness, sigma, kernel,
+                                                       kernel_radius, max_iter, start_label, d_labels, count);
+                            });
 }
 
 extern "C" int pcm_slic_gpu(pcm_handle* h, const uint8_t* frame, int H, int W, int64_t stride, const int rect[4], int n_segments,
                             double compactness, double sigma, const double* kernel, int kernel_radius, int max_iter,
                             int start_label, int32_t* labels_out, int* n_labels_out) {
-    if (!h || !frame || !rect) return fail(PCM_E_INVALID, "pcm_slic_gpu: NULL argument");
-    int rc = check_slic_args("pcm_slic_gpu", rect, H, W, n_segments, compactness, max_iter, start_label, kernel, kernel_radius);
+    int rc = begin_seg(h, "pcm_slic_gpu", frame, H, W, stride, rect);
     if (rc) return rc;
-    if (stride < (int64_t)W * 3) return fail(PCM_E_INVALID, "pcm_slic_gpu: stride %lld < 3*W", (long long)stride);
-    CUDA_TRY(cudaSetDevice(h->device));
-    const int cx = rect[0], cy = rect[1], cw = rect[2], ch = rect[3];
-    const size_t npx = (size_t)cw * ch, row_bytes = (size_t)cw * 3;
-    cudaStream_t st = h->stream;
-    h->qs_valid = false;
-    CUDA_TRY(h->h_frame.reserve(npx * 3));
-    CUDA_TRY(h->frame.reserve(npx * 3));
-    CUDA_TRY(cudaStreamSynchronize(st));
-    // crop rows -> pinned -> device, one pool dispatch (the crop stays there for pcm_update with labels == NULL)
-    const int frame_rows = rows_per_chunk((size_t)1 << 20, row_bytes);
-    const uint8_t* crop0 = frame + (size_t)cy * stride + (size_t)cx * 3;
-    uint8_t* hf = h->h_frame.as<uint8_t>();
-    uint8_t* df = h->frame.as<uint8_t>();
-    rc = stage_items(h, "pcm_slic_gpu", (ch + frame_rows - 1) / frame_rows, [&](int item) -> cudaError_t {
-        const int r0 = item * frame_rows;
-        return stage_rows(h, df, hf, crop0, (size_t)stride, row_bytes, r0, std::min(ch, r0 + frame_rows));
-    });
+    if ((rc = check_slic_args("pcm_slic_gpu", rect, n_segments, compactness, max_iter, start_label, kernel, kernel_radius))) return rc;
+    if ((rc = stage_crop(h, "pcm_slic_gpu", frame, stride, rect, 0, [](int) { return cudaSuccess; }))) return rc;
+    rc = enqueue_slic(h, h->frame.as<uint8_t>(), (int64_t)rect[2] * 3, 0, 0, rect[2], rect[3], n_segments, compactness, sigma, kernel,
+                      kernel_radius, max_iter, start_label);
     if (rc) return rc;
-    rc = enqueue_slic(h, df, (int64_t)row_bytes, 0, 0, cw, ch, n_segments, compactness, sigma, kernel, kernel_radius, max_iter,
-                      start_label, nullptr);
-    if (rc) return rc;
-    if (labels_out) {
-        CUDA_TRY(h->h_labels.reserve(npx * sizeof(int32_t)));
-        h->label_cache_px = 0;                        // the pinned label buffer no longer mirrors `labels`
-        CUDA_TRY(cudaMemcpyAsync(h->h_labels.p, h->qs_labels.p, npx * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        h->bytes_d2h += (int64_t)(npx * sizeof(int32_t));
-    }
-    int count = 0;
-    if ((rc = read_slic_count(h, &count))) return rc;
-    if (n_labels_out) *n_labels_out = count;
-    if (labels_out) memcpy(labels_out, h->h_labels.p, npx * sizeof(int32_t));
-    h->qs_n_labels = count;
-    h->qs_cw = cw; h->qs_ch = ch;
-    h->qs_frame_ptr = frame;
-    memcpy(h->qs_rect, rect, sizeof h->qs_rect);
-    h->qs_valid = true;
-    return PCM_OK;
+    return finish_host_seg(h, frame, rect, h->sl_count.as<int>(), 1, labels_out, n_labels_out);
 }
 
 extern "C" int pcm_slic_connectivity(pcm_handle* h, const int32_t* nearest, int width, int height, long long min_size,
@@ -2177,7 +2169,7 @@ extern "C" int pcm_slic_connectivity(pcm_handle* h, const int32_t* nearest, int 
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(labels_out, h->sl_labels.p, ib, cudaMemcpyDeviceToHost, st));
     int count = 0;
-    if ((rc = read_slic_count(h, &count))) return rc;
+    if ((rc = read_seg_count(h, h->sl_count.as<int>(), 1, &count))) return rc;
     if (n_labels_out) *n_labels_out = count;
     return PCM_OK;
 }

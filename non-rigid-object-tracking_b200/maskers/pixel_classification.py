@@ -70,17 +70,12 @@ class PixelClassificationNonRigidMasker(Masker):
         self.spaces = tokens[1].split("_")
         self.native = capi.Handle(device)
         self.native.set_features(self.n_neighbors, self.spaces)
-        # over-segmentation (:70-75), SURVEY §8 f-1: quickshift and SLIC run on the GPU (pcm_quickshift, pcm_slic_gpu),
-        # felzenszwalb in the library's host code (pcm_felzenszwalb: inherently sequential).  config `slic_provider`:
-        # "gpu" (default) or "host" (pcm_slic, the library's host code; same labels)
-        self.native_quickshift = segment_fn is None and params["over_segmentation"] == "quickshift"
-        self.native_felzenszwalb = segment_fn is None and params["over_segmentation"] == "felzenszwalb"
-        self.native_slic = segment_fn is None and params["over_segmentation"] == "SLIC"
-        self.slic_provider = self.config.get("slic_provider") or "gpu"
-        if self.slic_provider not in ("gpu", "host"):
-            raise ValueError("slic_provider must be gpu or host, got %r" % (self.slic_provider,))
-        self.segment_fn = segment_fn or (None if (self.native_quickshift or self.native_felzenszwalb or self.native_slic)
-                                         else make_segment_provider(params["over_segmentation"]))
+        # over-segmentation (:70-75), SURVEY §8 f-1, by the library unless segment_fn is given: native_seg is the
+        # algorithm it runs, or None.  quickshift and SLIC run on the GPU (pcm_quickshift, pcm_slic_gpu), felzenszwalb in
+        # the library's host code (pcm_felzenszwalb: inherently sequential)
+        method = params["over_segmentation"]
+        self.native_seg = method if segment_fn is None and method in ("quickshift", "SLIC", "felzenszwalb") else None
+        self.segment_fn = segment_fn or (None if self.native_seg else make_segment_provider(method))
         self._qs_noise_shape = None
         self._seg_prev = None                  # (provider's array object, crop shape) of the label map resident on the device
         self.reuse_resident_labels = True      # False: every update sends its label map, whatever the provider returns
@@ -211,13 +206,13 @@ class PixelClassificationNonRigidMasker(Masker):
             return self.prior_fn(self.prevFrame, self.prevForegroundMask, crop, segs, n)
         n_labels, priors = 0, None             # 0: the library takes max(label) + 1 while staging
         same_labels, self._seg_next = False, None
-        if self.native_quickshift or (self.native_slic and self.slic_provider == "gpu"):
+        if self.native_seg in ("quickshift", "SLIC"):
             # quickshift(crop, kernel_size=3, max_dist=6, ratio=0.5, random_seed=42) (:71) or
             # slic(crop, n_segments=250, compactness=10, sigma=1, start_label=0) (:75) on the GPU; the label
             # map stays on the device and only travels to the host when the SIFT prior needs it
             if frame.strides[2] != 1 or frame.strides[1] != 3:
                 frame = np.ascontiguousarray(frame)
-            if self.native_quickshift:
+            if self.native_seg == "quickshift":
                 noise = None
                 if self._qs_noise_shape != (h, w):
                     noise = np.random.RandomState(42).normal(scale=0.00001, size=(h, w))
@@ -234,7 +229,7 @@ class PixelClassificationNonRigidMasker(Masker):
                     priors = prior(segments, n_labels)
             segments = None                    # update() continues from the device-resident map
         else:
-            if self.native_felzenszwalb:
+            if self.native_seg == "felzenszwalb":
                 # felzenszwalb(crop, scale=100, sigma=0.5, min_size=50) (:73).  In a sweep the label map
                 # of (clip, frame, crop) is the same for every hyper-parameter combination: shared
                 # through the model cache when the caller says the frames are the clip's (cache_tag)
@@ -246,10 +241,6 @@ class PixelClassificationNonRigidMasker(Masker):
                         segments, n_labels = cache.get_or_compute((self.cache_tag, "felzenszwalb", self.index, (x, y, w, h)), segment)
                     else:
                         segments, n_labels = segment()
-            elif self.native_slic:
-                # slic(crop, n_segments=250, compactness=10, sigma=1, start_label=0) (:75), slic_provider "host"
-                with stages.stage("slic"):
-                    segments, n_labels = capi.slic(frame, (x, y, w, h), n_segments=250, compactness=10.0, sigma=1.0, start_label=0)
             else:
                 raw = self.segment_fn(crop)
                 # a provider that hands back the very same READ-ONLY array vouches that the map has not changed: it is

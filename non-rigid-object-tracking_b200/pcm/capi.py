@@ -156,6 +156,18 @@ def crop_rect(bbox, frame_h, frame_w):
     return tuple(out)
 
 
+def _packed(frame):                    # an HxWx3 uint8 array with packed pixels: the library reads it in place
+    return frame.dtype == np.uint8 and frame.ndim == 3 and frame.shape[2] == 3 and frame.strides[2] == 1 and frame.strides[1] == 3
+
+
+def _batch_args(frame_index, rects, label_offsets):
+    fi, off = np.ascontiguousarray(frame_index, np.int32), np.ascontiguousarray(label_offsets, np.int64)
+    rc = np.ascontiguousarray(rects, np.int32).reshape(-1, 4)
+    if not (len(fi) == len(rc) == len(off)):
+        raise ValueError("frame_index, rects and label_offsets must have one entry per crop")
+    return fi, rc, off, np.zeros(len(fi), np.int32)
+
+
 def _gaussian_weights(sigma):
     """(weights, radius) of the 1-D Gaussian filter scipy.ndimage applies for `sigma` (truncated at 4 sigma);
     (None, 0) when sigma is not positive."""
@@ -172,7 +184,7 @@ def felzenszwalb(frame, rect, scale=100, sigma=0.5, min_size=50):
     pixel_classification.py:73).  Host code in the library; returns (labels int32 HxW, n_labels).
     The Gaussian weights are computed here the way scipy.ndimage does."""
     lib = load_library()
-    if frame.dtype != np.uint8 or frame.ndim != 3 or frame.shape[2] != 3 or frame.strides[2] != 1 or frame.strides[1] != 3:
+    if not _packed(frame):
         frame = np.ascontiguousarray(frame, np.uint8)
     r = (C.c_int * 4)(*[int(v) for v in rect])
     kernel, radius = _gaussian_weights(sigma)
@@ -189,7 +201,7 @@ def slic(frame, rect, n_segments=250, compactness=10.0, sigma=1.0, max_iter=10, 
     """SLIC superpixels of the crop `rect` (defaults = the reference's call, pixel_classification.py:75).  Host code in the
     library; returns (labels int32 HxW, n_labels).  The Gaussian weights are computed here the way scipy.ndimage does."""
     lib = load_library()
-    if frame.dtype != np.uint8 or frame.ndim != 3 or frame.shape[2] != 3 or frame.strides[2] != 1 or frame.strides[1] != 3:
+    if not _packed(frame):
         frame = np.ascontiguousarray(frame, np.uint8)
     r = (C.c_int * 4)(*[int(v) for v in rect])
     kernel, radius = _gaussian_weights(sigma)
@@ -374,8 +386,7 @@ class Handle:
 
     def update(self, frame, rect, labels, n_labels, priors, params, mask, channel=2):
         """Host-buffer update: writes channel `channel` of `mask` (HxWxC u8) inside `rect`."""
-        if frame.dtype != np.uint8 or frame.ndim != 3 or frame.shape[2] != 3 or frame.strides[2] != 1 \
-                or frame.strides[1] != 3:
+        if not _packed(frame):
             frame = np.ascontiguousarray(frame, np.uint8)
         if mask.dtype != np.uint8 or mask.strides[-1] != 1 and mask.ndim == 3:
             raise ValueError("mask must be a uint8 array with unit channel stride")
@@ -401,8 +412,7 @@ class Handle:
         pixel_classification.py:71).  Returns (labels int32 HxW or None, n_labels); the map also
         stays on the device for `update(..., labels=None)`.  `noise`: h*w float64 tie-breaking
         noise, or None to reuse the previous call's (same crop size)."""
-        if frame.dtype != np.uint8 or frame.ndim != 3 or frame.shape[2] != 3 or frame.strides[2] != 1 \
-                or frame.strides[1] != 3:
+        if not _packed(frame):
             raise ValueError("frame must be an HxWx3 uint8 array with packed pixels")
         r = (C.c_int * 4)(*[int(v) for v in rect])
         nz = None if noise is None else np.ascontiguousarray(noise, np.float64)
@@ -431,12 +441,7 @@ class Handle:
         """quickshift_device for many crops of a device-resident clip in ONE native call (pcm_quickshift_device_batch):
         crop k = rects[k] of frame frame_index[k], label map at d_labels_out + 4 * label_offsets[k].  Returns the
         segment counts (int32 array)."""
-        fi = np.ascontiguousarray(frame_index, np.int32)
-        rc = np.ascontiguousarray(rects, np.int32).reshape(-1, 4)
-        off = np.ascontiguousarray(label_offsets, np.int64)
-        if not (len(fi) == len(rc) == len(off)):
-            raise ValueError("frame_index, rects and label_offsets must have one entry per crop")
-        counts = np.zeros(len(fi), np.int32)
+        fi, rc, off, counts = _batch_args(frame_index, rects, label_offsets)
         self._check(self.lib.pcm_quickshift_device_batch(self._h, len(fi), C.c_void_p(d_frames), int(frame_bytes), _ptr(fi), int(frame_h),
                                                          int(frame_w), int(stride), _ptr(rc), float(ratio), float(kernel_size),
                                                          float(max_dist), C.c_void_p(d_noise) if d_noise else None,
@@ -449,8 +454,7 @@ class Handle:
         pixel_classification.py:75): the labels and count of the host `capi.slic`.  Returns (labels int32 HxW or None,
         n_labels); the map also stays on the device for `update(..., labels=None)`.  `kernel`: Gaussian weights, or None
         to compute them from sigma as scipy.ndimage does."""
-        if frame.dtype != np.uint8 or frame.ndim != 3 or frame.shape[2] != 3 or frame.strides[2] != 1 \
-                or frame.strides[1] != 3:
+        if not _packed(frame):
             raise ValueError("frame must be an HxWx3 uint8 array with packed pixels")
         r = (C.c_int * 4)(*[int(v) for v in rect])
         weights, radius = self._slic_weights(sigma, kernel)
@@ -475,13 +479,8 @@ class Handle:
                           n_segments=250, compactness=10.0, sigma=1.0, max_iter=10, start_label=0):
         """SLIC of many crops of a device-resident clip in ONE native call (pcm_slic_device_batch), laid out like
         quickshift_device_batch.  Returns the segment counts (int32 array)."""
-        fi = np.ascontiguousarray(frame_index, np.int32)
-        rc = np.ascontiguousarray(rects, np.int32).reshape(-1, 4)
-        off = np.ascontiguousarray(label_offsets, np.int64)
-        if not (len(fi) == len(rc) == len(off)):
-            raise ValueError("frame_index, rects and label_offsets must have one entry per crop")
+        fi, rc, off, counts = _batch_args(frame_index, rects, label_offsets)
         weights, radius = _gaussian_weights(sigma)
-        counts = np.zeros(len(fi), np.int32)
         self._check(self.lib.pcm_slic_device_batch(self._h, len(fi), C.c_void_p(d_frames), int(frame_bytes), _ptr(fi), int(frame_h),
                                                    int(frame_w), int(stride), _ptr(rc), int(n_segments), float(compactness),
                                                    float(sigma), _ptr(weights), radius, int(max_iter), int(start_label),

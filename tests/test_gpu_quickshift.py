@@ -92,7 +92,7 @@ def test_update_from_resident_quickshift_labels():
     h.close()
 
 
-def test_masker_uses_native_quickshift():
+def test_masker_native_seg_quickshift():
     """config over_segmentation: quickshift -> the plugin API segments on the GPU and produces
     the same mask as the same masker fed the oracle's label map through segment_fn."""
     from maskers import getMaskerByName
@@ -112,7 +112,7 @@ def test_masker_uses_native_quickshift():
         return m
     a = make()
     b = make(segment_fn=lambda crop: qso.quickshift(crop, ratio=0.5, kernel_size=3, max_dist=6, random_seed=42))
-    assert a.native_quickshift and not b.native_quickshift
+    assert a.native_seg == "quickshift" and b.native_seg is None
     for i in range(3):
         ma, mb = np.zeros_like(frames[i]), np.zeros_like(frames[i])
         box = (340 - 4 * i, 20, 90, 180)
@@ -122,9 +122,9 @@ def test_masker_uses_native_quickshift():
     a.close(); b.close()
 
 
-def test_masker_uses_native_slic():
-    """config over_segmentation: SLIC -> the plugin runs pcm_slic (host code of the library) and produces the same mask as
-    the same masker fed the oracle's label map through segment_fn (oracle/slic_oracle.py; parity unpinned against
+def test_masker_native_seg_slic():
+    """config over_segmentation: SLIC -> the plugin segments on the GPU (pcm_slic_gpu) and produces the same mask as the
+    same masker fed the oracle's label map through segment_fn (oracle/slic_oracle.py; parity unpinned against
     scikit-image itself)."""
     import slic_oracle as so
     from maskers import getMaskerByName
@@ -144,7 +144,7 @@ def test_masker_uses_native_slic():
         return m
     a = make()
     b = make(segment_fn=lambda crop: so.slic(crop, n_segments=250, compactness=10, sigma=1, start_label=0))
-    assert a.native_slic and not b.native_slic
+    assert a.native_seg == "SLIC" and b.native_seg is None
     for i in range(3):
         ma, mb = np.zeros_like(frames[i]), np.zeros_like(frames[i])
         box = (340 - 4 * i, 20, 90, 180)
@@ -152,6 +152,22 @@ def test_masker_uses_native_slic():
         assert b.update(bbox=box, frame=frames[i], mask=mb, color=None) is None
         assert ma[..., 2].any() and np.array_equal(ma, mb)
     a.close(); b.close()
+
+
+def test_quickshift_device_refuses_short_stride():
+    """pcm_quickshift_device refuses a row stride below 3 * W, as pcm_quickshift and the GPU SLIC entry points do."""
+    import ctypes as C
+    import torch
+    from pcm import capi
+    H, W = 24, 32
+    d_frame = torch.zeros(H * W * 3, dtype=torch.uint8, device="cuda")
+    torch.cuda.synchronize()
+    h = capi.Handle(0)
+    n = C.c_int(0)
+    rc = h.lib.pcm_quickshift_device(h._h, C.c_void_p(d_frame.data_ptr()), H, W, 3 * W - 3, (C.c_int * 4)(0, 0, W, H), 0.5, 3.0,
+                                     6.0, None, None, C.byref(n))
+    assert rc == -1 and b"pcm_quickshift_device" in h.lib.pcm_last_error()
+    h.close()
 
 
 def test_quickshift_device_batch_equals_single_crops():

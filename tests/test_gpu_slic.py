@@ -270,9 +270,11 @@ def test_slic_device_batch_equals_host(handle):
 
 
 @pytest.mark.parametrize("prior", [False, True])
-def test_masker_slic_provider_gpu_equals_host(prior):
-    """config slic_provider: gpu (default) and host give the same masks over a SegTrack2 sequence, with the prior off and
-    on (a deterministic prior of the label map: what matters is that both paths hand it the same map)."""
+def test_masker_gpu_slic_equals_host_slic(prior):
+    """The plugin's SLIC on the GPU gives the masks of the same masker fed the host code's labels (capi.slic) through
+    segment_fn, over a SegTrack2 sequence, with the prior off and on (a deterministic prior of the label map: what matters
+    is that both paths hand it the same map)."""
+    from pcm import capi
     from maskers import getMaskerByName
     from test_gpu_parity import _random_forest_arrays
     rng = np.random.default_rng(10)
@@ -284,19 +286,21 @@ def test_masker_slic_provider_gpu_equals_host(prior):
         return (s / np.maximum(cnt, 1) / 255.0).astype(np.float32)
     trees = _random_forest_arrays(rng, 12, 5, 3 * 49)
 
-    def make(provider):
+    def host_slic(crop):
+        return capi.slic(crop, (0, 0, crop.shape[1], crop.shape[0]), n_segments=250, compactness=10.0, sigma=1.0, start_label=0)[0]
+
+    def make(**kw):
         cfg = dict(multi_selection=False, params=dict(n_estimators=20, max_depth=5, n_components=1, novelty_detection=False,
                                                       over_segmentation="SLIC", features="6 lab", dilation_kernel=7,
                                                       prior_weight=0.1 if prior else 0.0))
-        if provider:
-            cfg["slic_provider"] = provider
-        m = getMaskerByName("PC", debug=False, frame=frames[0], config=cfg, poly_roi=None, update_mask=False, prior_fn=prior_fn)
+        m = getMaskerByName("PC", debug=False, frame=frames[0], config=cfg, poly_roi=None, update_mask=False, prior_fn=prior_fn,
+                            **kw)
         m.native.add_model_arrays(0, trees)
         m.models.append({"n_frame": 0, "model": None})
         m.novelty_det.append({"n_frame": 0, "model": None, "threshold": 0.0})
         return m
-    a, b = make(None), make("host")
-    assert a.native_slic and b.native_slic and a.slic_provider == "gpu" and b.slic_provider == "host"
+    a, b = make(), make(segment_fn=host_slic)
+    assert a.native_seg == "SLIC" and b.native_seg is None
     any_mask = False
     for i in range(8):
         ma, mb = np.zeros_like(frames[i]), np.zeros_like(frames[i])
@@ -307,8 +311,6 @@ def test_masker_slic_provider_gpu_equals_host(prior):
         assert np.array_equal(ma, mb), i
     assert any_mask
     a.close(); b.close()
-    with pytest.raises(ValueError):
-        make("cpu")
 
 
 def test_clip_resident_slic_sequence_equals_the_per_frame_path():

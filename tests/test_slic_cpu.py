@@ -66,3 +66,31 @@ def test_slic_synthetic(case):
         frame, rect = rng.integers(0, 64, (60, 60, 3), dtype=np.uint8), (0, 0, 60, 60)
         kw = dict(n_segments=75, compactness=10.0, sigma=1.0, start_label=0)   # optical_flow_masker.py:60's call
     _check(frame, rect, **kw)
+
+
+def test_slic_refuses_bad_arguments():
+    """pcm_slic checks its arguments before it runs: PCM_E_INVALID (-1), or PCM_E_LIMIT (-4) above 2^28 pixels, with a
+    message that names it."""
+    import ctypes as C
+    from pcm import capi
+    lib = capi.load_library()
+    frame = np.zeros((16, 16, 3), np.uint8)
+    out = np.empty(16 * 16, np.int32)
+    weights = np.full(3, 1.0 / 3)
+    n = C.c_int(0)
+
+    def call(rect=(0, 0, 16, 16), H=16, W=16, n_segments=10, compactness=10.0, max_iter=10, start_label=0, kernel=None,
+             radius=0):
+        rc = lib.pcm_slic(frame.ctypes.data_as(C.c_void_p), H, W, W * 3, (C.c_int * 4)(*rect), n_segments, compactness, 1.0,
+                          kernel, radius, max_iter, start_label, out.ctypes.data_as(C.c_void_p), C.byref(n))
+        assert rc == 0 or b"pcm_slic" in lib.pcm_last_error(), lib.pcm_last_error()
+        return rc
+    assert call() == 0 and n.value >= 1
+    assert call(n_segments=0) == -1
+    assert call(compactness=0.0) == -1 and call(compactness=float("nan")) == -1
+    assert call(max_iter=-1) == -1
+    assert call(start_label=-1) == -1
+    assert call(rect=(0, 0, 0, 16)) == -1 and call(rect=(0, 0, 17, 16)) == -1
+    assert call(kernel=weights.ctypes.data_as(C.c_void_p), radius=-1) == -1
+    big = 1 << 14
+    assert call(rect=(0, 0, big + 1, big), H=big, W=big + 1) == -4           # more than 2^28 pixels
