@@ -141,7 +141,7 @@ int pcm_update(pcm_handle* h, const uint8_t* frame, int frame_h, int frame_w, in
                const pcm_update_params* params,
                uint8_t* mask, int64_t mask_row_stride, int64_t mask_pixel_stride);
 
-/* labels == NULL: continue from the preceding pcm_quickshift or pcm_slic_gpu on this handle -- the label map
+/* labels == NULL: continue from the preceding pcm_quickshift, pcm_slic_gpu or pcm_felzenszwalb_gpu on this handle -- the label map
  * AND the crop pixels are the ones that call left on the device (`frame` and `rect` must be
  * the same as in that call; the frame is not read again).  n_labels is ignored. */
 
@@ -150,7 +150,7 @@ int pcm_update(pcm_handle* h, const uint8_t* frame, int frame_h, int frame_w, in
  * whole map (default: on). */
 int pcm_set_label_cache(pcm_handle* h, int on);
 
-/* labels == NULL with no pcm_quickshift / pcm_slic_gpu pending: the label map the previous pcm_update left on the device is used
+/* labels == NULL with no pcm_quickshift / pcm_slic_gpu / pcm_felzenszwalb_gpu pending: the label map the previous pcm_update left on the device is used
  * again (same crop size required; n_labels is ignored).  The caller vouches that the map has not changed -- the
  * plugin does this when its over-segmentation provider hands back the very same read-only array. */
 
@@ -218,9 +218,9 @@ int pcm_quickshift_device_batch(pcm_handle* h, int n, const uint8_t* d_frames, i
                                 const int64_t* label_offsets, int32_t* n_labels_out);
 
 /* skimage.segmentation.felzenszwalb(crop, scale, sigma, min_size) of scikit-image 0.17.2 (:72-73) on
- * the crop `rect` of a HOST frame.  HOST code (no handle, no device): the edge-ordered merge is
- * inherently sequential, and it is not part of the per-frame hot path.  Edges of equal cost are
- * processed in a fixed order (right, down, down-right, up-right; raster order within each).
+ * the crop `rect` of a HOST frame.  HOST code (no handle, no device): the reference the GPU variant
+ * pcm_felzenszwalb_gpu is tested against.  Edges of equal cost are processed in a fixed order
+ * (right, down, down-right, up-right; raster order within each).
  *   kernel      2 * kernel_radius + 1 Gaussian weights (scipy's _gaussian_kernel1d), or NULL to
  *               compute them from sigma
  *   labels_out  h*w int32, labels numbered like np.unique(root, return_inverse=True) */
@@ -280,6 +280,40 @@ int pcm_slic_debug_last(pcm_handle* h, double* smoothed, double* image, int32_t*
  * segment_image_index.h:85-91) in tests/test_felzenszwalb_ref.py.  labels_out: n_vertices int32. */
 int pcm_felzenszwalb_graph(int n_vertices, int n_edges, const int32_t* a, const int32_t* b, const double* cost,
                            double scale, int min_size, int32_t* labels_out, int* n_labels_out);
+
+/* pcm_felzenszwalb on the GPU: the same labels and count as pcm_felzenszwalb for the same arguments (DESIGN.md §9).  The
+ * cost-ordered merge runs in rounds that decide, in parallel, only edges whose outcome is already certain, so the partition
+ * is the host's exactly.  The crop of a HOST frame is staged like pcm_quickshift's, and the label map stays on the device:
+ * pcm_update with labels == NULL (same frame and rect) continues from it.  Synchronous.
+ *   kernel      2 * kernel_radius + 1 Gaussian weights on the host, or NULL to compute them from sigma as pcm_felzenszwalb does
+ *   labels_out  h*w int32 on the host, or NULL when only the device-resident map is needed
+ * Limits: crop of at most 2^28 pixels; kernel_radius >= 0 with a kernel; frame_stride >= 3 * frame_w. */
+int pcm_felzenszwalb_gpu(pcm_handle* h, const uint8_t* frame, int frame_h, int frame_w, int64_t frame_stride, const int rect[4],
+                         double scale, double sigma, int min_size, const double* kernel, int kernel_radius,
+                         int32_t* labels_out, int* n_labels_out);
+
+/* Device variant: d_frame and d_labels_out (h*w int32, may be NULL) are device pointers, `kernel` is on the host; waits
+ * for the stream to return the segment count. */
+int pcm_felzenszwalb_device(pcm_handle* h, const uint8_t* d_frame, int frame_h, int frame_w, int64_t frame_stride,
+                            const int rect[4], double scale, double sigma, int min_size, const double* kernel, int kernel_radius,
+                            int32_t* d_labels_out, int* n_labels_out);
+
+/* The Felzenszwalb maps of n crops of a device-resident clip in one call, laid out like pcm_quickshift_device_batch's:
+ * exactly n calls of pcm_felzenszwalb_device without returning to the caller in between. */
+int pcm_felzenszwalb_device_batch(pcm_handle* h, int n, const uint8_t* d_frames, int64_t frame_bytes, const int32_t* frame_index,
+                                  int frame_h, int frame_w, int64_t frame_stride, const int32_t* rects, double scale, double sigma,
+                                  int min_size, const double* kernel, int kernel_radius, int32_t* d_labels_out,
+                                  const int64_t* label_offsets, int32_t* n_labels_out);
+
+/* Parity tap: the device twin of pcm_felzenszwalb_graph (same arguments, same validation; a, b, cost and labels_out on the
+ * host): the sort, the two passes in rounds and the labelling of pcm_felzenszwalb_gpu on a caller's edge list. */
+int pcm_felzenszwalb_graph_gpu(pcm_handle* h, int n_vertices, int n_edges, const int32_t* a, const int32_t* b,
+                               const double* cost, double scale, int min_size, int32_t* labels_out, int* n_labels_out);
+
+/* Parity tap: for the last pcm_felzenszwalb_gpu / _device / _graph_gpu call on the handle, smoothed (h*w*3 float64 of that
+ * crop: /255 and the Gaussian; NULL skips it, and it must be NULL after the graph tap) and rounds[2] (int32: the rounds
+ * of the merge pass and of the min-size pass; NULL skips it).  PCM_E_STATE before any such call. */
+int pcm_felzenszwalb_debug_last(pcm_handle* h, double* smoothed, int32_t* rounds);
 
 /* ---- a whole sequence of frames in one call (main.py:280-343 for one target) ---- */
 

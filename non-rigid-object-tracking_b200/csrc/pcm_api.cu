@@ -10,6 +10,7 @@
 #include "pcm_forest_fit.cuh"
 #include "pcm_prior.cuh"
 #include "pcm_slic.cuh"
+#include "pcm_felzenszwalb.cuh"
 #include "pcm_host.h"
 
 #include <cudaTypedefs.h>
@@ -293,8 +294,8 @@ struct pcm_handle {
     std::vector<int> label_chunk_max;
     bool label_cache_on = true;   // pcm_set_label_cache
 
-    // over-segmentation on the GPU (quickshift, SLIC): the label map of the last call, and the handoff to pcm_update with
-    // labels == NULL, armed by pcm_quickshift / pcm_slic_gpu: the crop `rect` of the host frame `frame` is in `frame` (the
+    // over-segmentation on the GPU (quickshift, SLIC, Felzenszwalb): the label map of the last call, and the handoff to
+    // pcm_update with labels == NULL, armed by pcm_quickshift / pcm_slic_gpu / pcm_felzenszwalb_gpu: the crop `rect` of the host frame `frame` is in `frame` (the
     // device buffer above) and its map of n_labels segments in seg_labels
     DevBuf seg_labels;
     struct {
@@ -316,6 +317,13 @@ struct pcm_handle {
     DevBuf sl_parent, sl_root, sl_csize, sl_piece, sl_psize, sl_off, sl_queue, sl_seen, sl_adj, sl_nxt, sl_val, sl_labels;
     PinBuf h_slic;                // Gaussian weights + seed centres
     int sl_w = 0, sl_h = 0;       // crop of the stage results; 0: none
+    // Felzenszwalb (pcm_felzenszwalb_gpu / _device* / _graph_gpu): edges, sort, the state of the rounds, labels.  fz_smooth
+    // and fz_ctr (round counts) keep the stage results of the last call (pcm_felzenszwalb_debug_last).
+    DevBuf fz_kernel, fz_smooth, fz_tmp, fz_ea, fz_eb, fz_key, fz_key_sorted, fz_idx, fz_idx_sorted, fz_list0, fz_list1, fz_parent,
+           fz_size, fz_limit, fz_m, fz_root, fz_flag, fz_rank, fz_sums, fz_ctr, fz_count, fz_cub;
+    PinBuf h_fz;                  // Gaussian weights
+    int fz_w = 0, fz_h = 0;       // crop of fz_smooth; 0: the last call was the graph tap
+    bool fz_valid = false;        // a call has left round counts
     // forest training (pcm_fit_forest): feature-major rows resident between calls, scratch, outputs
     DevBuf fit_x, fit_xt, fit_y, fit_counts, fit_rand, fit_samples, fit_tmp, fit_out;
     DevBuf prior_scratch;         // pcm_prior_device: per-keypoint match records
@@ -1316,13 +1324,13 @@ static int upload_priors(pcm_handle* h, const float* priors, int n, const float*
 }
 
 // pcm_update(labels == NULL): the crop pixels and the label map are the ones the preceding
-// pcm_quickshift or pcm_slic_gpu on this handle left on the device (h->handoff)
+// pcm_quickshift, pcm_slic_gpu or pcm_felzenszwalb_gpu on this handle left on the device (h->handoff)
 static int update_from_handoff(pcm_handle* h, const uint8_t* frame, int H, int W, int64_t stride, const int rect[4],
                                const float* priors, const pcm_update_params* params, uint8_t* mask,
                                int64_t mask_row_stride, int64_t mask_pixel_stride) {
     if (!rect) return fail(PCM_E_INVALID, "pcm_update: NULL rect");
     if (!h->handoff.valid || h->handoff.frame != frame || memcmp(h->handoff.rect, rect, sizeof h->handoff.rect) != 0)
-        return fail(PCM_E_STATE, "pcm_update: labels == NULL needs a preceding pcm_quickshift or pcm_slic_gpu of the same frame and rect");
+        return fail(PCM_E_STATE, "pcm_update: labels == NULL needs a preceding pcm_quickshift, pcm_slic_gpu or pcm_felzenszwalb_gpu of the same frame and rect");
     int rc = validate_update(h, H, W, rect, h->handoff.n_labels, params);
     if (rc) return rc;
     CUDA_TRY(cudaSetDevice(h->device));
@@ -1367,7 +1375,7 @@ extern "C" int pcm_update(pcm_handle* h, const uint8_t* frame, int H, int W, int
     const bool reuse_labels = !labels;
     if (reuse_labels) {
         if (!rect || h->resident_labels <= 0 || rect[2] != h->resident_cw || rect[3] != h->resident_ch)
-            return fail(PCM_E_STATE, "pcm_update: labels == NULL needs a preceding pcm_quickshift or pcm_slic_gpu of the same frame and rect, or a "
+            return fail(PCM_E_STATE, "pcm_update: labels == NULL needs a preceding pcm_quickshift, pcm_slic_gpu or pcm_felzenszwalb_gpu of the same frame and rect, or a "
                                      "preceding pcm_update with a label map for a crop of the same size");
         n_labels = h->resident_labels;
     }
@@ -1608,7 +1616,7 @@ extern "C" int pcm_host_unregister(void* p) {
 }
 
 // ---------------------------------------------------------------------------------
-// over-segmentation on the GPU: the front end quickshift and SLIC share.  Each algorithm's enqueue_* queues it on a crop
+// over-segmentation on the GPU: the front end quickshift, SLIC and Felzenszwalb share.  Each algorithm's enqueue_* queues it on a crop
 // of a device frame, writes the label map into h->seg_labels and leaves its count in a device word.
 // ---------------------------------------------------------------------------------
 // The checks and set-up every entry point below starts with.  The handoff ends here: the call replaces the label map,
@@ -1937,6 +1945,19 @@ static bool slic_seed_grid(int h, int w, int n_points, int& start_y, int& step_y
 
 static int bit_length(unsigned v) { int b = 0; while (v) { ++b; v >>= 1; } return b; }
 
+// Gaussian weights of the GPU SLIC and Felzenszwalb: the caller's, or scipy's _gaussian_kernel1d computed as pcm_slic.cpp and
+// pcm_felzenszwalb.cpp do (truncate = 4), held in `kw`.  No weights and radius 0 when sigma is not positive.
+static const double* gaussian_weights(double sigma, const double* kernel, int& radius, std::vector<double>& kw) {
+    if (!(sigma > 0)) { radius = 0; return nullptr; }
+    if (kernel) return kernel;
+    radius = (int)(4.0 * sigma + 0.5);
+    kw.resize(2 * radius + 1);
+    double sum = 0;
+    for (int x = -radius; x <= radius; ++x) { kw[x + radius] = std::exp(-0.5 / (sigma * sigma) * (double)(x * x)); sum += kw[x + radius]; }
+    for (double& v : kw) v /= sum;
+    return kw.data();
+}
+
 // CUB scratch for a stable sort of n (int key, int value) pairs and an exclusive sum of n ints
 static int reserve_slic_cub(pcm_handle* h, int n, size_t* bytes) {
     size_t a = 0, b = 0;
@@ -2016,17 +2037,8 @@ static int enqueue_slic(pcm_handle* h, const uint8_t* d_frame, int64_t stride, i
     cudaStream_t st = h->stream;
     h->chain_tail = false;
     h->sl_w = h->sl_h = 0;
-    // Gaussian weights: the caller's, or scipy's _gaussian_kernel1d computed as pcm_slic.cpp does (truncate = 4)
     std::vector<double> kw;
-    if (sigma > 0 && !kernel) {
-        radius = (int)(4.0 * sigma + 0.5);
-        kw.resize(2 * radius + 1);
-        double sum = 0;
-        for (int x = -radius; x <= radius; ++x) { kw[x + radius] = std::exp(-0.5 / (sigma * sigma) * (double)(x * x)); sum += kw[x + radius]; }
-        for (double& v : kw) v /= sum;
-        kernel = kw.data();
-    }
-    if (!(sigma > 0)) radius = 0;
+    kernel = gaussian_weights(sigma, kernel, radius, kw);
     // seeds on the regular grid (every pixel when there are no more pixels than segments)
     int sy = 0, ty = 1, sx = 0, tx = 1;
     const bool grid = slic_seed_grid(hh, w, n_segments, sy, ty, sx, tx);
@@ -2183,6 +2195,246 @@ extern "C" int pcm_slic_debug_last(pcm_handle* h, double* smoothed, double* imag
     if (smoothed) CUDA_TRY(cudaMemcpyAsync(smoothed, h->sl_smooth.p, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (image) CUDA_TRY(cudaMemcpyAsync(image, h->sl_img.p, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (nearest) CUDA_TRY(cudaMemcpyAsync(nearest, h->sl_nearest.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    return PCM_OK;
+}
+
+// ---------------------------------------------------------------------------------
+// API: Felzenszwalb over-segmentation on the GPU (pcm_felzenszwalb.cuh).  Same labels as pcm_felzenszwalb; see DESIGN.md §9.
+// ---------------------------------------------------------------------------------
+// the arguments of pcm_felzenszwalb's GPU variants besides the frame and a crop rect already checked with check_rect
+static int check_felzenszwalb_args(const char* who, const int rect[4], const double* kernel, int kernel_radius) {
+    if ((long long)rect[2] * rect[3] > (1LL << 28)) return fail(PCM_E_LIMIT, "%s: crop too large (more than 2^28 pixels)", who);
+    if (kernel && kernel_radius < 0) return fail(PCM_E_INVALID, "%s: kernel_radius %d", who, kernel_radius);
+    return PCM_OK;
+}
+
+// cooperative launch of the rounds of one pass over the n_edges edges of fz_list0 (fz_ctr[0] = n_edges, [1..3] = 0);
+// the number of rounds goes to *rounds
+template <bool MIN_SIZE>
+static int launch_fz_rounds(pcm_handle* h, int n_vertices, int n_edges, double sc, int min_size, int* rounds) {
+    static int occ = 0;                               // resident CTAs per SM, queried once
+    if (!occ) CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fz_rounds_kernel<MIN_SIZE>, FZ_THREADS, 0));
+    if (occ < 1) return fail(PCM_E_CUDA, "felzenszwalb: the rounds kernel cannot be resident");
+    CUDA_TRY(cudaMemsetAsync(h->fz_m.p, 0xff, (size_t)n_vertices * sizeof(unsigned long long), h->stream));
+    FzRounds s{};
+    s.parent = h->fz_parent.as<int>();
+    s.size = h->fz_size.as<int>();
+    s.limit = h->fz_limit.as<double>();
+    s.m = h->fz_m.as<unsigned long long>();
+    s.key = h->fz_key_sorted.as<unsigned long long>();
+    s.list[0] = h->fz_list0.as<FzEdge>();
+    s.list[1] = h->fz_list1.as<FzEdge>();
+    s.ctr = h->fz_ctr.as<int>();
+    s.rounds = rounds;
+    s.sc = sc;
+    s.min_size = min_size;
+    const int blocks = (int)std::max<long long>(1, std::min<long long>((long long)occ * h->sm_count, ((long long)n_edges + FZ_THREADS - 1) / FZ_THREADS));
+    void* args[] = {&s};
+    CUDA_TRY(cudaLaunchCooperativeKernel((const void*)fz_rounds_kernel<MIN_SIZE>, blocks, FZ_THREADS, args, 0, h->stream));
+    CHECK_LAUNCH(h, MIN_SIZE ? "fz_rounds_kernel<true>" : "fz_rounds_kernel<false>");
+    return PCM_OK;
+}
+
+// F3-F6 of pcm_felzenszwalb.cuh on the n_edges edges in fz_ea / fz_eb / fz_key / fz_idx (edge order): labels into d_labels,
+// their count into fz_count, the round counts of the two passes into fz_ctr[4..5].  Asynchronous.
+static int enqueue_fz_merge(pcm_handle* h, int n, int n_edges, double sc, int min_size, int32_t* d_labels) {
+    cudaStream_t st = h->stream;
+    const size_t ib = (size_t)n * sizeof(int);
+    for (DevBuf* b : {&h->fz_parent, &h->fz_size, &h->fz_root, &h->fz_flag, &h->fz_rank}) CUDA_TRY(b->reserve(ib));
+    CUDA_TRY(h->fz_limit.reserve((size_t)n * sizeof(double)));
+    CUDA_TRY(h->fz_m.reserve((size_t)n * sizeof(unsigned long long)));
+    const int n_scan = (int)((n + QS_SCAN_ELEMS - 1) / QS_SCAN_ELEMS);
+    CUDA_TRY(h->fz_sums.reserve((size_t)n_scan * sizeof(int)));
+    const size_t ne = (size_t)std::max(n_edges, 1);
+    CUDA_TRY(h->fz_key_sorted.reserve(ne * sizeof(unsigned long long)));
+    CUDA_TRY(h->fz_idx_sorted.reserve(ne * sizeof(int)));
+    CUDA_TRY(h->fz_list0.reserve(ne * sizeof(FzEdge)));
+    CUDA_TRY(h->fz_list1.reserve(ne * sizeof(FzEdge)));
+    CUDA_TRY(h->fz_ctr.reserve(8 * sizeof(int)));
+    CUDA_TRY(h->fz_count.reserve(sizeof(int)));
+    size_t cub_bytes = 0;
+    CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, (const unsigned long long*)nullptr, (unsigned long long*)nullptr,
+                                             (const int*)nullptr, (int*)nullptr, n_edges));
+    CUDA_TRY(h->fz_cub.reserve(std::max<size_t>(cub_bytes, 1)));
+    int* ctr = h->fz_ctr.as<int>();
+    const int blocks = (int)std::min<long long>(((long long)std::max(n, n_edges) + 255) / 256, (long long)h->sm_count * 16);
+    int* parent = h->fz_parent.as<int>();
+    int* root = h->fz_root.as<int>();
+    int* flag = h->fz_flag.as<int>();
+    FzEdge* list = h->fz_list0.as<FzEdge>();
+
+    // F3: stable order of (cost bits, edge index)
+    if (n_edges > 0)
+        CUDA_TRY(cub::DeviceRadixSort::SortPairs(h->fz_cub.p, cub_bytes, h->fz_key.as<unsigned long long>(),
+                                                 h->fz_key_sorted.as<unsigned long long>(), h->fz_idx.as<int>(),
+                                                 h->fz_idx_sorted.as<int>(), n_edges, 0, 64, st));
+    // F4: every pixel its own component (limit = 0.0 + sc / 1, as the host sets it), then the merge pass
+    fz_init_kernel<<<blocks, 256, 0, st>>>(parent, h->fz_size.as<int>(), h->fz_limit.as<double>(), 0.0 + sc / 1, n);
+    CHECK_LAUNCH(h, "fz_init_kernel");
+    fz_gather_kernel<<<blocks, 256, 0, st>>>(h->fz_idx_sorted.as<int>(), h->fz_ea.as<int>(), h->fz_eb.as<int>(), nullptr, n_edges,
+                                             list, ctr);
+    CHECK_LAUNCH(h, "fz_gather_kernel");
+    if (int rc = launch_fz_rounds<false>(h, n, n_edges, sc, min_size, ctr + 4)) return rc;
+    // F5: every pixel's root, then the min-size pass over all edges again, in the same order
+    CUDA_TRY(cudaMemsetAsync(flag, 0, ib, st));
+    qs_root_kernel<<<blocks, 256, 0, st>>>(parent, root, flag, n);
+    CHECK_LAUNCH(h, "qs_root_kernel");
+    fz_gather_kernel<<<blocks, 256, 0, st>>>(h->fz_idx_sorted.as<int>(), h->fz_ea.as<int>(), h->fz_eb.as<int>(), root, n_edges,
+                                             list, ctr);
+    CHECK_LAUNCH(h, "fz_gather_kernel");
+    if (int rc = launch_fz_rounds<true>(h, n, n_edges, sc, min_size, ctr + 5)) return rc;
+    // F6: label = rank of the root among all roots, count = number of roots
+    CUDA_TRY(cudaMemsetAsync(flag, 0, ib, st));
+    qs_root_kernel<<<blocks, 256, 0, st>>>(parent, root, flag, n);
+    CHECK_LAUNCH(h, "qs_root_kernel");
+    qs_scan_reduce_kernel<<<n_scan, 256, 0, st>>>(flag, n, h->fz_sums.as<int>());
+    CHECK_LAUNCH(h, "qs_scan_reduce_kernel");
+    qs_scan_sums_kernel<<<1, 256, 0, st>>>(h->fz_sums.as<int>(), n_scan, h->fz_count.as<int>());
+    CHECK_LAUNCH(h, "qs_scan_sums_kernel");
+    qs_scan_apply_kernel<<<n_scan, 256, 0, st>>>(flag, n, h->fz_sums.as<int>(), h->fz_rank.as<int>());
+    CHECK_LAUNCH(h, "qs_scan_apply_kernel");
+    qs_label_kernel<<<blocks, 256, 0, st>>>(root, h->fz_rank.as<int>(), d_labels, n);
+    CHECK_LAUNCH(h, "qs_label_kernel");
+    h->fz_valid = true;
+    return PCM_OK;
+}
+
+// The whole Felzenszwalb of the crop (cx, cy, w, hh) of a device frame into seg_labels, its count into fz_count.
+// Asynchronous apart from the host-side staging of the weights (the caller has synchronised the stream).
+static int enqueue_felzenszwalb(pcm_handle* h, const uint8_t* d_frame, int64_t stride, int cx, int cy, int w, int hh, double scale,
+                                double sigma, int min_size, const double* kernel, int radius) {
+    const int n = w * hh;
+    const long long n_edges = (long long)hh * (w - 1) + (long long)(hh - 1) * w + 2LL * (hh - 1) * (w - 1);
+    cudaStream_t st = h->stream;
+    h->chain_tail = false;
+    h->fz_w = h->fz_h = 0;
+    h->fz_valid = false;
+    std::vector<double> kw;
+    kernel = gaussian_weights(sigma, kernel, radius, kw);
+    const size_t nk = kernel ? (size_t)(2 * radius + 1) : 0;
+    const size_t db = (size_t)n * 3 * sizeof(double), ne = (size_t)std::max(n_edges, 1LL);
+    CUDA_TRY(h->fz_kernel.reserve(std::max<size_t>(nk, 1) * sizeof(double)));
+    CUDA_TRY(h->fz_smooth.reserve(db));
+    if (nk) CUDA_TRY(h->fz_tmp.reserve(db));
+    CUDA_TRY(h->fz_ea.reserve(ne * sizeof(int)));
+    CUDA_TRY(h->fz_eb.reserve(ne * sizeof(int)));
+    CUDA_TRY(h->fz_idx.reserve(ne * sizeof(int)));
+    CUDA_TRY(h->fz_key.reserve(ne * sizeof(unsigned long long)));
+    CUDA_TRY(h->seg_labels.reserve((size_t)n * sizeof(int32_t)));
+    if (nk) {
+        CUDA_TRY(h->h_fz.reserve(nk * sizeof(double)));
+        memcpy(h->h_fz.p, kernel, nk * sizeof(double));
+        CUDA_TRY(cudaMemcpyAsync(h->fz_kernel.p, h->h_fz.p, nk * sizeof(double), cudaMemcpyHostToDevice, st));
+        h->bytes_h2d += (int64_t)(nk * sizeof(double));
+    }
+    const int blocks = (int)std::min<long long>(((long long)n + SLIC_THREADS - 1) / SLIC_THREADS, (long long)h->sm_count * 16);
+    const double* dk = h->fz_kernel.as<double>();
+    double* smooth = h->fz_smooth.as<double>();
+    // F1: byte / 255 and the Gaussian along rows, then columns (no Gaussian when sigma <= 0)
+    slic_load_kernel<<<blocks, SLIC_THREADS, 0, st>>>(d_frame, stride, cx, cy, w, hh, dk, radius, 0, smooth);
+    CHECK_LAUNCH(h, "slic_load_kernel");
+    if (nk) {
+        slic_smooth_kernel<<<blocks, SLIC_THREADS, 0, st>>>(smooth, h->fz_tmp.as<double>(), hh, w, 0, dk, radius);
+        CHECK_LAUNCH(h, "slic_smooth_kernel");
+        slic_smooth_kernel<<<blocks, SLIC_THREADS, 0, st>>>(h->fz_tmp.as<double>(), smooth, hh, w, 1, dk, radius);
+        CHECK_LAUNCH(h, "slic_smooth_kernel");
+    }
+    // F2: the edges in the host's order
+    if (n_edges > 0) {
+        const int eblocks = (int)std::min<long long>((n_edges + 255) / 256, (long long)h->sm_count * 16);
+        fz_cost_kernel<<<eblocks, 256, 0, st>>>(smooth, hh, w, h->fz_ea.as<int>(), h->fz_eb.as<int>(),
+                                                h->fz_key.as<unsigned long long>(), h->fz_idx.as<int>());
+        CHECK_LAUNCH(h, "fz_cost_kernel");
+    }
+    if (int rc = enqueue_fz_merge(h, n, (int)n_edges, scale / 255.0, min_size, h->seg_labels.as<int32_t>())) return rc;
+    h->fz_w = w; h->fz_h = hh;
+    return PCM_OK;
+}
+
+extern "C" int pcm_felzenszwalb_device(pcm_handle* h, const uint8_t* d_frame, int H, int W, int64_t stride, const int rect[4],
+                                       double scale, double sigma, int min_size, const double* kernel, int kernel_radius,
+                                       int32_t* d_labels_out, int* n_labels_out) {
+    return seg_device(h, "pcm_felzenszwalb_device", d_frame, H, W, stride, rect, &pcm_handle::fz_count, 0, d_labels_out, n_labels_out,
+                      [&] {
+                          if (int rc = check_felzenszwalb_args("pcm_felzenszwalb_device", rect, kernel, kernel_radius)) return rc;
+                          CUDA_TRY(cudaStreamSynchronize(h->stream));      // the pinned weight buffer is reused between calls
+                          return enqueue_felzenszwalb(h, d_frame, stride, rect[0], rect[1], rect[2], rect[3], scale, sigma, min_size,
+                                                      kernel, kernel_radius);
+                      });
+}
+
+extern "C" int pcm_felzenszwalb_device_batch(pcm_handle* h, int n, const uint8_t* d_frames, int64_t frame_bytes,
+                                             const int32_t* frame_index, int H, int W, int64_t stride, const int32_t* rects,
+                                             double scale, double sigma, int min_size, const double* kernel, int kernel_radius,
+                                             int32_t* d_labels_out, const int64_t* label_offsets, int32_t* n_labels_out) {
+    return seg_device_batch(h, "pcm_felzenszwalb_device_batch", n, d_frames, frame_bytes, frame_index, rects, d_labels_out,
+                            label_offsets, n_labels_out, [&](const uint8_t* d_frame, const int rect[4], int32_t* d_labels, int* count) {
+                                return pcm_felzenszwalb_device(h, d_frame, H, W, stride, rect, scale, sigma, min_size, kernel,
+                                                               kernel_radius, d_labels, count);
+                            });
+}
+
+extern "C" int pcm_felzenszwalb_gpu(pcm_handle* h, const uint8_t* frame, int H, int W, int64_t stride, const int rect[4],
+                                    double scale, double sigma, int min_size, const double* kernel, int kernel_radius,
+                                    int32_t* labels_out, int* n_labels_out) {
+    int rc = begin_seg(h, "pcm_felzenszwalb_gpu", frame, H, W, stride, rect);
+    if (rc) return rc;
+    if ((rc = check_felzenszwalb_args("pcm_felzenszwalb_gpu", rect, kernel, kernel_radius))) return rc;
+    if ((rc = stage_crop(h, "pcm_felzenszwalb_gpu", frame, stride, rect, 0, [](int) { return cudaSuccess; }))) return rc;
+    rc = enqueue_felzenszwalb(h, h->frame.as<uint8_t>(), (int64_t)rect[2] * 3, 0, 0, rect[2], rect[3], scale, sigma, min_size, kernel,
+                              kernel_radius);
+    if (rc) return rc;
+    return finish_host_seg(h, frame, rect, h->fz_count.as<int>(), 0, labels_out, n_labels_out);
+}
+
+extern "C" int pcm_felzenszwalb_graph_gpu(pcm_handle* h, int n_vertices, int n_edges, const int32_t* a, const int32_t* b,
+                                          const double* cost, double scale, int min_size, int32_t* labels_out, int* n_labels_out) {
+    if (!h || !a || !b || !cost || !labels_out) return fail(PCM_E_INVALID, "pcm_felzenszwalb_graph_gpu: NULL argument");
+    if (n_vertices <= 0 || n_vertices > (1 << 28) || n_edges < 0) return fail(PCM_E_INVALID, "pcm_felzenszwalb_graph_gpu: bad sizes");
+    for (int i = 0; i < n_edges; ++i)
+        if (a[i] < 0 || a[i] >= n_vertices || b[i] < 0 || b[i] >= n_vertices || !(cost[i] >= 0.0))
+            return fail(PCM_E_INVALID, "pcm_felzenszwalb_graph_gpu: vertex index out of range or negative / NaN cost");
+    CUDA_TRY(cudaSetDevice(h->device));
+    cudaStream_t st = h->stream;
+    h->chain_tail = false;
+    h->fz_w = h->fz_h = 0;
+    h->fz_valid = false;
+    const size_t ne = (size_t)std::max(n_edges, 1), ib = (size_t)n_vertices * sizeof(int32_t);
+    CUDA_TRY(h->fz_ea.reserve(ne * sizeof(int)));
+    CUDA_TRY(h->fz_eb.reserve(ne * sizeof(int)));
+    CUDA_TRY(h->fz_idx.reserve(ne * sizeof(int)));
+    CUDA_TRY(h->fz_key.reserve(ne * sizeof(unsigned long long)));
+    CUDA_TRY(h->seg_labels.reserve(ib));
+    h->handoff.valid = false;                          // seg_labels is about to be replaced
+    // the cost bits are the sort keys
+    CUDA_TRY(cudaMemcpyAsync(h->fz_ea.p, a, (size_t)n_edges * sizeof(int), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(h->fz_eb.p, b, (size_t)n_edges * sizeof(int), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(h->fz_key.p, cost, (size_t)n_edges * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (n_edges > 0) {
+        slic_ccl_init_kernel<<<(int)std::min<long long>((n_edges + 255) / 256, (long long)h->sm_count * 16), 256, 0, st>>>(
+            h->fz_idx.as<int>(), n_edges);
+        CHECK_LAUNCH(h, "slic_ccl_init_kernel");
+    }
+    int rc = enqueue_fz_merge(h, n_vertices, n_edges, scale, min_size, h->seg_labels.as<int32_t>());
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(labels_out, h->seg_labels.p, ib, cudaMemcpyDeviceToHost, st));
+    int count = 0;
+    if ((rc = read_seg_count(h, h->fz_count.as<int>(), 0, &count))) return rc;
+    if (n_labels_out) *n_labels_out = count;
+    return PCM_OK;
+}
+
+extern "C" int pcm_felzenszwalb_debug_last(pcm_handle* h, double* smoothed, int32_t* rounds) {
+    if (!h) return fail(PCM_E_INVALID, "pcm_felzenszwalb_debug_last: NULL handle");
+    if (!h->fz_valid) return fail(PCM_E_STATE, "pcm_felzenszwalb_debug_last: no GPU Felzenszwalb on this handle yet");
+    if (smoothed && !h->fz_w)
+        return fail(PCM_E_STATE, "pcm_felzenszwalb_debug_last: the last call was pcm_felzenszwalb_graph_gpu: no smoothed image");
+    CUDA_TRY(cudaSetDevice(h->device));
+    cudaStream_t st = h->stream;
+    if (smoothed)
+        CUDA_TRY(cudaMemcpyAsync(smoothed, h->fz_smooth.p, (size_t)h->fz_w * h->fz_h * 3 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (rounds) CUDA_TRY(cudaMemcpyAsync(rounds, h->fz_ctr.as<int>() + 4, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return PCM_OK;
 }

@@ -71,8 +71,7 @@ class PixelClassificationNonRigidMasker(Masker):
         self.native = capi.Handle(device)
         self.native.set_features(self.n_neighbors, self.spaces)
         # over-segmentation (:70-75), SURVEY §8 f-1, by the library unless segment_fn is given: native_seg is the
-        # algorithm it runs, or None.  quickshift and SLIC run on the GPU (pcm_quickshift, pcm_slic_gpu), felzenszwalb in
-        # the library's host code (pcm_felzenszwalb: inherently sequential)
+        # algorithm it runs, or None.  All three run on the GPU (pcm_quickshift, pcm_slic_gpu, pcm_felzenszwalb_gpu)
         method = params["over_segmentation"]
         self.native_seg = method if segment_fn is None and method in ("quickshift", "SLIC", "felzenszwalb") else None
         self.segment_fn = segment_fn or (None if self.native_seg else make_segment_provider(method))
@@ -206,8 +205,9 @@ class PixelClassificationNonRigidMasker(Masker):
             return self.prior_fn(self.prevFrame, self.prevForegroundMask, crop, segs, n)
         n_labels, priors = 0, None             # 0: the library takes max(label) + 1 while staging
         same_labels, self._seg_next = False, None
-        if self.native_seg in ("quickshift", "SLIC"):
-            # quickshift(crop, kernel_size=3, max_dist=6, ratio=0.5, random_seed=42) (:71) or
+        if self.native_seg is not None:
+            # quickshift(crop, kernel_size=3, max_dist=6, ratio=0.5, random_seed=42) (:71),
+            # felzenszwalb(crop, scale=100, sigma=0.5, min_size=50) (:73) or
             # slic(crop, n_segments=250, compactness=10, sigma=1, start_label=0) (:75) on the GPU; the label
             # map stays on the device and only travels to the host when the SIFT prior needs it
             if frame.strides[2] != 1 or frame.strides[1] != 3:
@@ -220,6 +220,10 @@ class PixelClassificationNonRigidMasker(Masker):
                 with stages.stage("gpu_quickshift_call"):
                     segments, n_labels = self.native.quickshift(frame, (x, y, w, h), ratio=0.5, kernel_size=3, max_dist=6,
                                                                 noise=noise, want_labels=want_prior)
+            elif self.native_seg == "felzenszwalb":
+                with stages.stage("gpu_felzenszwalb_call"):
+                    segments, n_labels = self.native.felzenszwalb(frame, (x, y, w, h), scale=100, sigma=0.5, min_size=50,
+                                                                  want_labels=want_prior)
             else:
                 with stages.stage("gpu_slic_call"):
                     segments, n_labels = self.native.slic(frame, (x, y, w, h), n_segments=250, compactness=10.0, sigma=1.0,
@@ -229,26 +233,13 @@ class PixelClassificationNonRigidMasker(Masker):
                     priors = prior(segments, n_labels)
             segments = None                    # update() continues from the device-resident map
         else:
-            if self.native_seg == "felzenszwalb":
-                # felzenszwalb(crop, scale=100, sigma=0.5, min_size=50) (:73).  In a sweep the label map
-                # of (clip, frame, crop) is the same for every hyper-parameter combination: shared
-                # through the model cache when the caller says the frames are the clip's (cache_tag)
-                def segment():
-                    return capi.felzenszwalb(frame, (x, y, w, h), scale=100, sigma=0.5, min_size=50)
-                cache = self.model_cache if self.cache_tag is not None else None
-                with stages.stage("felzenszwalb"):
-                    if cache is not None and hasattr(cache, "get_or_compute"):
-                        segments, n_labels = cache.get_or_compute((self.cache_tag, "felzenszwalb", self.index, (x, y, w, h)), segment)
-                    else:
-                        segments, n_labels = segment()
-            else:
-                raw = self.segment_fn(crop)
-                # a provider that hands back the very same READ-ONLY array vouches that the map has not changed: it is
-                # still on the device from the previous update and does not travel again (pcm_update, labels == NULL)
-                same_labels = (self.reuse_resident_labels and self._seg_prev is not None and raw is self._seg_prev[0] and self._seg_prev[1] == (h, w)
-                               and isinstance(raw, np.ndarray) and not raw.flags.writeable)
-                self._seg_next = (raw, (h, w))
-                segments = np.ascontiguousarray(raw, np.int32)
+            raw = self.segment_fn(crop)
+            # a provider that hands back the very same READ-ONLY array vouches that the map has not changed: it is
+            # still on the device from the previous update and does not travel again (pcm_update, labels == NULL)
+            same_labels = (self.reuse_resident_labels and self._seg_prev is not None and raw is self._seg_prev[0] and self._seg_prev[1] == (h, w)
+                           and isinstance(raw, np.ndarray) and not raw.flags.writeable)
+            self._seg_next = (raw, (h, w))
+            segments = np.ascontiguousarray(raw, np.int32)
             if want_prior:
                 n_labels = int(segments.max()) + 1
                 with stages.stage("sift_prior"):

@@ -67,6 +67,11 @@ _SIGNATURES = {
     "pcm_quickshift_device_batch": (I, [P, I, P, L, P, I, I, L, P, D, D, D, P, P, P, P]),
     "pcm_felzenszwalb": (I, [P, I, I, L, P, D, D, I, P, I, P, C.POINTER(I)]),
     "pcm_felzenszwalb_graph": (I, [I, I, P, P, P, D, I, P, C.POINTER(I)]),
+    "pcm_felzenszwalb_gpu": (I, [P, P, I, I, L, P, D, D, I, P, I, P, C.POINTER(I)]),
+    "pcm_felzenszwalb_device": (I, [P, P, I, I, L, P, D, D, I, P, I, P, C.POINTER(I)]),
+    "pcm_felzenszwalb_device_batch": (I, [P, I, P, L, P, I, I, L, P, D, D, I, P, I, P, P, P]),
+    "pcm_felzenszwalb_graph_gpu": (I, [P, I, I, P, P, P, D, I, P, C.POINTER(I)]),
+    "pcm_felzenszwalb_debug_last": (I, [P, P, P]),
     "pcm_slic": (I, [P, I, I, L, P, I, D, D, P, I, I, I, P, C.POINTER(I)]),
     "pcm_slic_gpu": (I, [P, P, I, I, L, P, I, D, D, P, I, I, I, P, C.POINTER(I)]),
     "pcm_slic_device": (I, [P, P, I, I, L, P, I, D, D, P, I, I, I, P, C.POINTER(I)]),
@@ -447,6 +452,61 @@ class Handle:
                                                          float(max_dist), C.c_void_p(d_noise) if d_noise else None,
                                                          C.c_void_p(d_labels_out), _ptr(off), _ptr(counts)))
         return counts
+
+    def felzenszwalb(self, frame, rect, scale=100, sigma=0.5, min_size=50, want_labels=True, kernel=None):
+        """Felzenszwalb over-segmentation of the crop `rect` on the GPU (pcm_felzenszwalb_gpu; defaults = the reference's
+        call, pixel_classification.py:73): the labels and count of the host `capi.felzenszwalb`.  Returns (labels int32 HxW
+        or None, n_labels); the map also stays on the device for `update(..., labels=None)`.  `kernel`: Gaussian weights,
+        or None to compute them from sigma as scipy.ndimage does."""
+        if not _packed(frame):
+            raise ValueError("frame must be an HxWx3 uint8 array with packed pixels")
+        r = (C.c_int * 4)(*[int(v) for v in rect])
+        weights, radius = self._slic_weights(sigma, kernel)
+        out = np.empty((rect[3], rect[2]), np.int32) if want_labels else None
+        n = C.c_int(0)
+        self._check(self.lib.pcm_felzenszwalb_gpu(self._h, _ptr(frame), frame.shape[0], frame.shape[1], frame.strides[0], r,
+                                                  float(scale), float(sigma), int(min_size), _ptr(weights), radius, _ptr(out),
+                                                  C.byref(n)))
+        self._felzenszwalb_shape = (int(rect[3]), int(rect[2]))
+        return out, n.value
+
+    def felzenszwalb_device_batch(self, d_frames, frame_bytes, frame_index, frame_h, frame_w, stride, rects, d_labels_out,
+                                  label_offsets, scale=100, sigma=0.5, min_size=50):
+        """Felzenszwalb of many crops of a device-resident clip in ONE native call (pcm_felzenszwalb_device_batch), laid out
+        like quickshift_device_batch.  Returns the segment counts (int32 array)."""
+        fi, rc, off, counts = _batch_args(frame_index, rects, label_offsets)
+        weights, radius = _gaussian_weights(sigma)
+        self._check(self.lib.pcm_felzenszwalb_device_batch(self._h, len(fi), C.c_void_p(d_frames), int(frame_bytes), _ptr(fi),
+                                                           int(frame_h), int(frame_w), int(stride), _ptr(rc), float(scale),
+                                                           float(sigma), int(min_size), _ptr(weights), radius,
+                                                           C.c_void_p(d_labels_out), _ptr(off), _ptr(counts)))
+        if len(fi):
+            self._felzenszwalb_shape = (int(rc[-1, 3]), int(rc[-1, 2]))
+        return counts
+
+    def felzenszwalb_graph(self, n_vertices, a, b, cost, scale, min_size):
+        """Parity tap: the device twin of `capi.felzenszwalb_graph` (pcm_felzenszwalb_graph_gpu).  Returns (labels
+        int32[n_vertices], n_labels)."""
+        a = np.ascontiguousarray(a, np.int32)
+        b = np.ascontiguousarray(b, np.int32)
+        cost = np.ascontiguousarray(cost, np.float64)
+        if not (a.shape == b.shape == cost.shape and a.ndim == 1):
+            raise ValueError("a, b and cost must be 1-D arrays of one length")
+        out = np.empty(int(n_vertices), np.int32)
+        n = C.c_int(0)
+        self._check(self.lib.pcm_felzenszwalb_graph_gpu(self._h, int(n_vertices), a.size, _ptr(a), _ptr(b), _ptr(cost), float(scale),
+                                                        int(min_size), _ptr(out), C.byref(n)))
+        self._felzenszwalb_shape = None
+        return out, n.value
+
+    def felzenszwalb_debug_last(self):
+        """For the last GPU Felzenszwalb on this handle: smoothed (HxWx3 float64, /255 and the Gaussian; None after the
+        graph tap) and rounds (the rounds of the merge pass and of the min-size pass)."""
+        shape = getattr(self, "_felzenszwalb_shape", None)
+        smoothed = np.empty(shape + (3,), np.float64) if shape else None
+        rounds = np.zeros(2, np.int32)
+        self._check(self.lib.pcm_felzenszwalb_debug_last(self._h, _ptr(smoothed), _ptr(rounds)))
+        return dict(smoothed=smoothed, rounds=(int(rounds[0]), int(rounds[1])))
 
     def slic(self, frame, rect, n_segments=250, compactness=10.0, sigma=1.0, max_iter=10, start_label=0, want_labels=True,
              kernel=None):

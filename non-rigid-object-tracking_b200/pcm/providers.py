@@ -44,8 +44,8 @@ def make_segment_provider(name, **kw):
     """Resolve `params.over_segmentation` (config.yaml:29) to a label provider.
 
     'grid[:block]' and 'voronoi[:sites]' are deterministic test providers.  The reference's names ('quickshift',
-    'felzenszwalb', 'SLIC') normally never get here -- the masker runs all three natively (pcm_quickshift / pcm_slic_gpu on
-    the GPU, pcm_felzenszwalb in the library's host code, SURVEY.md §8 f-1); asked for explicitly they map to the grid
+    'felzenszwalb', 'SLIC') normally never get here -- the masker runs all three natively on the GPU (pcm_quickshift /
+    pcm_felzenszwalb_gpu / pcm_slic_gpu, SURVEY.md §8 f-1); asked for explicitly they map to the grid
     provider with a block size giving a comparable superpixel count.
     """
     name = str(name)
