@@ -299,7 +299,11 @@ int pcm_felzenszwalb_device(pcm_handle* h, const uint8_t* d_frame, int frame_h, 
                             int32_t* d_labels_out, int* n_labels_out);
 
 /* The Felzenszwalb maps of n crops of a device-resident clip in one call, laid out like pcm_quickshift_device_batch's:
- * exactly n calls of pcm_felzenszwalb_device without returning to the caller in between. */
+ * the same maps and counts as n calls of pcm_felzenszwalb_device.  The crops run in one batched pass: consecutive crops
+ * are grouped into chunks of at most 2^23 pixels (a larger crop is a chunk of its own), and each chunk is one graph of
+ * disjoint pieces whose merge rounds serve all its crops at once, so it takes as many rounds as its slowest crop.  Every
+ * crop is checked before any work is queued; the counts come back with one wait for the whole batch.  Like every
+ * over-segmentation call (n > 0), it ends a pending pcm_update(labels == NULL) handoff. */
 int pcm_felzenszwalb_device_batch(pcm_handle* h, int n, const uint8_t* d_frames, int64_t frame_bytes, const int32_t* frame_index,
                                   int frame_h, int frame_w, int64_t frame_stride, const int32_t* rects, double scale, double sigma,
                                   int min_size, const double* kernel, int kernel_radius, int32_t* d_labels_out,
@@ -310,9 +314,10 @@ int pcm_felzenszwalb_device_batch(pcm_handle* h, int n, const uint8_t* d_frames,
 int pcm_felzenszwalb_graph_gpu(pcm_handle* h, int n_vertices, int n_edges, const int32_t* a, const int32_t* b,
                                const double* cost, double scale, int min_size, int32_t* labels_out, int* n_labels_out);
 
-/* Parity tap: for the last pcm_felzenszwalb_gpu / _device / _graph_gpu call on the handle, smoothed (h*w*3 float64 of that
- * crop: /255 and the Gaussian; NULL skips it, and it must be NULL after the graph tap) and rounds[2] (int32: the rounds
- * of the merge pass and of the min-size pass; NULL skips it).  PCM_E_STATE before any such call. */
+/* Parity tap: for the last pcm_felzenszwalb_gpu / _device / _device_batch / _graph_gpu call on the handle, smoothed (h*w*3
+ * float64 of that call's last crop: /255 and the Gaussian; NULL skips it, and it must be NULL after the graph tap) and
+ * rounds[2] (int32: the rounds of the merge pass and of the min-size pass -- after a batch, the largest over its crops;
+ * NULL skips it).  PCM_E_STATE before any such call. */
 int pcm_felzenszwalb_debug_last(pcm_handle* h, double* smoothed, int32_t* rounds);
 
 /* ---- a whole sequence of frames in one call (main.py:280-343 for one target) ---- */

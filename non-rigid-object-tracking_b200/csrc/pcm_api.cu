@@ -317,12 +317,15 @@ struct pcm_handle {
     DevBuf sl_parent, sl_root, sl_csize, sl_piece, sl_psize, sl_off, sl_queue, sl_seen, sl_adj, sl_nxt, sl_val, sl_labels;
     PinBuf h_slic;                // Gaussian weights + seed centres
     int sl_w = 0, sl_h = 0;       // crop of the stage results; 0: none
-    // Felzenszwalb (pcm_felzenszwalb_gpu / _device* / _graph_gpu): edges, sort, the state of the rounds, labels.  fz_smooth
-    // and fz_ctr (round counts) keep the stage results of the last call (pcm_felzenszwalb_debug_last).
-    DevBuf fz_kernel, fz_smooth, fz_tmp, fz_ea, fz_eb, fz_key, fz_key_sorted, fz_idx, fz_idx_sorted, fz_list0, fz_list1, fz_parent,
-           fz_size, fz_limit, fz_m, fz_root, fz_flag, fz_rank, fz_sums, fz_ctr, fz_count, fz_cub;
-    PinBuf h_fz;                  // Gaussian weights
-    int fz_w = 0, fz_h = 0;       // crop of fz_smooth; 0: the last call was the graph tap
+    // Felzenszwalb (pcm_felzenszwalb_gpu / _device* / _graph_gpu): edges, sort, the state of the rounds, labels, one count
+    // per crop (fz_count).  fz_smooth and fz_rounds (two round counts per chunk) keep the stage results of the last call
+    // (pcm_felzenszwalb_debug_last).
+    DevBuf fz_args, fz_smooth, fz_tmp, fz_ea, fz_eb, fz_key, fz_key_sorted, fz_idx, fz_idx_sorted, fz_list0, fz_list1, fz_parent,
+           fz_size, fz_limit, fz_m, fz_root, fz_flag, fz_rank, fz_sums, fz_ctr, fz_count, fz_rounds, fz_cub;
+    PinBuf h_fz;                  // Gaussian weights + crop table (fz_args)
+    int fz_w = 0, fz_h = 0;       // last crop of the last call, at pixel fz_px of fz_smooth; 0: the last call was the graph tap
+    int fz_px = 0;
+    int fz_chunks = 0;            // chunks of the last call
     bool fz_valid = false;        // a call has left round counts
     // forest training (pcm_fit_forest): feature-major rows resident between calls, scratch, outputs
     DevBuf fit_x, fit_xt, fit_y, fit_counts, fit_rand, fit_samples, fit_tmp, fit_out;
@@ -1699,7 +1702,7 @@ static int seg_device(pcm_handle* h, const char* who, const uint8_t* d_frame, in
     return PCM_OK;
 }
 
-// The *_device_batch entry points: crop k = rects[4k .. 4k+3] of the frame d_frames + frame_index[k] * frame_bytes through
+// The quickshift and SLIC *_device_batch entry points: crop k = rects[4k .. 4k+3] of the frame d_frames + frame_index[k] * frame_bytes through
 // one(d_frame, rect, d_labels, &count), the single-crop entry point, into d_labels_out + label_offsets[k]
 template <typename One>
 static int seg_device_batch(pcm_handle* h, const char* who, int n, const uint8_t* d_frames, int64_t frame_bytes,
@@ -2236,9 +2239,11 @@ static int launch_fz_rounds(pcm_handle* h, int n_vertices, int n_edges, double s
     return PCM_OK;
 }
 
-// F3-F6 of pcm_felzenszwalb.cuh on the n_edges edges in fz_ea / fz_eb / fz_key / fz_idx (edge order): labels into d_labels,
-// their count into fz_count, the round counts of the two passes into fz_ctr[4..5].  Asynchronous.
-static int enqueue_fz_merge(pcm_handle* h, int n, int n_edges, double sc, int min_size, int32_t* d_labels) {
+// F3-F6 of pcm_felzenszwalb.cuh on a chunk: the n_crops crops at d_crops (device), n pixels, the n_edges edges in fz_ea /
+// fz_eb / fz_key / fz_idx (edge order).  Labels into each crop's `labels`, counts into d_counts[0 .. n_crops), the round
+// counts of the two passes into rounds[0..1].  Asynchronous.
+static int enqueue_fz_merge(pcm_handle* h, const FzCrop* d_crops, int n_crops, int n, int n_edges, double sc, int min_size,
+                            int* d_counts, int* rounds) {
     cudaStream_t st = h->stream;
     const size_t ib = (size_t)n * sizeof(int);
     for (DevBuf* b : {&h->fz_parent, &h->fz_size, &h->fz_root, &h->fz_flag, &h->fz_rank}) CUDA_TRY(b->reserve(ib));
@@ -2252,7 +2257,6 @@ static int enqueue_fz_merge(pcm_handle* h, int n, int n_edges, double sc, int mi
     CUDA_TRY(h->fz_list0.reserve(ne * sizeof(FzEdge)));
     CUDA_TRY(h->fz_list1.reserve(ne * sizeof(FzEdge)));
     CUDA_TRY(h->fz_ctr.reserve(8 * sizeof(int)));
-    CUDA_TRY(h->fz_count.reserve(sizeof(int)));
     size_t cub_bytes = 0;
     CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, (const unsigned long long*)nullptr, (unsigned long long*)nullptr,
                                              (const int*)nullptr, (int*)nullptr, n_edges));
@@ -2275,7 +2279,7 @@ static int enqueue_fz_merge(pcm_handle* h, int n, int n_edges, double sc, int mi
     fz_gather_kernel<<<blocks, 256, 0, st>>>(h->fz_idx_sorted.as<int>(), h->fz_ea.as<int>(), h->fz_eb.as<int>(), nullptr, n_edges,
                                              list, ctr);
     CHECK_LAUNCH(h, "fz_gather_kernel");
-    if (int rc = launch_fz_rounds<false>(h, n, n_edges, sc, min_size, ctr + 4)) return rc;
+    if (int rc = launch_fz_rounds<false>(h, n, n_edges, sc, min_size, rounds)) return rc;
     // F5: every pixel's root, then the min-size pass over all edges again, in the same order
     CUDA_TRY(cudaMemsetAsync(flag, 0, ib, st));
     qs_root_kernel<<<blocks, 256, 0, st>>>(parent, root, flag, n);
@@ -2283,29 +2287,51 @@ static int enqueue_fz_merge(pcm_handle* h, int n, int n_edges, double sc, int mi
     fz_gather_kernel<<<blocks, 256, 0, st>>>(h->fz_idx_sorted.as<int>(), h->fz_ea.as<int>(), h->fz_eb.as<int>(), root, n_edges,
                                              list, ctr);
     CHECK_LAUNCH(h, "fz_gather_kernel");
-    if (int rc = launch_fz_rounds<true>(h, n, n_edges, sc, min_size, ctr + 5)) return rc;
-    // F6: label = rank of the root among all roots, count = number of roots
+    if (int rc = launch_fz_rounds<true>(h, n, n_edges, sc, min_size, rounds + 1)) return rc;
+    // F6: rank of each root among the chunk's roots (their number into ctr[6]), then label = rank within the crop
     CUDA_TRY(cudaMemsetAsync(flag, 0, ib, st));
     qs_root_kernel<<<blocks, 256, 0, st>>>(parent, root, flag, n);
     CHECK_LAUNCH(h, "qs_root_kernel");
     qs_scan_reduce_kernel<<<n_scan, 256, 0, st>>>(flag, n, h->fz_sums.as<int>());
     CHECK_LAUNCH(h, "qs_scan_reduce_kernel");
-    qs_scan_sums_kernel<<<1, 256, 0, st>>>(h->fz_sums.as<int>(), n_scan, h->fz_count.as<int>());
+    qs_scan_sums_kernel<<<1, 256, 0, st>>>(h->fz_sums.as<int>(), n_scan, ctr + 6);
     CHECK_LAUNCH(h, "qs_scan_sums_kernel");
     qs_scan_apply_kernel<<<n_scan, 256, 0, st>>>(flag, n, h->fz_sums.as<int>(), h->fz_rank.as<int>());
     CHECK_LAUNCH(h, "qs_scan_apply_kernel");
-    qs_label_kernel<<<blocks, 256, 0, st>>>(root, h->fz_rank.as<int>(), d_labels, n);
-    CHECK_LAUNCH(h, "qs_label_kernel");
+    fz_label_kernel<<<blocks, 256, 0, st>>>(d_crops, n_crops, n, root, h->fz_rank.as<int>(), ctr + 6, d_counts);
+    CHECK_LAUNCH(h, "fz_label_kernel");
     h->fz_valid = true;
     return PCM_OK;
 }
 
-// The whole Felzenszwalb of the crop (cx, cy, w, hh) of a device frame into seg_labels, its count into fz_count.
-// Asynchronous apart from the host-side staging of the weights (the caller has synchronised the stream).
-static int enqueue_felzenszwalb(pcm_handle* h, const uint8_t* d_frame, int64_t stride, int cx, int cy, int w, int hh, double scale,
-                                double sigma, int min_size, const double* kernel, int radius) {
-    const int n = w * hh;
-    const long long n_edges = (long long)hh * (w - 1) + (long long)(hh - 1) * w + 2LL * (hh - 1) * (w - 1);
+// Stages the Gaussian weights (nk of them) and n crop descriptors in h_fz and uploads them to fz_args in one copy; *dk and
+// *dc point at them there.  The caller has synchronised the stream (h_fz is reused between calls).
+static int upload_fz_args(pcm_handle* h, const double* kernel, size_t nk, const FzCrop* crops, int n, const double** dk,
+                          const FzCrop** dc) {
+    const size_t wbytes = nk * sizeof(double), bytes = wbytes + (size_t)n * sizeof(FzCrop);
+    CUDA_TRY(h->h_fz.reserve(bytes));
+    CUDA_TRY(h->fz_args.reserve(bytes));
+    if (nk) memcpy(h->h_fz.p, kernel, wbytes);
+    memcpy(h->h_fz.as<char>() + wbytes, crops, (size_t)n * sizeof(FzCrop));
+    CUDA_TRY(cudaMemcpyAsync(h->fz_args.p, h->h_fz.p, bytes, cudaMemcpyHostToDevice, h->stream));
+    h->bytes_h2d += (int64_t)bytes;
+    *dk = h->fz_args.as<double>();
+    *dc = reinterpret_cast<const FzCrop*>(h->fz_args.as<char>() + wbytes);
+    return PCM_OK;
+}
+
+// Crops per chunk of one pass: at most this many pixels, and so fewer than four times as many edges.  That keeps the chunk's
+// indices in int32 and its working memory (about 400 B per pixel) bounded.  A larger crop is a chunk of its own, up to the
+// single-crop limit of 2^28 pixels.
+constexpr long long FZ_CHUNK_PIXELS = 1LL << 23;
+
+// The whole Felzenszwalb of the crops `crops` (frame, labels and rect set; px and eb are set here) of frames with row stride
+// `stride`: consecutive crops are grouped into chunks of at most FZ_CHUNK_PIXELS pixels, and each chunk is one pass of
+// F1-F6, with a number of launches that does not depend on its number of crops.  Crop k's count goes to d_counts[k].
+// Asynchronous apart from the host-side staging of the weights and the crop table (the caller has synchronised the stream).
+static int enqueue_felzenszwalb(pcm_handle* h, std::vector<FzCrop>& crops, int64_t stride, double scale, double sigma, int min_size,
+                                const double* kernel, int radius, int* d_counts) {
+    const int n = (int)crops.size();
     cudaStream_t st = h->stream;
     h->chain_tail = false;
     h->fz_w = h->fz_h = 0;
@@ -2313,43 +2339,71 @@ static int enqueue_felzenszwalb(pcm_handle* h, const uint8_t* d_frame, int64_t s
     std::vector<double> kw;
     kernel = gaussian_weights(sigma, kernel, radius, kw);
     const size_t nk = kernel ? (size_t)(2 * radius + 1) : 0;
-    const size_t db = (size_t)n * 3 * sizeof(double), ne = (size_t)std::max(n_edges, 1LL);
-    CUDA_TRY(h->fz_kernel.reserve(std::max<size_t>(nk, 1) * sizeof(double)));
+    std::vector<int> first;                           // first crop of each chunk, then n
+    long long px = 0, eb = 0, max_px = 1, max_edges = 1;
+    for (int k = 0; k < n; ++k) {
+        const long long p = (long long)crops[k].w * crops[k].h;
+        if (k == 0 || px + p > FZ_CHUNK_PIXELS) { first.push_back(k); px = eb = 0; }
+        crops[k].px = (int)px;
+        crops[k].eb = (int)eb;
+        px += p;
+        eb += fz_edge_count(crops[k].w, crops[k].h);
+        max_px = std::max(max_px, px);
+        max_edges = std::max(max_edges, eb);
+    }
+    first.push_back(n);
+    const int n_chunks = (int)first.size() - 1;
+    const size_t db = (size_t)max_px * 3 * sizeof(double);
     CUDA_TRY(h->fz_smooth.reserve(db));
     if (nk) CUDA_TRY(h->fz_tmp.reserve(db));
-    CUDA_TRY(h->fz_ea.reserve(ne * sizeof(int)));
-    CUDA_TRY(h->fz_eb.reserve(ne * sizeof(int)));
-    CUDA_TRY(h->fz_idx.reserve(ne * sizeof(int)));
-    CUDA_TRY(h->fz_key.reserve(ne * sizeof(unsigned long long)));
-    CUDA_TRY(h->seg_labels.reserve((size_t)n * sizeof(int32_t)));
-    if (nk) {
-        CUDA_TRY(h->h_fz.reserve(nk * sizeof(double)));
-        memcpy(h->h_fz.p, kernel, nk * sizeof(double));
-        CUDA_TRY(cudaMemcpyAsync(h->fz_kernel.p, h->h_fz.p, nk * sizeof(double), cudaMemcpyHostToDevice, st));
-        h->bytes_h2d += (int64_t)(nk * sizeof(double));
-    }
-    const int blocks = (int)std::min<long long>(((long long)n + SLIC_THREADS - 1) / SLIC_THREADS, (long long)h->sm_count * 16);
-    const double* dk = h->fz_kernel.as<double>();
+    CUDA_TRY(h->fz_ea.reserve((size_t)max_edges * sizeof(int)));
+    CUDA_TRY(h->fz_eb.reserve((size_t)max_edges * sizeof(int)));
+    CUDA_TRY(h->fz_idx.reserve((size_t)max_edges * sizeof(int)));
+    CUDA_TRY(h->fz_key.reserve((size_t)max_edges * sizeof(unsigned long long)));
+    CUDA_TRY(h->fz_rounds.reserve((size_t)n_chunks * 2 * sizeof(int)));
+    const double* dk = nullptr;
+    const FzCrop* dc = nullptr;
+    if (int rc = upload_fz_args(h, kernel, nk, crops.data(), n, &dk, &dc)) return rc;
     double* smooth = h->fz_smooth.as<double>();
-    // F1: byte / 255 and the Gaussian along rows, then columns (no Gaussian when sigma <= 0)
-    slic_load_kernel<<<blocks, SLIC_THREADS, 0, st>>>(d_frame, stride, cx, cy, w, hh, dk, radius, 0, smooth);
-    CHECK_LAUNCH(h, "slic_load_kernel");
-    if (nk) {
-        slic_smooth_kernel<<<blocks, SLIC_THREADS, 0, st>>>(smooth, h->fz_tmp.as<double>(), hh, w, 0, dk, radius);
-        CHECK_LAUNCH(h, "slic_smooth_kernel");
-        slic_smooth_kernel<<<blocks, SLIC_THREADS, 0, st>>>(h->fz_tmp.as<double>(), smooth, hh, w, 1, dk, radius);
-        CHECK_LAUNCH(h, "slic_smooth_kernel");
+    for (int c = 0; c < n_chunks; ++c) {
+        const int k0 = first[c], nc = first[c + 1] - k0;
+        const FzCrop& last = crops[first[c + 1] - 1];
+        const int n_px = last.px + last.w * last.h;
+        const long long n_edges = last.eb + fz_edge_count(last.w, last.h);
+        const int blocks = (int)std::min<long long>(((long long)n_px + 255) / 256, (long long)h->sm_count * 16);
+        // F1: byte / 255 and the Gaussian along rows, then columns (no Gaussian when sigma <= 0)
+        fz_load_kernel<<<blocks, 256, 0, st>>>(dc + k0, nc, stride, n_px, smooth);
+        CHECK_LAUNCH(h, "fz_load_kernel");
+        if (nk) {
+            fz_smooth_kernel<<<blocks, 256, 0, st>>>(dc + k0, nc, n_px, smooth, h->fz_tmp.as<double>(), 0, dk, radius);
+            CHECK_LAUNCH(h, "fz_smooth_kernel");
+            fz_smooth_kernel<<<blocks, 256, 0, st>>>(dc + k0, nc, n_px, h->fz_tmp.as<double>(), smooth, 1, dk, radius);
+            CHECK_LAUNCH(h, "fz_smooth_kernel");
+        }
+        // F2: the edges in the host's order, crop after crop
+        if (n_edges > 0) {
+            const int eblocks = (int)std::min<long long>((n_edges + 255) / 256, (long long)h->sm_count * 16);
+            fz_cost_kernel<<<eblocks, 256, 0, st>>>(dc + k0, nc, (int)n_edges, smooth, h->fz_ea.as<int>(), h->fz_eb.as<int>(),
+                                                    h->fz_key.as<unsigned long long>(), h->fz_idx.as<int>());
+            CHECK_LAUNCH(h, "fz_cost_kernel");
+        }
+        if (int rc = enqueue_fz_merge(h, dc + k0, nc, n_px, (int)n_edges, scale / 255.0, min_size, d_counts + k0,
+                                      h->fz_rounds.as<int>() + 2 * c))
+            return rc;
     }
-    // F2: the edges in the host's order
-    if (n_edges > 0) {
-        const int eblocks = (int)std::min<long long>((n_edges + 255) / 256, (long long)h->sm_count * 16);
-        fz_cost_kernel<<<eblocks, 256, 0, st>>>(smooth, hh, w, h->fz_ea.as<int>(), h->fz_eb.as<int>(),
-                                                h->fz_key.as<unsigned long long>(), h->fz_idx.as<int>());
-        CHECK_LAUNCH(h, "fz_cost_kernel");
-    }
-    if (int rc = enqueue_fz_merge(h, n, (int)n_edges, scale / 255.0, min_size, h->seg_labels.as<int32_t>())) return rc;
-    h->fz_w = w; h->fz_h = hh;
+    h->fz_chunks = n_chunks;
+    h->fz_w = crops[n - 1].w; h->fz_h = crops[n - 1].h;
+    h->fz_px = crops[n - 1].px;
     return PCM_OK;
+}
+
+// The single-crop entry points: the crop (cx, cy, w, hh) of a device frame into seg_labels, its count into fz_count
+static int enqueue_felzenszwalb_one(pcm_handle* h, const uint8_t* d_frame, int64_t stride, int cx, int cy, int w, int hh,
+                                    double scale, double sigma, int min_size, const double* kernel, int radius) {
+    CUDA_TRY(h->seg_labels.reserve((size_t)w * hh * sizeof(int32_t)));
+    CUDA_TRY(h->fz_count.reserve(sizeof(int)));
+    std::vector<FzCrop> crop{{d_frame, h->seg_labels.as<int32_t>(), cx, cy, w, hh, 0, 0}};
+    return enqueue_felzenszwalb(h, crop, stride, scale, sigma, min_size, kernel, radius, h->fz_count.as<int>());
 }
 
 extern "C" int pcm_felzenszwalb_device(pcm_handle* h, const uint8_t* d_frame, int H, int W, int64_t stride, const int rect[4],
@@ -2358,9 +2412,9 @@ extern "C" int pcm_felzenszwalb_device(pcm_handle* h, const uint8_t* d_frame, in
     return seg_device(h, "pcm_felzenszwalb_device", d_frame, H, W, stride, rect, &pcm_handle::fz_count, 0, d_labels_out, n_labels_out,
                       [&] {
                           if (int rc = check_felzenszwalb_args("pcm_felzenszwalb_device", rect, kernel, kernel_radius)) return rc;
-                          CUDA_TRY(cudaStreamSynchronize(h->stream));      // the pinned weight buffer is reused between calls
-                          return enqueue_felzenszwalb(h, d_frame, stride, rect[0], rect[1], rect[2], rect[3], scale, sigma, min_size,
-                                                      kernel, kernel_radius);
+                          CUDA_TRY(cudaStreamSynchronize(h->stream));      // the pinned staging buffer is reused between calls
+                          return enqueue_felzenszwalb_one(h, d_frame, stride, rect[0], rect[1], rect[2], rect[3], scale, sigma,
+                                                          min_size, kernel, kernel_radius);
                       });
 }
 
@@ -2368,11 +2422,34 @@ extern "C" int pcm_felzenszwalb_device_batch(pcm_handle* h, int n, const uint8_t
                                              const int32_t* frame_index, int H, int W, int64_t stride, const int32_t* rects,
                                              double scale, double sigma, int min_size, const double* kernel, int kernel_radius,
                                              int32_t* d_labels_out, const int64_t* label_offsets, int32_t* n_labels_out) {
-    return seg_device_batch(h, "pcm_felzenszwalb_device_batch", n, d_frames, frame_bytes, frame_index, rects, d_labels_out,
-                            label_offsets, n_labels_out, [&](const uint8_t* d_frame, const int rect[4], int32_t* d_labels, int* count) {
-                                return pcm_felzenszwalb_device(h, d_frame, H, W, stride, rect, scale, sigma, min_size, kernel,
-                                                               kernel_radius, d_labels, count);
-                            });
+    const char* who = "pcm_felzenszwalb_device_batch";
+    if (!h || !d_frames || !frame_index || !rects || !d_labels_out || !label_offsets || !n_labels_out)
+        return fail(PCM_E_INVALID, "%s: NULL argument", who);
+    if (n < 0 || frame_bytes < 0) return fail(PCM_E_INVALID, "%s: bad count / frame size", who);
+    if (n == 0) return PCM_OK;
+    if (stride < (int64_t)W * 3) return fail(PCM_E_INVALID, "%s: stride %lld < 3*W", who, (long long)stride);
+    // every crop is checked before any work is queued
+    std::vector<FzCrop> crops((size_t)n);
+    char where[64];
+    for (int k = 0; k < n; ++k) {
+        if (frame_index[k] < 0 || label_offsets[k] < 0) return fail(PCM_E_INVALID, "%s: crop %d: negative index", who, k);
+        const int rect[4] = {rects[4 * k], rects[4 * k + 1], rects[4 * k + 2], rects[4 * k + 3]};
+        snprintf(where, sizeof where, "%s: crop %d", who, k);
+        if (int rc = check_rect(where, rect, H, W)) return rc;
+        if (int rc = check_felzenszwalb_args(where, rect, kernel, kernel_radius)) return rc;
+        crops[k] = {d_frames + (int64_t)frame_index[k] * frame_bytes, d_labels_out + label_offsets[k], rect[0], rect[1], rect[2],
+                    rect[3], 0, 0};
+    }
+    CUDA_TRY(cudaSetDevice(h->device));
+    h->handoff.valid = false;
+    CUDA_TRY(h->fz_count.reserve((size_t)n * sizeof(int)));
+    CUDA_TRY(cudaStreamSynchronize(h->stream));      // the pinned staging buffer is reused between calls
+    if (int rc = enqueue_felzenszwalb(h, crops, stride, scale, sigma, min_size, kernel, kernel_radius, h->fz_count.as<int>()))
+        return rc;
+    // every crop's count, one copy and one wait for the batch
+    CUDA_TRY(cudaMemcpyAsync(n_labels_out, h->fz_count.p, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(cudaStreamSynchronize(h->stream));
+    return PCM_OK;
 }
 
 extern "C" int pcm_felzenszwalb_gpu(pcm_handle* h, const uint8_t* frame, int H, int W, int64_t stride, const int rect[4],
@@ -2382,8 +2459,8 @@ extern "C" int pcm_felzenszwalb_gpu(pcm_handle* h, const uint8_t* frame, int H, 
     if (rc) return rc;
     if ((rc = check_felzenszwalb_args("pcm_felzenszwalb_gpu", rect, kernel, kernel_radius))) return rc;
     if ((rc = stage_crop(h, "pcm_felzenszwalb_gpu", frame, stride, rect, 0, [](int) { return cudaSuccess; }))) return rc;
-    rc = enqueue_felzenszwalb(h, h->frame.as<uint8_t>(), (int64_t)rect[2] * 3, 0, 0, rect[2], rect[3], scale, sigma, min_size, kernel,
-                              kernel_radius);
+    rc = enqueue_felzenszwalb_one(h, h->frame.as<uint8_t>(), (int64_t)rect[2] * 3, 0, 0, rect[2], rect[3], scale, sigma, min_size,
+                                  kernel, kernel_radius);
     if (rc) return rc;
     return finish_host_seg(h, frame, rect, h->fz_count.as<int>(), 0, labels_out, n_labels_out);
 }
@@ -2406,7 +2483,15 @@ extern "C" int pcm_felzenszwalb_graph_gpu(pcm_handle* h, int n_vertices, int n_e
     CUDA_TRY(h->fz_idx.reserve(ne * sizeof(int)));
     CUDA_TRY(h->fz_key.reserve(ne * sizeof(unsigned long long)));
     CUDA_TRY(h->seg_labels.reserve(ib));
+    CUDA_TRY(h->fz_count.reserve(sizeof(int)));
+    CUDA_TRY(h->fz_rounds.reserve(2 * sizeof(int)));
     h->handoff.valid = false;                          // seg_labels is about to be replaced
+    CUDA_TRY(cudaStreamSynchronize(st));               // the pinned staging buffer is reused between calls
+    // the graph is one crop of n_vertices x 1 pixels whose labels go to seg_labels
+    const FzCrop crop{nullptr, h->seg_labels.as<int32_t>(), 0, 0, n_vertices, 1, 0, 0};
+    const double* dk = nullptr;
+    const FzCrop* dc = nullptr;
+    if (int rc = upload_fz_args(h, nullptr, 0, &crop, 1, &dk, &dc)) return rc;
     // the cost bits are the sort keys
     CUDA_TRY(cudaMemcpyAsync(h->fz_ea.p, a, (size_t)n_edges * sizeof(int), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(h->fz_eb.p, b, (size_t)n_edges * sizeof(int), cudaMemcpyHostToDevice, st));
@@ -2416,8 +2501,9 @@ extern "C" int pcm_felzenszwalb_graph_gpu(pcm_handle* h, int n_vertices, int n_e
             h->fz_idx.as<int>(), n_edges);
         CHECK_LAUNCH(h, "slic_ccl_init_kernel");
     }
-    int rc = enqueue_fz_merge(h, n_vertices, n_edges, scale, min_size, h->seg_labels.as<int32_t>());
+    int rc = enqueue_fz_merge(h, dc, 1, n_vertices, n_edges, scale, min_size, h->fz_count.as<int>(), h->fz_rounds.as<int>());
     if (rc) return rc;
+    h->fz_chunks = 1;
     CUDA_TRY(cudaMemcpyAsync(labels_out, h->seg_labels.p, ib, cudaMemcpyDeviceToHost, st));
     int count = 0;
     if ((rc = read_seg_count(h, h->fz_count.as<int>(), 0, &count))) return rc;
@@ -2433,9 +2519,19 @@ extern "C" int pcm_felzenszwalb_debug_last(pcm_handle* h, double* smoothed, int3
     CUDA_TRY(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
     if (smoothed)
-        CUDA_TRY(cudaMemcpyAsync(smoothed, h->fz_smooth.p, (size_t)h->fz_w * h->fz_h * 3 * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (rounds) CUDA_TRY(cudaMemcpyAsync(rounds, h->fz_ctr.as<int>() + 4, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(smoothed, h->fz_smooth.as<double>() + 3LL * h->fz_px, (size_t)h->fz_w * h->fz_h * 3 * sizeof(double),
+                                 cudaMemcpyDeviceToHost, st));
+    std::vector<int32_t> per_chunk((size_t)2 * h->fz_chunks);
+    if (rounds)
+        CUDA_TRY(cudaMemcpyAsync(per_chunk.data(), h->fz_rounds.p, per_chunk.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
+    if (rounds) {                                      // a batch takes as many rounds as its slowest chunk
+        rounds[0] = rounds[1] = 0;
+        for (int c = 0; c < h->fz_chunks; ++c) {
+            rounds[0] = std::max(rounds[0], per_chunk[2 * c]);
+            rounds[1] = std::max(rounds[1], per_chunk[2 * c + 1]);
+        }
+    }
     return PCM_OK;
 }
 

@@ -1,15 +1,20 @@
 // pcm_felzenszwalb.cuh -- Felzenszwalb-Huttenlocher over-segmentation of the crop on the GPU, the second over-segmentation
 // the reference offers (maskers/pixel_classification.py:72-73: felzenszwalb(crop, scale=100, sigma=0.5, min_size=50)).
 //
-// The specification is the host code of pcm_felzenszwalb.cpp; the labels and the count are the same, bit for bit:
-//   F1 slic_load_kernel (depth 0) and two slic_smooth_kernel passes (pcm_slic.cuh): byte / 255, the Gaussian along rows,
-//      then along columns -- the host's smooth_axis, operation for operation
-//   F2 fz_cost_kernel      the edges in the host's order (right, down, down-right, up-right; raster order within a class):
-//                          endpoints and the bit pattern of sqrt((d0*d0 + d1*d1) + d2*d2)
-//   F3 CUB radix sort of (cost bits, edge index): stable, so equal costs keep edge order, as the host's sort does
+// The specification is the host code of pcm_felzenszwalb.cpp; the labels and the count are the same, bit for bit.  Every
+// call runs on a chunk of crops (FzCrop; one crop for the single-crop entry points), as one graph of disjoint pieces:
+//   F1 fz_load_kernel, two fz_smooth_kernel passes: byte / 255, the Gaussian along rows, then along columns -- the code of
+//      slic_load_kernel / slic_smooth_kernel (pcm_slic.cuh), and so the host's smooth_axis, operation for operation
+//   F2 fz_cost_kernel      each crop's edges in the host's order (right, down, down-right, up-right; raster order within a
+//                          class), crop after crop: endpoints and the bit pattern of sqrt((d0*d0 + d1*d1) + d2*d2)
+//   F3 CUB radix sort of (cost bits, edge index): stable, so equal costs keep edge order, as the host's sort does; restricted
+//      to one crop it is that crop's own order
 //   F4 fz_rounds_kernel<false>   the greedy merge pass, in rounds (below)
 //   F5 qs_root_kernel, then fz_rounds_kernel<true>   the min-size pass, in rounds
-//   F6 qs_root_kernel + the qs_scan_* kernels + qs_label_kernel (pcm_quickshift.cuh): label = rank of the root
+//   F6 qs_root_kernel + the qs_scan_* kernels (pcm_quickshift.cuh) + fz_label_kernel: label = rank of the root in its crop
+// A round decides an edge from its own two components only, and no component spans two crops, so every round makes in
+// every crop exactly the decisions that crop makes alone: the labels are the crop's own, and a chunk takes as many rounds
+// as its slowest crop.
 //
 // The merge pass in rounds.  A component X (root = its smallest pixel, as the host's join keeps it) has size[X] and
 // limit[X] = Int(X) + sc / |X|.  Each round looks at the remaining edges, in sorted position p, with current roots ra, rb:
@@ -32,6 +37,8 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "pcm_slic.cuh"
+
 namespace pcm {
 
 constexpr int FZ_THREADS = 512;
@@ -39,36 +46,88 @@ constexpr int FZ_THREADS = 512;
 // sync, and on SegTrack2 crops most rounds see under 1 % of the edges
 constexpr int FZ_TAIL_EDGES = 4 * FZ_THREADS;
 
-// F2: edge i of the host's array: endpoints (a, b) and the bit pattern of its cost (>= +0, so the bits order like the value)
-__global__ void __launch_bounds__(256) fz_cost_kernel(const double* __restrict__ img, int h, int w, int* __restrict__ ea,
-                                                      int* __restrict__ eb, unsigned long long* __restrict__ key,
-                                                      int* __restrict__ idx) {
-    const long long n_right = (long long)h * (w - 1), n_down = (long long)(h - 1) * w, n_diag = (long long)(h - 1) * (w - 1);
-    const long long total = n_right + n_down + 2 * n_diag;
+// One crop of a batched pass.  A chunk of crops is one graph of disjoint pieces: crop k owns the chunk's pixels px ..
+// px + w*h - 1 and its edges eb .. eb + edges(w, h) - 1, in crop order; its labels go to `labels` (w*h, raster order).
+struct FzCrop {
+    const uint8_t* frame;          // the frame the crop is cut from (row stride: the batch's)
+    int32_t* labels;
+    int cx, cy, w, h;
+    int px, eb;                    // pixel base and edge base within the chunk
+};
+
+__host__ __device__ __forceinline__ long long fz_edge_count(int w, int h) {
+    return (long long)h * (w - 1) + (long long)(h - 1) * w + 2LL * (h - 1) * (w - 1);
+}
+
+// the crop of chunk element v: the last of the n crops whose pixel base (EDGE = false) or edge base (true) is <= v (a
+// crop without edges shares its edge base with the next one)
+template <bool EDGE>
+__device__ __forceinline__ int fz_crop_of(const FzCrop* __restrict__ crops, int n, long long v) {
+    int lo = 0, hi = n - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if ((EDGE ? crops[mid].eb : crops[mid].px) <= v) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// F1 of a chunk: pixel-channel i -> byte / 255 (slic_load_value, depth 0) into img, the chunk's pixels back to back
+__global__ void __launch_bounds__(256) fz_load_kernel(const FzCrop* __restrict__ crops, int n_crops, long long stride, int n_px,
+                                                      double* __restrict__ img) {
+    const long long total = 3LL * n_px;
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const FzCrop c = crops[fz_crop_of<false>(crops, n_crops, i / 3)];
+        img[i] = slic_load_value(c.frame, stride, c.cx, c.cy, c.w, nullptr, 0, 0, i - 3LL * c.px);
+    }
+}
+
+// F1 of a chunk: the Gaussian along rows (axis 0) or columns (1) of every crop (slic_smooth_pixel)
+__global__ void __launch_bounds__(256) fz_smooth_kernel(const FzCrop* __restrict__ crops, int n_crops, int n_px,
+                                                        const double* __restrict__ in, double* __restrict__ out, int axis,
+                                                        const double* __restrict__ k, int radius) {
+    for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < n_px; p += gridDim.x * blockDim.x) {
+        const FzCrop c = crops[fz_crop_of<false>(crops, n_crops, p)];
+        slic_smooth_pixel(in + 3LL * c.px, out + 3LL * c.px, c.h, c.w, axis, k, radius, p - c.px);
+    }
+}
+
+// F2: edge i of the host's array for an h x w image: endpoints (a, b) and the bit pattern of its cost (>= +0, so the bits
+// order like the value)
+__device__ __forceinline__ unsigned long long fz_edge(const double* __restrict__ img, int h, int w, long long i, int& a, int& b) {
+    const long long n_right = (long long)h * (w - 1), n_down = (long long)(h - 1) * w, n_diag = (long long)(h - 1) * (w - 1);
+    if (i < n_right) {                                      // (r, c) - (r, c-1), c >= 1
+        const int r = (int)(i / (w - 1)), c = (int)(i - (long long)r * (w - 1)) + 1;
+        a = r * w + c; b = a - 1;
+    } else if (i < n_right + n_down) {                      // (r, c) - (r-1, c), r >= 1
+        const long long j = i - n_right;
+        a = (int)j + w; b = (int)j;
+    } else {
+        const long long j = i - n_right - n_down;
+        const bool dr = j < n_diag;                         // down-right: (r, c) - (r-1, c-1); up-right: (r-1, c) - (r, c-1)
+        const long long k = dr ? j : j - n_diag;
+        const int r = (int)(k / (w - 1)) + 1, c = (int)(k - (long long)(r - 1) * (w - 1)) + 1;
+        if (dr) { a = r * w + c; b = (r - 1) * w + c - 1; }
+        else    { a = (r - 1) * w + c; b = r * w + c - 1; }
+    }
+    const double* p = img + 3LL * a;
+    const double* q = img + 3LL * b;
+    const double d0 = __dsub_rn(p[0], q[0]), d1 = __dsub_rn(p[1], q[1]), d2 = __dsub_rn(p[2], q[2]);
+    const double c = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(d0, d0), __dmul_rn(d1, d1)), __dmul_rn(d2, d2)));
+    return (unsigned long long)__double_as_longlong(c);
+}
+
+// F2 of a chunk: edge i = edge i - eb of its crop, endpoints as chunk pixel indices; idx = i, so that the stable sort
+// keeps crop k's edges after crop k-1's and, within a crop, in the host's order
+__global__ void __launch_bounds__(256) fz_cost_kernel(const FzCrop* __restrict__ crops, int n_crops, int n_edges,
+                                                      const double* __restrict__ img, int* __restrict__ ea, int* __restrict__ eb,
+                                                      unsigned long long* __restrict__ key, int* __restrict__ idx) {
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_edges; i += gridDim.x * blockDim.x) {
+        const FzCrop c = crops[fz_crop_of<true>(crops, n_crops, i)];
         int a, b;
-        if (i < n_right) {                                      // (r, c) - (r, c-1), c >= 1
-            const int r = (int)(i / (w - 1)), c = (int)(i - (long long)r * (w - 1)) + 1;
-            a = r * w + c; b = a - 1;
-        } else if (i < n_right + n_down) {                      // (r, c) - (r-1, c), r >= 1
-            const long long j = i - n_right;
-            a = (int)j + w; b = (int)j;
-        } else {
-            const long long j = i - n_right - n_down;
-            const bool dr = j < n_diag;                         // down-right: (r, c) - (r-1, c-1); up-right: (r-1, c) - (r, c-1)
-            const long long k = dr ? j : j - n_diag;
-            const int r = (int)(k / (w - 1)) + 1, c = (int)(k - (long long)(r - 1) * (w - 1)) + 1;
-            if (dr) { a = r * w + c; b = (r - 1) * w + c - 1; }
-            else    { a = (r - 1) * w + c; b = r * w + c - 1; }
-        }
-        const double* p = img + 3LL * a;
-        const double* q = img + 3LL * b;
-        const double d0 = __dsub_rn(p[0], q[0]), d1 = __dsub_rn(p[1], q[1]), d2 = __dsub_rn(p[2], q[2]);
-        const double c = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(d0, d0), __dmul_rn(d1, d1)), __dmul_rn(d2, d2)));
-        ea[i] = a;
-        eb[i] = b;
-        key[i] = (unsigned long long)__double_as_longlong(c);
-        idx[i] = (int)i;
+        key[i] = fz_edge(img + 3LL * c.px, c.h, c.w, i - c.eb, a, b);
+        ea[i] = c.px + a;
+        eb[i] = c.px + b;
+        idx[i] = i;
     }
 }
 
@@ -214,6 +273,21 @@ __global__ void __launch_bounds__(FZ_THREADS, 1) fz_rounds_kernel(FzRounds s) {
         if (single) __syncthreads(); else grid.sync();
     }
     if (blockIdx.x == 0 && threadIdx.x == 0) *s.rounds = round - 1;
+}
+
+// F6 of a chunk: roots are the smallest chunk pixel of their component, so within a crop they come in the crop's raster
+// order.  rank = exclusive scan of the root flags over the chunk, total = number of roots: crop k's label of pixel p is
+// rank[root[p]] - rank[px], its count rank[next crop's px] (or total) - rank[px], written by the crop's first pixel.
+__global__ void __launch_bounds__(256) fz_label_kernel(const FzCrop* __restrict__ crops, int n_crops, int n_px,
+                                                       const int* __restrict__ root, const int* __restrict__ rank,
+                                                       const int* __restrict__ total, int* __restrict__ counts) {
+    for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < n_px; p += gridDim.x * blockDim.x) {
+        const int k = fz_crop_of<false>(crops, n_crops, p);
+        const FzCrop c = crops[k];
+        const int base = rank[c.px];
+        c.labels[p - c.px] = rank[root[p]] - base;
+        if (p == c.px) counts[k] = (k + 1 < n_crops ? rank[crops[k + 1].px] : *total) - base;
+    }
 }
 
 }  // namespace pcm

@@ -35,49 +35,58 @@ __device__ __forceinline__ int slic_reflect(int i, int n) {     // scipy 'reflec
 }
 
 // S1: img = byte / 255 (h*w*3, interleaved as the crop); with `depth`, the Gaussian along the depth axis of length 1:
-// a = v*k[r], then a = a + (v+v)*k[r-j] for j = r..1
+// a = v*k[r], then a = a + (v+v)*k[r-j] for j = r..1.  Element i of the crop (cx, cy, w, *) of a frame of row stride
+// `stride`; the batched Felzenszwalb load runs the same code.
+__device__ __forceinline__ double slic_load_value(const uint8_t* __restrict__ frame, long long stride, int cx, int cy, int w,
+                                                  const double* __restrict__ k, int radius, int depth, long long i) {
+    const long long r = i / (3LL * w), rem = i - r * 3LL * w;
+    double v = __ddiv_rn((double)frame[(cy + r) * stride + (long long)cx * 3 + rem], 255.0);
+    if (depth) {
+        double a = __dmul_rn(v, k[radius]);
+        const double vv = __dadd_rn(v, v);
+        for (int j = radius; j >= 1; --j) a = __dadd_rn(a, __dmul_rn(vv, k[radius - j]));
+        v = a;
+    }
+    return v;
+}
+
 __global__ void __launch_bounds__(SLIC_THREADS) slic_load_kernel(const uint8_t* __restrict__ frame, long long stride, int cx, int cy,
                                                                  int w, int h, const double* __restrict__ k, int radius, int depth,
                                                                  double* __restrict__ out) {
     const long long total = (long long)w * h * 3;
-    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-        const long long r = i / (3LL * w), rem = i - r * 3LL * w;
-        double v = __ddiv_rn((double)frame[(cy + r) * stride + (long long)cx * 3 + rem], 255.0);
-        if (depth) {
-            double a = __dmul_rn(v, k[radius]);
-            const double vv = __dadd_rn(v, v);
-            for (int j = radius; j >= 1; --j) a = __dadd_rn(a, __dmul_rn(vv, k[radius - j]));
-            v = a;
-        }
-        out[i] = v;
-    }
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x)
+        out[i] = slic_load_value(frame, stride, cx, cy, w, k, radius, depth, i);
 }
 
 // S2: symmetric correlate along one axis (0: rows, 1: columns) of an h x w x 3 image: centre tap first, then the pairs
-// from the outside in
+// from the outside in.  Pixel p of the image; the batched Felzenszwalb smoothing runs the same code.
+__device__ __forceinline__ void slic_smooth_pixel(const double* __restrict__ in, double* __restrict__ out, int h, int w, int axis,
+                                                  const double* __restrict__ k, int radius, long long p) {
+    const int len = axis == 0 ? h : w;
+    const long long step = axis == 0 ? 3LL * w : 3;
+    const int r = (int)(p / w), c = (int)(p - (long long)r * w);
+    const int pos = axis == 0 ? r : c;
+    const long long line0 = axis == 0 ? 3LL * c : 3LL * r * w;
+    const double* ctr = in + line0 + pos * step;
+    const double kc = k[radius];
+    double a0 = __dmul_rn(ctr[0], kc), a1 = __dmul_rn(ctr[1], kc), a2 = __dmul_rn(ctr[2], kc);
+    for (int j = radius; j >= 1; --j) {
+        const double* lo = in + line0 + slic_reflect(pos - j, len) * step;
+        const double* hi = in + line0 + slic_reflect(pos + j, len) * step;
+        const double wj = k[radius - j];
+        a0 = __dadd_rn(a0, __dmul_rn(__dadd_rn(lo[0], hi[0]), wj));
+        a1 = __dadd_rn(a1, __dmul_rn(__dadd_rn(lo[1], hi[1]), wj));
+        a2 = __dadd_rn(a2, __dmul_rn(__dadd_rn(lo[2], hi[2]), wj));
+    }
+    double* o = out + 3 * p;
+    o[0] = a0; o[1] = a1; o[2] = a2;
+}
+
 __global__ void __launch_bounds__(SLIC_THREADS) slic_smooth_kernel(const double* __restrict__ in, double* __restrict__ out, int h, int w,
                                                                    int axis, const double* __restrict__ k, int radius) {
     const long long n = (long long)w * h;
-    const int len = axis == 0 ? h : w;
-    const long long step = axis == 0 ? 3LL * w : 3;
-    for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < n; p += (long long)gridDim.x * blockDim.x) {
-        const int r = (int)(p / w), c = (int)(p - (long long)r * w);
-        const int pos = axis == 0 ? r : c;
-        const long long line0 = axis == 0 ? 3LL * c : 3LL * r * w;
-        const double* ctr = in + line0 + pos * step;
-        const double kc = k[radius];
-        double a0 = __dmul_rn(ctr[0], kc), a1 = __dmul_rn(ctr[1], kc), a2 = __dmul_rn(ctr[2], kc);
-        for (int j = radius; j >= 1; --j) {
-            const double* lo = in + line0 + slic_reflect(pos - j, len) * step;
-            const double* hi = in + line0 + slic_reflect(pos + j, len) * step;
-            const double wj = k[radius - j];
-            a0 = __dadd_rn(a0, __dmul_rn(__dadd_rn(lo[0], hi[0]), wj));
-            a1 = __dadd_rn(a1, __dmul_rn(__dadd_rn(lo[1], hi[1]), wj));
-            a2 = __dadd_rn(a2, __dmul_rn(__dadd_rn(lo[2], hi[2]), wj));
-        }
-        double* o = out + 3 * p;
-        o[0] = a0; o[1] = a1; o[2] = a2;
-    }
+    for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < n; p += (long long)gridDim.x * blockDim.x)
+        slic_smooth_pixel(in, out, h, w, axis, k, radius, p);
 }
 
 // S3: rgb2lab of skimage.color on float pixels (channel 0 plays 'R'), times ratio = 1 / compactness.  pow and cbrt are

@@ -473,7 +473,9 @@ class Handle:
     def felzenszwalb_device_batch(self, d_frames, frame_bytes, frame_index, frame_h, frame_w, stride, rects, d_labels_out,
                                   label_offsets, scale=100, sigma=0.5, min_size=50):
         """Felzenszwalb of many crops of a device-resident clip in ONE native call (pcm_felzenszwalb_device_batch), laid out
-        like quickshift_device_batch.  Returns the segment counts (int32 array)."""
+        like quickshift_device_batch: the maps and counts of one call per crop, computed in one batched pass whose merge
+        rounds serve all crops at once.  Returns the segment counts (int32 array).  `felzenszwalb_debug_last` then
+        reports the smoothed image of the last crop and the largest round counts of the batch."""
         fi, rc, off, counts = _batch_args(frame_index, rects, label_offsets)
         weights, radius = _gaussian_weights(sigma)
         self._check(self.lib.pcm_felzenszwalb_device_batch(self._h, len(fi), C.c_void_p(d_frames), int(frame_bytes), _ptr(fi),
